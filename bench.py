@@ -46,7 +46,15 @@ def parse_args():
     ap.add_argument("--cli-clock", type=int, default=0, metavar="READS",
                     help="also time the `talc` command line end to end (process start -> .fa closed) on READS reads, "
                          "from the text dump and from --tableCache (SURVEY 8d second clock)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="CUDA path only: write what the last timed step computed (rank 0) to DIR/*.npy, so that two "
+                         "builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "talc_b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
+    return args
 
 
 def measured_traffic():
@@ -290,6 +298,10 @@ def run_gpu(args, rank, world, local_rank):
     clocks = sampler.stop()
     if errors:
         raise errors[0]
+    if args.dump_outputs and rank == 0:
+        # timed step j ran on lane j mod L, into that lane's buffers; read them before the runs below reuse lane 0's
+        last = (args.steps - 1) % L
+        dump_outputs(args.dump_outputs, *bufs[last], B, results[last][-1][0])
     bases, agg, launches = 0, None, 0
     for c, nb in [x for l in range(L) for x in results[l]]:
         bases += nb
@@ -476,6 +488,44 @@ def run_gpu(args, rank, world, local_rank):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_MAX_READS = 1 << 20
+DUMP_SAMPLE_READS = 6144
+DUMP_MAX_BASES = 10 << 20
+
+
+def read_digests(out, off, m):
+    """48 bits of BLAKE2b over each of the first m corrected reads: exact in a float64, so that a difference in any
+    base of any read shows in a float array."""
+    import hashlib
+    import numpy as np
+    return np.array([int.from_bytes(hashlib.blake2b(out[off[i]:off[i + 1]].tobytes(), digest_size=6).digest(), "little")
+                     for i in range(m)], dtype=np.float64)
+
+
+def dump_outputs(path, d_out, d_ooff, d_st, n, counters):
+    """What one talc_correct_batch_device call hands back for a batch of n reads, as .npy files.  For the first
+    DUMP_MAX_READS reads: out_offsets.npy (float64, offsets into the corrected bases), status.npy (float32) and
+    read_digests.npy (float64, read_digests of the corrected bases).  For a fixed seeded sample of DUMP_SAMPLE_READS
+    reads (sample_reads.npy, their indices): their corrected bases as ASCII codes (sample_bases.npy, float32, at most
+    DUMP_MAX_BASES of them).  counter_<name>.npy (float64): the call's counters, except its ms_* timings.
+    At most 63 MB in all (42 MB for the default config-2 batch of 131072 reads)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    off = d_ooff[: n + 1].cpu().numpy().astype(np.int64)
+    out = d_out[: int(off[-1])].cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SAMPLE_READS), replace=False))
+    bases = np.concatenate([out[off[i]:off[i + 1]] for i in idx])[:DUMP_MAX_BASES]
+    m = min(n, DUMP_MAX_READS)
+    np.save(os.path.join(path, "out_offsets.npy"), off[: m + 1].astype(np.float64))
+    np.save(os.path.join(path, "status.npy"), d_st[:m].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "read_digests.npy"), read_digests(out, off, m))
+    np.save(os.path.join(path, "sample_reads.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "sample_bases.npy"), bases.astype(np.float32))
+    for name, v in counters.items():
+        if not name.startswith("ms_"):
+            np.save(os.path.join(path, "counter_%s.npy" % name), np.array([v], dtype=np.float64))
 
 
 def table_load_timings(api, cfg, cpu_keys, use_j):

@@ -4,10 +4,9 @@ import ctypes
 import os
 import re
 import subprocess
+import sys
 
-import pytest
-
-from conftest import ROOT, have_gpu
+from conftest import ROOT
 
 
 def _declared_symbols():
@@ -26,12 +25,13 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback():
-    from talc_b200 import api
-    if have_gpu():
-        pytest.skip("a GPU is visible here")
-    with pytest.raises(api.TalcError) as e:
-        api.Talc(api.default_params(21))
-    assert "no CPU path" in str(e.value)
+    """Run with the devices hidden (child process), so that it holds on a machine with a GPU as well."""
+    code = ("import sys; sys.path.insert(0, %r)\nfrom talc_b200 import api\n"
+            "try:\n    api.Talc(api.default_params(21))\n    print('CREATED')\n"
+            "except api.TalcError as e:\n    print('REFUSED', e)\n") % ROOT
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True).stdout
+    assert "REFUSED" in out and "no CPU path" in out
 
 
 def test_product_does_not_reference_the_oracle():

@@ -41,11 +41,42 @@ def test_one_json_line_on_stdout_whatever_else_is_printed(tmp_path):
     assert "python noise" in pr.stderr and "C stdio noise" in pr.stderr and "raw fd noise" in pr.stderr
 
 
-def test_no_numbers_without_a_gpu():
+def test_dump_outputs_writes_the_batch_as_float_arrays(tmp_path):
+    """--dump-outputs: offsets, status and a digest of every read of the batch, the corrected bases of a fixed seeded
+    sample of reads and the call's counters, as float32 / float64 .npy files; the same outputs give the same files,
+    and one changed base anywhere changes the digests."""
+    import numpy as np
     import torch
-    if torch.cuda.is_available():
-        import pytest
-        pytest.skip("needs a machine without a CUDA device")
+    b = _bench()
+    rng = np.random.default_rng(1)
+    n = 8000
+    off = np.concatenate([[0], np.cumsum(rng.integers(0, 50, n))]).astype(np.int64)
+    out = rng.choice(np.frombuffer(b"ACGT", dtype=np.uint8), int(off[-1]) + 100)  # device buffers are larger than the batch
+    st = rng.integers(0, 5, n).astype(np.uint8)
+    ctr = {"lookups_walk": 12345678901, "reads": n, "ms_total": 1.5}
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), torch.from_numpy(out), torch.from_numpy(off), torch.from_numpy(st), n, ctr)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["counter_lookups_walk.npy", "counter_reads.npy", "out_offsets.npy", "read_digests.npy",
+                     "sample_bases.npy", "sample_reads.npy", "status.npy"]
+    got = {}
+    for f in files:
+        x = np.load(tmp_path / "a" / f)
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, np.load(tmp_path / "b" / f)), f
+        got[f[:-4]] = x
+    assert np.array_equal(got["out_offsets"], off) and np.array_equal(got["status"], st)
+    assert got["counter_lookups_walk"][0] == 12345678901 and got["counter_reads"][0] == n
+    idx = got["sample_reads"].astype(np.int64)
+    assert len(idx) == b.DUMP_SAMPLE_READS and (np.diff(idx) > 0).all() and idx[-1] < n
+    assert np.array_equal(got["sample_bases"], np.concatenate([out[off[i]:off[i + 1]] for i in idx]))
+    r = next(i for i in range(n) if i not in set(idx.tolist()) and off[i + 1] > off[i])  # a read outside the sample
+    out[off[r]] ^= 1
+    dig = b.read_digests(out, off, n)
+    assert len(dig) == n and np.nonzero(dig != got["read_digests"])[0].tolist() == [r]
+
+
+def test_no_numbers_without_a_gpu():
+    # the devices are hidden, so that this holds on a machine with a GPU as well
     pr = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"], capture_output=True,
-                        text=True, cwd=ROOT)
+                        text=True, cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert pr.returncode != 0 and pr.stdout.strip() == "" and "no CPU fallback" in pr.stderr

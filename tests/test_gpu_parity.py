@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import have_gpu
+from conftest import ROOT, have_gpu
 
 pytestmark = pytest.mark.gpu
 
@@ -659,3 +659,45 @@ def test_execution_shapes_give_identical_results(api, case_c1, case_c5, case_c3,
     out, off, st, ctr = t.correct(case_c1.reads, case_c1.off)
     assert ctr["reads_second_tier"] > 0
     _assert_same(case_c1, out, off, st, ctr)
+
+
+@pytest.mark.parametrize("steps", [2, 3])
+def test_bench_dumps_what_its_last_timed_step_computed(api, tmp_path, steps):
+    """bench.py --dump-outputs against one correct_device call on the slice of the last timed step, generated here as
+    bench.py generates it.  With two lanes the last step runs on lane 1 (2 steps) or on lane 0 (3 steps)."""
+    import importlib.util
+    import subprocess
+    import sys
+    import torch
+    from talc_b200 import synth
+    B, warmup, dev = 1500, 1, "cuda:0"
+    d = tmp_path / "dump"
+    pr = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                         "--scale", "0.02", "--batch-reads", str(B), "--lanes", "2", "--no-table-load", "--no-cpu-baseline",
+                         "--dump-outputs", str(d)], capture_output=True, text=True, cwd=ROOT)
+    assert pr.returncode == 0, pr.stderr[-3000:]
+    cfg = synth.baseline_config(2, 0.02)
+    tr = synth.make_transcriptome(cfg, dev)
+    keys, counts, _, _ = synth.make_counts(cfg, tr, dev)
+    reads, roff = synth.make_reads(cfg, tr, B * (warmup + steps + 1), dev, seed_offset=3)
+    roff = roff.to(torch.int64)
+    lo = (warmup + steps - 1) * B
+    b0, b1 = int(roff[lo]), int(roff[lo + B])
+    t = api.Talc(api.default_params(cfg.k))
+    t.load_packed(keys.cpu().numpy().astype(np.uint64), counts.cpu().numpy())
+    d_out = torch.empty(2 * (b1 - b0) + 64 * B + 4096, dtype=torch.uint8, device=dev)
+    d_ooff = torch.zeros(B + 1, dtype=torch.int64, device=dev)
+    d_st = torch.zeros(B, dtype=torch.uint8, device=dev)
+    ctr = t.correct_device(reads[b0:b1].contiguous(), (roff[lo:lo + B + 1] - roff[lo]).contiguous(), b1 - b0, d_out, d_ooff, d_st)
+    off = d_ooff.cpu().numpy()
+    out = d_out[: int(off[-1])].cpu().numpy()
+    spec = importlib.util.spec_from_file_location("talc_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    assert np.array_equal(np.load(d / "out_offsets.npy"), off)
+    assert np.array_equal(np.load(d / "status.npy"), d_st.cpu().numpy())
+    assert np.array_equal(np.load(d / "read_digests.npy"), bench.read_digests(out, off, B))
+    idx = np.load(d / "sample_reads.npy").astype(np.int64)
+    assert np.array_equal(np.load(d / "sample_bases.npy"), np.concatenate([out[off[r]:off[r + 1]] for r in idx]))
+    for k in SHARED + ["reads", "bases_in", "reads_ok"]:
+        assert np.load(d / ("counter_%s.npy" % k))[0] == ctr[k], k
