@@ -11,6 +11,8 @@
  *       <- the body of the OpenMP loop over reads                                  main.cpp:247-306
  *          Read r(id,seq); if len>K: r.reCoverage() -> r.defineStructure2() -> r.correct2(); r.getCorrSeq()
  *          (Read.cpp:174-386, Explorer.cpp, Trail.cpp, Trajectory.cpp)
+ *   talc_ctx_set_reverse
+ *       <- if (reverse) reverseComplement(seq) before, and of the corrected read after, the above   main.cpp:253,285-286
  *   talc_coverage_batch
  *       <- getLRCountsInSR(seq, K, SR_DBG, ..)                                     Jellyfish.cpp:471-496
  *   talc_table_lookup
@@ -60,7 +62,9 @@ enum {
   TALC_READ_SHORT = 3,         /* len <= K: passed through, nothing logged        */
   TALC_READ_RESOURCE = 4       /* not in the reference (which has no memory bound): the search of this read outgrew even
                                   the second-tier scratch arena (talc_ctx_set_scratch); the read is passed through
-                                  uncorrected and counted in talc_counters.reads_overflow; the batch itself succeeds */
+                                  uncorrected and counted in talc_counters.reads_overflow; the batch itself succeeds.
+                                  In reverse mode (talc_ctx_set_reverse) it comes back like every other read that is not
+                                  TALC_READ_OK: as the reverse complement of its input */
 };
 
 /* algorithmic work of a batch (properties of the algorithm on the input, SURVEY 8d) and timings */
@@ -113,6 +117,16 @@ int talc_ctx_set_scratch(talc_ctx* ctx, uint32_t tier1_bytes, uint32_t tier2_byt
  * (the round-1 shape, kept for A/B measurements).  Results are identical (tests/test_gpu_parity.py).  read_contexts =
  * reads in flight in split mode (each owns a first-tier arena), walk_step_cap = steps per frontier and round.  */
 int talc_ctx_set_exec(talc_ctx* ctx, uint32_t split_walk, uint32_t read_contexts, uint32_t walk_step_cap);
+
+/* main.cpp:253,285-286 (--reverse): long reads sequenced from the strand opposite to the short reads.  reverse != 0:
+ * every read is reverse-complemented (Dna5: ACGT in either case -> complement, anything else -> N) before anything
+ * else, the len <= K test included; a corrected read comes back as the reverse complement of its corrected sequence,
+ * i.e. in the read's input orientation; every other read comes back as the reverse complement of its input (SURVEY
+ * Q24: the reference does not undo the flip for reads it cannot correct).  Coverage (talc_coverage_batch) and the
+ * read_stats of the stream describe the reverse-complemented read.  The k-mer table is not affected.  Set on a
+ * context, not on a lane (a lane follows its parent, TALC_ERR_ARG on a lane); not while a stream on the context has
+ * batches pending.  Default 0.                                                                                     */
+int talc_ctx_set_reverse(talc_ctx* ctx, int reverse);
 
 /* ---- k-mer table (main.cpp:231-232) -------------------------------------------------------- */
 /* Jellyfish `dump -c` text (KMER<ws>COUNT per line), optional junction dump (NULL = none).      */

@@ -55,6 +55,7 @@ def lib():
         L.talc_last_error.argtypes = [vp]
         L.talc_ctx_set_scratch.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32]
         L.talc_ctx_set_exec.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32]
+        L.talc_ctx_set_reverse.argtypes = [vp, C.c_int]
         L.talc_table_load_dump.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_table_load_dump_host.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_dump_write_packed.argtypes = [C.c_char_p, vp, vp, C.c_uint64, C.c_uint32]
@@ -152,6 +153,11 @@ class Talc:
     def set_exec(self, split_walk=0, read_contexts=0, walk_step_cap=0):
         """split_walk: 1 = suspendable reads + walk kernel, 2 = one monolithic kernel (the default); 0 keeps a value."""
         self._check(lib().talc_ctx_set_exec(self.h, split_walk, read_contexts, walk_step_cap), "talc_ctx_set_exec")
+
+    def set_reverse(self, reverse: bool):
+        """talc --reverse: reads are corrected on the opposite strand; corrected reads come back in their input
+        orientation, all others reverse-complemented (talc_ctx_set_reverse).  Raises on a lane."""
+        self._check(lib().talc_ctx_set_reverse(self.h, 1 if reverse else 0), "talc_ctx_set_reverse")
 
     # ---- table
     def load_dump(self, dump: str, junctions: Optional[str] = None):

@@ -1,7 +1,7 @@
 // talc_main.cpp -- the drop-in `talc` command line on top of libtalc_b200.so.
 //
 // Same interface and the same output files as the reference program (main.cpp:83-325):
-//   talc <reads.fa|fq> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [tunables]
+//   talc <reads.fa|fq> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse] [tunables]
 //   <prefix>.config.txt (Settings.cpp:160-185)   <prefix>.stats_basics.txt header (Read.cpp:394-415)
 //   <prefix>.log, appended, one line per failed read (io.cpp:105-111; messages main.cpp:290,294)
 //   <prefix>.fa, every read in input order, 70 columns (main.cpp:310, io.cpp:50-75)
@@ -94,7 +94,6 @@ static int parse(int argc, const char** argv, Cli& c) {
     else pos.push_back(a);
   }
   if (pos.size() != 1 || !c.haveK || !c.haveSR) return 1;
-  if (c.reverse) { std::cerr << "talc: --reverse is not supported by the GPU build\n"; return 1; }
   if (c.queryMode != "memory") { std::cerr << "talc: only query mode 'memory' is supported\n"; return 1; }
   c.reads = pos[0];
   return 0;
@@ -134,7 +133,7 @@ int main(int argc, const char** argv) {
   Cli cli;
   const int pr = parse(argc, argv, cli);
   if (pr == 2) {
-    std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--gpus <N>] [--tableCache <file>]"
+    std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse] [--gpus <N>] [--tableCache <file>]"
                  " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer]\n";
     return 0;
   }
@@ -163,6 +162,11 @@ int main(int argc, const char** argv) {
   for (int g = 0; g < cli.gpus; ++g) {  // (one thread per device was measured: no faster, the driver serialises it)
     if (talc_ctx_create(&cli.p, g, &ctx[g]) != 0) {
       std::cerr << "talc: cannot create a GPU context on device " << g << ": " << talc_last_error(nullptr) << "\n";
+      return 2;
+    }
+    // --reverse (main.cpp:253,285-286): the long reads only; the stream's lanes follow their context
+    if (cli.reverse && talc_ctx_set_reverse(ctx[g], 1) != 0) {
+      std::cerr << "talc: " << talc_last_error(ctx[g]) << "\n";
       return 2;
     }
   }

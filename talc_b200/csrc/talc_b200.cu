@@ -7,6 +7,7 @@
 //   cost_key_kernel (+ cub radix sort)                                  processing order: estimated cost, descending
 //   correct_kernel                                                      segmentation + graph search + scoring
 //   gather_kernel                                                       corrected reads back into input order
+//   revcomp_reads_kernel                                                --reverse: every read reverse-complemented first
 // Grid sizes are multiples of the SM count; per-thread scratch lives in HBM (180 GB makes that cheap).
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -575,16 +576,46 @@ __global__ void ctx_init_kernel(ReadCtx* ctxs, u32 nCtx, u32* readyList, u32* nR
   if (i == 0) *nReady = nCtx;
 }
 
-// corrected reads from allocation order into input order; one warp per read, 16-byte chunks
+// Dna5 conversion followed by SeqAn's reverseComplement, one base: ACGT in either case -> complement, anything else -> N
+__device__ __forceinline__ u8 dna5_complement(u8 c) {
+  switch (c) {
+    case 'A': case 'a': return 'T';
+    case 'C': case 'c': return 'G';
+    case 'G': case 'g': return 'C';
+    case 'T': case 't': return 'A';
+    default: return 'N';
+  }
+}
+
+// --reverse (main.cpp:253): every read reverse-complemented before anything else; one warp per read, same offsets
+__global__ void revcomp_reads_kernel(const u8* __restrict__ in, const u64* __restrict__ offs, u32 n, u8* __restrict__ out) {
+  const u32 lane = threadIdx.x & 31;
+  const u32 warpsPerBlock = blockDim.x >> 5;
+  for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
+    const u64 off = offs[r];
+    const u64 L = offs[r + 1] - off;
+    const u8* src = in + off + L - 1;
+    u8* dst = out + off;
+    for (u64 i = lane; i < L; i += 32) dst[i] = dna5_complement(src[-(i64)i]);
+  }
+}
+
+// corrected reads from allocation order into input order; one warp per read.  reverse (uniform per launch): a read
+// that was corrected goes back to the input's strand (main.cpp:285-286); every other read leaves as its reverse-
+// complemented input (Q24)
 __global__ void gather_kernel(const u8* __restrict__ arena, const u64* __restrict__ pos, const u32* __restrict__ len,
-                              const u64* __restrict__ outOff, u32 n, u8* __restrict__ out) {
+                              const u64* __restrict__ outOff, u32 n, u8* __restrict__ out, const u8* __restrict__ status,
+                              u32 reverse) {
   const u32 lane = threadIdx.x & 31;
   const u32 warpsPerBlock = blockDim.x >> 5;
   for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
     const u8* src = arena + pos[r];
     u8* dst = out + outOff[r];
     const u32 L = len[r];
-    for (u32 i = lane; i < L; i += 32) dst[i] = src[i];
+    if (reverse && status[r] == TALC_READ_OK)
+      for (u32 i = lane; i < L; i += 32) dst[i] = dna5_complement(src[L - 1 - i]);
+    else
+      for (u32 i = lane; i < L; i += 32) dst[i] = src[i];
   }
 }
 __global__ void len_to_u64_kernel(const u32* len, u32 n, u64* out) {
@@ -757,11 +788,12 @@ struct talc_ctx {
   u32 walkStepCap = 48;    // steps a frontier may take per round of the walk kernel (bounds the round's tail)
   u32 pauseCycles = 200000;  // SM cycles (~100 us) a read may run per round of the control kernel
   u32 inlineInner = 6, inlineBorder = 6;
+  u32 reverse = 0;  // talc_ctx_set_reverse: the long reads are corrected on the opposite strand (rcBases)
   u64 lastRounds = 0;
   double* modelTabs = nullptr;  // 3 x kModelTabN doubles
   // cached device buffers
   DevBuf bases, offs, kmerOff, nk, cov, order, sortKey, sortKeyOut, sortVal, cubTmp, arenas, outArena, outPos, outLen,
-      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists;
+      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases;
 };
 
 static const u32 kModelTabN = 16384;
@@ -885,7 +917,7 @@ void talc_ctx_destroy(talc_ctx* c) {
   if (c->modelTabs) cudaFree(c->modelTabs);
   DevBuf* bufs[] = {&c->bases, &c->offs, &c->kmerOff, &c->nk, &c->cov, &c->order, &c->sortKey, &c->sortKeyOut, &c->sortVal,
                     &c->cubTmp, &c->arenas, &c->outArena, &c->outPos, &c->outLen, &c->outLen64, &c->status, &c->outOffs,
-                    &c->out, &c->misc, &c->overflowList, &c->readCtxs, &c->roundLists};
+                    &c->out, &c->misc, &c->overflowList, &c->readCtxs, &c->roundLists, &c->rcBases};
   for (DevBuf* b : bufs) b->release();
   for (int i = 0; i < 8; ++i) cudaEventDestroy(c->ev[i]);
   cudaStreamDestroy(c->stream);
@@ -919,6 +951,7 @@ static void lane_follow(talc_ctx* sh) {
   sh->pauseCycles = c->pauseCycles;
   sh->inlineInner = c->inlineInner;
   sh->inlineBorder = c->inlineBorder;
+  sh->reverse = c->reverse;
 }
 int talc_ctx_create_lane(talc_ctx* parent, talc_ctx** out) {
   if (!parent || !out || parent->parent) return TALC_ERR_ARG;
@@ -944,6 +977,14 @@ int talc_ctx_set_exec(talc_ctx* c, uint32_t split_walk, uint32_t read_contexts, 
   if (split_walk) c->splitWalk = split_walk == 1 ? 1u : 0u;
   if (read_contexts) c->nCtxTier1 = read_contexts < 4 ? 4 : read_contexts;
   if (walk_step_cap) c->walkStepCap = walk_step_cap;
+  return TALC_OK;
+}
+
+// --reverse (main.cpp:253,285-286).  A lane follows its parent; the stream's lanes read it at the start of each batch.
+int talc_ctx_set_reverse(talc_ctx* c, int reverse) {
+  if (!c) return TALC_ERR_ARG;
+  if (c->parent) { c->err = "a lane follows the strand setting of the context it was made from"; return TALC_ERR_ARG; }
+  c->reverse = reverse != 0;
   return TALC_OK;
 }
 
@@ -1663,8 +1704,9 @@ static int run_pass(talc_ctx* c, CorrectArgs& A, u32 nCtx, u64* launches) {
 }
 
 // ---------------------------------------------------------------------------------- correction
-// shared front end: k-mer offsets, length-sorted order, coverage.  d_bases/d_offs on device.
-static int prepare_batch(talc_ctx* c, const u8* dBases, const u64* dOffs, u32 n, u64 totalBases, u64& totalKmers) {
+// shared front end: k-mer offsets, length-sorted order, coverage.  d_bases/d_offs on device.  In reverse mode the reads
+// are first reverse-complemented into rcBases (same offsets) and dBases is pointed there for the rest of the batch.
+static int prepare_batch(talc_ctx* c, const u8*& dBases, const u64* dOffs, u32 n, u64 totalBases, u64& totalKmers) {
   const u32 K = c->params.K;
   CUDA_TRY(c, c->nk.reserve((size_t)(n + 1) * 8));
   CUDA_TRY(c, c->kmerOff.reserve((size_t)(n + 1) * 8));
@@ -1682,13 +1724,20 @@ static int prepare_batch(talc_ctx* c, const u8* dBases, const u64* dOffs, u32 n,
   CUDA_TRY(c, c->cubTmp.reserve(std::max(tmp1, tmp2)));
   size_t tb = c->cubTmp.cap;
   CUDA_TRY(c, cub::DeviceScan::ExclusiveSum(c->cubTmp.p, tb, (u64*)c->nk.p, (u64*)c->kmerOff.p, n + 1, c->stream));
-  u64 hk = 0;
+  u64 hk = 0, hEnd = 0;
   CUDA_TRY(c, cudaMemcpyAsync(&hk, (u64*)c->kmerOff.p + n, 8, cudaMemcpyDeviceToHost, c->stream));
+  if (c->reverse) CUDA_TRY(c, cudaMemcpyAsync(&hEnd, dOffs + n, 8, cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   totalKmers = hk;
   CUDA_TRY(c, c->cov.reserve((size_t)(hk + 4) * 4));
   TableView tv{c->slots, c->capacity - 1};
   const int blocks = c->sms * 8;
+  if (c->reverse) {  // sized from the offsets themselves: the caller's buffer is read where they point
+    CUDA_TRY(c, c->rcBases.reserve(hEnd + 64));
+    revcomp_reads_kernel<<<blocks, 256, 0, c->stream>>>(dBases, dOffs, n, (u8*)c->rcBases.p);
+    CUDA_TRY(c, cudaGetLastError());
+    dBases = (const u8*)c->rcBases.p;
+  }
   CUDA_TRY(c, cudaEventRecord(c->ev[1], c->stream));
   coverage_kernel<<<blocks, 256, 0, c->stream>>>(tv, K, dBases, dOffs, (const u64*)c->kmerOff.p, n, (u32*)c->cov.p);
   CUDA_TRY(c, cudaGetLastError());
@@ -1834,7 +1883,7 @@ static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const u
   if (hOutFull) { c->err = "internal output arena too small"; return TALC_ERR_CAPACITY; }
   if (hTotalOut > outCapacity) { c->err = "out_capacity too small for the corrected reads"; return TALC_ERR_CAPACITY; }
   gather_kernel<<<c->sms * 8, 256, 0, c->stream>>>((const u8*)c->outArena.p, (const u64*)c->outPos.p, (const u32*)c->outLen.p,
-                                                  dOutOffs, n, dOut);
+                                                  dOutOffs, n, dOut, dStatus, c->reverse);
   CUDA_TRY(c, cudaGetLastError());
   CUDA_TRY(c, cudaEventRecord(c->ev[5], c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
@@ -1924,6 +1973,7 @@ int talc_correct_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offset
 int talc_coverage_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offsets, uint32_t n, uint32_t* counts,
                         uint64_t countsCapacity) {
   if (!c || !offsets || (n && !bases)) return TALC_ERR_ARG;
+  if (c->parent) lane_follow(c);
   if (!c->tableReady) return TALC_ERR_NO_TABLE;
   if (!n) return TALC_OK;
   CUDA_TRY(c, cudaSetDevice(c->device));
@@ -1933,7 +1983,8 @@ int talc_coverage_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offse
   CUDA_TRY(c, cudaMemcpyAsync(c->bases.p, bases, total, cudaMemcpyHostToDevice, c->stream));
   CUDA_TRY(c, cudaMemcpyAsync(c->offs.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, c->stream));
   u64 totalKmers = 0;
-  int rc = prepare_batch(c, (const u8*)c->bases.p, (const u64*)c->offs.p, n, total, totalKmers);
+  const u8* dBases = (const u8*)c->bases.p;  // the reverse-complemented copy in reverse mode
+  int rc = prepare_batch(c, dBases, (const u64*)c->offs.p, n, total, totalKmers);
   if (rc) return rc;
   if (totalKmers > countsCapacity) { c->err = "counts_capacity too small"; return TALC_ERR_CAPACITY; }
   CUDA_TRY(c, cudaMemcpyAsync(counts, c->cov.p, totalKmers * 4, cudaMemcpyDeviceToHost, c->stream));
