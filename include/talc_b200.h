@@ -245,6 +245,17 @@ int talc_bench_random_sectors(talc_ctx* ctx, uint64_t buffer_bytes, int dependen
  * cand_ext, score, stop; aux = xdrop, aux2 = direction_right, K from the context)                 */
 int talc_test_align(talc_ctx* ctx, int op, const uint8_t* a, const uint64_t* a_off, const uint8_t* b,
                     const uint64_t* b_off, uint32_t n, int aux, int aux2, int32_t* result);
+/* the same operations on the views the correction builds.  reads (concatenated bytes, read_off[n_reads+1]) are
+ * packed as the corrector packs them (2 bits per base, 4 when the read holds an N); desc[8*i..] = {read, start,
+ * step, len} of side a, then of side b.  step +1 / -1: bases start, start+step, ... of the packed read (walk order);
+ * step 0: read[start, start+len) (A, C, G, T only) copied into a 2-bit trail slot whose bits past len are random.
+ * op 0-2: result[i]; op 3: as above; op 4: X-drop of query a against database b, result[4*i..]: ext_rows,
+ * ext_cols, DP cells visited, end score (aux = xdrop); op 5: result[4*i..]: NW score, LCS length of the fused pass;
+ * op 6: every aux consecutive pairs form one gardening frontier, the a side of its first pair the reference and the
+ * b sides its trails (step 0, equal lengths): result[i] = overlap score of trail i with the shared-prefix stripe
+ * reuse of the corrector.  A score of INT32_MIN means the per-pair scratch (2 MB) was too small.                  */
+int talc_test_align_slices(talc_ctx* ctx, int op, const uint8_t* reads, const uint64_t* read_off, uint32_t n_reads,
+                           const int32_t* desc, uint32_t n, int aux, int aux2, int32_t* result);
 /* permutation produced by the device replica of libstdc++ std::sort on keys[n] (operator<)        */
 int talc_test_sort(talc_ctx* ctx, const int64_t* keys, uint32_t n, uint32_t* perm);
 

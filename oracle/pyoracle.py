@@ -61,6 +61,7 @@ def lib():
         L.orc_lcs.argtypes = [C.c_char_p, C.c_char_p]
         L.orc_overlap.argtypes = [C.c_char_p, C.c_char_p, C.c_int]
         L.orc_xdrop.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+        L.orc_xdrop_counted.argtypes = L.orc_xdrop.argtypes + [C.POINTER(C.c_uint64)]
         L.orc_seed_extend.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_uint32, C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_double),
                                       C.POINTER(C.c_int32)]
@@ -185,6 +186,13 @@ def xdrop(query: bytes, database: bytes, left: bool, x: int):
     r, c = C.c_uint64(0), C.c_uint64(0)
     lib().orc_xdrop(query, database, 1 if left else 0, x, C.byref(r), C.byref(c))
     return r.value, c.value
+
+
+def xdrop_counted(query: bytes, database: bytes, left: bool, x: int):
+    """xdrop() plus the number of DP cells the extension visited: (ext_rows, ext_cols, cells)."""
+    r, c, n = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+    lib().orc_xdrop_counted(query, database, 1 if left else 0, x, C.byref(r), C.byref(c), C.byref(n))
+    return r.value, c.value, n.value
 
 
 def seed_extend(reference: bytes, candidate: bytes, x: int, right: bool, k: int):

@@ -177,6 +177,16 @@ void orc_xdrop(const char* query_seg, const char* database_seg, int extend_left,
   *ext_rows = r;
   *ext_cols = c;
 }
+// orc_xdrop plus the number of DP cells the extension visited (Counters::cells_xdrop)
+void orc_xdrop_counted(const char* query_seg, const char* database_seg, int extend_left, int xdrop, uint64_t* ext_rows,
+                       uint64_t* ext_cols, uint64_t* cells) {
+  Counters ctr;
+  size_t r = 0, c = 0;
+  xdrop_extend(query_seg, database_seg, extend_left != 0, xdrop, r, c, &ctr);
+  *ext_rows = r;
+  *ext_cols = c;
+  *cells = ctr.cells_xdrop;
+}
 // getSeedAndExtension: returns lengths of (refExtension, histExtension), posOnRef, score, stop
 void orc_seed_extend(const char* reference, const char* candidate, int xdrop, int direction_right, uint32_t K,
                      int32_t* ref_ext_len, int32_t* hist_ext_len, int32_t* pos_on_ref, double* score, int32_t* stop) {

@@ -92,6 +92,7 @@ def lib():
         L.talc_stream_last_error.argtypes = [vp]
         L.talc_stream_close.argtypes = [vp]
         L.talc_test_align.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_uint32, C.c_int, C.c_int, vp]
+        L.talc_test_align_slices.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, C.c_uint32, C.c_int, C.c_int, vp]
         L.talc_test_sort.argtypes = [vp, vp, C.c_uint32, vp]
         _lib = L
     return _lib
@@ -312,6 +313,20 @@ class Talc:
         self._check(lib().talc_test_align(self.h, op, _ptr(a), _ptr(ao), _ptr(b), _ptr(bo), n, aux, aux2, _ptr(res)),
                     "talc_test_align")
         return res.reshape(n, 4) if op >= 3 else res
+
+    def test_align_slices(self, op: int, reads, desc, aux: int = 0, aux2: int = 0) -> np.ndarray:
+        """talc_test_align_slices: `reads` a list of byte strings, `desc` an [n, 8] array of {read, start, step, len}
+        for side a, then side b."""
+        off = np.zeros(len(reads) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([len(r) for r in reads])
+        data = np.frombuffer(b"".join(reads) + b"\0", dtype=np.uint8).copy()
+        desc = np.ascontiguousarray(desc, dtype=np.int32).reshape(-1, 8)
+        n = len(desc)
+        wide = 3 <= op <= 5
+        res = np.zeros(n * (4 if wide else 1), dtype=np.int32)
+        self._check(lib().talc_test_align_slices(self.h, op, _ptr(data), _ptr(off), len(reads), _ptr(desc), n, aux, aux2,
+                                                 _ptr(res)), "talc_test_align_slices")
+        return res.reshape(n, 4) if wide else res
 
     def test_sort(self, keys) -> np.ndarray:
         keys = np.ascontiguousarray(keys, dtype=np.int64)

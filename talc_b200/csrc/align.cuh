@@ -108,7 +108,7 @@ TALC_HDN void build_peq(const SeqView& pat, u32 pn, u32 block, u64 peq[5]) {
   for (u32 r = r0; r < r1; ++r) peq[pat.code(r)] |= 1ull << (r - r0);
 }
 
-// unit-cost edit distance between a[0..an) and b[0..bn) (both non-empty)
+// unit-cost edit distance between a[0..an) and b[0..bn) (either may be empty)
 TALC_HDN int nw_distance_scalar(const SeqView& a, u32 an, const SeqView& b, u32 bn, Arena& ar, DpStats* st) {
   // pattern (rows, bit-parallel) = the shorter one, text (columns) = the longer one
   const bool a_is_pat = an <= bn;
@@ -116,6 +116,7 @@ TALC_HDN int nw_distance_scalar(const SeqView& a, u32 an, const SeqView& b, u32 
   const SeqView txt = a_is_pat ? b : a;
   const u32 pn = a_is_pat ? an : bn;
   const u32 tn = a_is_pat ? bn : an;
+  if (pn == 0) return (int)tn;  // no block: the text is inserted whole
   if (st) st->cells_nw += (u64)an * bn;
   const u32 nblocks = (pn + 63) / 64;
   const u32 mk = ar.mark();
@@ -155,7 +156,7 @@ TALC_HDN int nw_distance_scalar(const SeqView& a, u32 an, const SeqView& b, u32 
   return score;
 }
 
-// length of the longest common subsequence of a[0..an) and b[0..bn) (both non-empty)
+// length of the longest common subsequence of a[0..an) and b[0..bn) (either may be empty)
 TALC_HDN int lcs_length_scalar(const SeqView& a, u32 an, const SeqView& b, u32 bn, Arena& ar, DpStats* st) {
   const bool a_is_pat = an <= bn;
   const SeqView pat = a_is_pat ? a : b;
@@ -208,6 +209,10 @@ TALC_HDN int lcs_length_scalar(const SeqView& a, u32 an, const SeqView& b, u32 b
 __device__ __noinline__ int nw_lcs_fused(const SeqView& a, u32 an, const SeqView& b, u32 bn, Arena& ar, DpStats* st, int& lcsOut,
                                          int what) {
   const u32 longer = an >= bn ? an : bn;
+  if (an == 0 || bn == 0) {  // the pipeline below needs a text character and a block
+    lcsOut = 0;
+    return (int)longer;
+  }
   if (longer > 2048) {  // more than one stripe of 32 blocks: the striped scalar forms (rare)
     const int d = (what & 1) ? nw_distance_scalar(a, an, b, bn, ar, st) : 0;
     lcsOut = (what & 2) ? lcs_length_scalar(a, an, b, bn, ar, st) : 0;
@@ -440,6 +445,30 @@ __device__ __forceinline__ u32 packed_lcp(const u64* a, const u64* b, u32 n) {
   }
   return n;
 }
+// Gardening (scoreBridges, Explorer.cpp:689-706): the n trails of a frontier, each cn bases long in a 2-bit slot
+// (trail(j) -> words; bases past cn are stale), against the same reference.  The stripes of the DP that lie inside
+// the prefix a trail shares with its predecessor in the list (siblings are neighbours) are not recomputed: their
+// boundary columns are still parked from an earlier trail.  store(j, score) receives each result; false when the
+// arena cannot hold the parked columns.
+template <class TrailWords, class Store>
+__device__ __forceinline__ bool overlap_score_frontier(const SeqView& ref, u32 rn, u32 cn, u32 n, TrailWords trail,
+                                                       Store store, Arena& ar, DpStats* st) {
+  const u32 W = 32u * kOvlCols, ns = (cn + W - 1) / W;
+  const u32 mk = ar.mark();
+  i32* bufs = (i32*)ar.alloc(ns * (rn + 1) * 4);
+  if (!bufs) return false;
+  TALC_ROLLED
+  for (u32 j = 0; j < n; ++j) {
+    u32 skip = 0;
+    if (j) {
+      skip = packed_lcp(trail(j), trail(j - 1), cn) / W;
+      if (skip > ns - 1) skip = ns - 1;  // the last stripe carries the result
+    }
+    store(j, overlap_score_stripes(ref, rn, view_of_path(trail(j), cn), cn, bufs, skip, st));
+  }
+  ar.release(mk);
+  return true;
+}
 #else
 inline int overlap_score(const SeqView& ref, u32 rn, const SeqView& cand, u32 cn, Arena& ar, DpStats* st) {
   return overlap_score_scalar(ref, rn, cand, cn, ar, st);
@@ -647,6 +676,81 @@ TALC_HDN SeedExt seed_and_extension(const SeqView& refArg, const SeqView& candAr
     r.stop = true;
   }
   return r;
+}
+
+// ---- self-tests of the scoring primitives (talc_test_align*, and the host emulation in tests/hostemu)
+// One side of a pair as the pipeline hands it over: with step +1 / -1, `len` bases of `rd` from `start` in walk order,
+// the read packed as the Corrector packs it (2 bits per base, 4 when the read holds an N); with step 0, the bases
+// rd[start, start + len) (A, C, G, T only) as a 2-bit trail slot whose bits past `len` are stale (seeded by `salt`).
+// Must be called by all lanes of the warp with identical arguments; nullptr words when the arena is exhausted.
+TALC_HD SeqView selftest_view(const ReadView& rd, i32 start, i32 step, u32 len, u64 salt, Arena& ar) {
+  SeqView v;
+  v.start = start;
+  v.step = step;
+  v.len = len;
+  v.lg = 5;
+  if (step != 0) {
+    u64* w = (u64*)ar.alloc(packed_read_alloc(rd.len) * 8);
+    v.w = w;
+    if (!w) return v;
+    bool hasN = false;
+    for (u32 i = lane_id(); i < rd.len; i += lane_count()) hasN |= rd.code(i) > 3;
+    hasN = warp_any(hasN);
+    for (u32 wi = lane_id(); wi < packed_read_words(rd.len, hasN); wi += lane_count()) w[wi] = packed_read_word(rd, wi, hasN);
+    v.lg = hasN ? 4u : 5u;
+  } else {
+    const u32 nw = (len + 31) / 32 + 1;
+    u64* w = (u64*)ar.alloc(nw * 8);
+    v.w = w;
+    v.start = 0;
+    v.step = 1;
+    if (!w) return v;
+    for (u32 wi = lane_id(); wi < nw; wi += lane_count()) {
+      u64 x = (salt << 20) + wi + 1;  // splitmix64
+      x = (x ^ (x >> 30)) * 0xbf58476d1ce4e5b9ull;
+      x = (x ^ (x >> 27)) * 0x94d049bb133111ebull;
+      x ^= x >> 31;
+      for (u32 j = 0; j < 32 && 32 * wi + j < len; ++j) {
+        const u32 sh = 62 - 2 * j;
+        x = (x & ~(3ull << sh)) | ((u64)(rd.code((u32)start + 32 * wi + j) & 3u) << sh);
+      }
+      w[wi] = x;
+    }
+  }
+  warp_sync();
+  return v;
+}
+// op 0: -edit distance, 1: LCS length, 2: overlap score (a = reference, b = candidate) -> r[0];
+// 3: seed_and_extension(a, b, X = aux, right = aux2) -> {ref_ext, cand_ext, score, stop};
+// 4: X-drop of query a against database b from the origin, X = aux -> {ext_rows, ext_cols, cells, end score};
+// 5: distance and LCS of one fused pass -> {-distance, LCS length}.  r[0] = INT32_MIN when the arena overflowed.
+TALC_HDN void selftest_align_op(int op, const SeqView& va, const SeqView& vb, int aux, int aux2, u32 K, Arena& ar, i32 r[4]) {
+  r[0] = r[1] = r[2] = r[3] = 0;
+  if (op == 0) r[0] = -nw_distance(va, va.len, vb, vb.len, ar, nullptr);
+  else if (op == 1) r[0] = lcs_length(va, va.len, vb, vb.len, ar, nullptr);
+  else if (op == 2) r[0] = overlap_score(va, va.len, vb, vb.len, ar, nullptr);
+  else if (op == 5) {
+    int l = 0;
+    r[0] = -nw_lcs_fused(va, va.len, vb, vb.len, ar, nullptr, l, 3);
+    r[1] = l;
+  } else if (op == 4) {
+    DpStats ds;
+    ds.cells_xdrop = 0;
+    u32 er = 0, ec = 0;
+    i32 es = 0;
+    xdrop_extend(va, 0, va.len, vb, 0, vb.len, aux, er, ec, es, ar, true, &ds);
+    r[0] = (i32)er;
+    r[1] = (i32)ec;
+    r[2] = (i32)ds.cells_xdrop;
+    r[3] = es;
+  } else {
+    const SeedExt e = seed_and_extension(va, vb, aux, aux2 != 0, K, ar, true, nullptr);
+    r[0] = (i32)e.ref_ext;
+    r[1] = (i32)e.cand_ext;
+    r[2] = e.score;
+    r[3] = e.stop ? 1 : 0;
+  }
+  if (ar.overflow) r[0] = INT32_MIN;
 }
 
 }  // namespace talc

@@ -1311,23 +1311,9 @@ class Corrector {
           const u32 rn = (bound >= ref.len) ? ref.len : bound;
           if (P.q11_zero) {
 #if defined(__CUDA_ARCH__)
-            // every trail of the frontier against the same reference: the stripes of the DP that lie inside the
-            // prefix a trail shares with its predecessor in the list (siblings are neighbours) are not recomputed
-            const u32 cn = k + step, W = 32u * kOvlCols, ns = (cn + W - 1) / W;
-            const u32 mks = scratch.mark();
-            i32* bufs = (i32*)scratch.alloc(ns * (rn + 1) * 4);
-            if (!bufs) return false;
-            TALC_ROLLED
-            for (u32 j = 0; j < nNxt; ++j) {
-              u32 skip = 0;
-              if (j) {
-                skip = packed_lcp(slot_ptr(nxt[j].slot), slot_ptr(nxt[j - 1].slot), cn) / W;
-                if (skip > ns - 1) skip = ns - 1;  // the last stripe carries the result
-              }
-              const SeqView pv = view_of_path(slot_ptr(nxt[j].slot), cn);
-              nxt[j].score = overlap_score_stripes(refv, rn, pv, cn, bufs, skip, &dps);
-            }
-            scratch.release(mks);
+            if (!overlap_score_frontier(refv, rn, k + step, nNxt, [&](u32 j) { return (const u64*)slot_ptr(nxt[j].slot); },
+                                        [&](u32 j, int s) { nxt[j].score = s; }, scratch, &dps))
+              return false;
 #else
             TALC_ROLLED
             for (u32 j = 0; j < nNxt; ++j) {
@@ -2083,25 +2069,15 @@ class Corrector {
     keep.init(job.arena, keepBytes & ~7u);
     scratch.init(job.arena + (keepBytes & ~7u), job.arena_bytes - (keepBytes & ~7u));
     {  // packed copy of the read for the scoring loops: 2 bits per base, 4 when the read holds an N
-      const u32 nw4 = (rd.len + 15) / 16 + 2;
-      u64* pw = (u64*)keep.alloc(nw4 * 8);
+      u64* pw = (u64*)keep.alloc(packed_read_alloc(rd.len) * 8);
       if (!pw) return kReadOverflow;
       bool hasN = false;
       TALC_ROLLED
       for (u32 i = lane_id(); i < rd.len; i += lane_count()) hasN |= rd.code(i) > 3;
       hasN = warp_any(hasN);
-      const u32 per = hasN ? 16u : 32u, bits = hasN ? 4u : 2u;
-      const u32 nw = (rd.len + per - 1) / per + 1;
+      const u32 nw = packed_read_words(rd.len, hasN);
       TALC_ROLLED
-      for (u32 wi = lane_id(); wi < nw; wi += lane_count()) {
-        u64 x = 0;
-        TALC_ROLLED
-        for (u32 j = 0; j < per; ++j) {
-          const u32 idx = wi * per + j;
-          x = (x << bits) | (u64)((idx < rd.len) ? rd.code(idx) : 0u);
-        }
-        pw[wi] = x;
-      }
+      for (u32 wi = lane_id(); wi < nw; wi += lane_count()) pw[wi] = packed_read_word(rd, wi, hasN);
       warp_sync();
       rdw = pw;
       rdlg = hasN ? 4u : 5u;

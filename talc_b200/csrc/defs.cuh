@@ -165,6 +165,20 @@ TALC_HD u32 packed_code(const u64* w, u32 idx, u32 lg) {
   const u32 sh = (~idx & ((1u << lg) - 1u)) << (6u - lg);
   return (u32)(w[idx >> lg] >> sh) & (lg == 5u ? 3u : 15u);
 }
+// The packed read: words [0, packed_read_words(len, hasN)) are filled, one more than the bases need, with zeros past
+// the read's end; a buffer of packed_read_alloc(len) words holds either layout.
+TALC_HD u32 packed_read_alloc(u32 len) { return (len + 15) / 16 + 2; }
+TALC_HD u32 packed_read_words(u32 len, bool hasN) { return hasN ? (len + 15) / 16 + 1 : (len + 31) / 32 + 1; }
+TALC_HD u64 packed_read_word(const ReadView& rd, u32 wi, bool hasN) {
+  const u32 per = hasN ? 16u : 32u, bits = hasN ? 4u : 2u;
+  u64 x = 0;
+  TALC_ROLLED
+  for (u32 j = 0; j < per; ++j) {
+    const u32 idx = wi * per + j;
+    x = (x << bits) | (u64)((idx < rd.len) ? rd.code(idx) : 0u);
+  }
+  return x;
+}
 struct RefView {
   const u64* w;  // packed read
   i32 start;

@@ -690,40 +690,56 @@ __global__ void test_align_kernel(int op, const u8* a, const u64* aoff, const u8
     vb = view_of_path(packed, vb.len);
   }
   __syncwarp();
-  i32 r0 = 0, r1 = 0, r2 = 0, r3 = 0;
-  if (op == 0) r0 = -nw_distance(va, va.len, vb, vb.len, ar, nullptr);
-  else if (op == 1) r0 = lcs_length(va, va.len, vb, vb.len, ar, nullptr);
-  else if (op == 2) r0 = overlap_score(va, va.len, vb, vb.len, ar, nullptr);
-  else if (op == 5) {  // fused distance + LCS
-    int l = 0;
-    r0 = -nw_lcs_fused(va, va.len, vb, vb.len, ar, nullptr, l, 3);
-    r1 = l;
-  } else if (op == 4) {  // raw X-drop: a = query segment, b = database segment, aux = score drop-off
-    DpStats ds;
-    ds.cells_xdrop = 0;
-    u32 er = 0, ec = 0;
-    i32 es = 0;
-    xdrop_extend(va, 0, va.len, vb, 0, vb.len, aux, er, ec, es, ar, true, &ds);
-    r0 = (i32)er;
-    r1 = (i32)ec;
-    r2 = (i32)ds.cells_xdrop;
-    r3 = es;
-  } else {
-    const SeedExt e = seed_and_extension(va, vb, aux, aux2 != 0, K, ar, true, nullptr);
-    r0 = (i32)e.ref_ext;
-    r1 = (i32)e.cand_ext;
-    r2 = e.score;
-    r3 = e.stop ? 1 : 0;
-  }
-  if (ar.overflow) r0 = INT32_MIN;
+  i32 r[4];
+  selftest_align_op(op, va, vb, aux, aux2, K, ar, r);
   if (lane == 0) {
     if (op >= 3) {
-      result[4 * i + 0] = r0;
-      result[4 * i + 1] = r1;
-      result[4 * i + 2] = r2;
-      result[4 * i + 3] = r3;
+      for (int q = 0; q < 4; ++q) result[4 * i + q] = r[q];
     } else
-      result[i] = r0;
+      result[i] = r[0];
+  }
+}
+// The same operations on the views the pipeline builds: slices of a packed read in either walk direction and trail
+// slots (selftest_view).  desc[8 * i ..] = {read, start, step, len} of side a, then of side b.  Ops 0-5: one warp per
+// pair.  Op 6: one warp per frontier of `aux` consecutive pairs -- the a side of its first pair is the reference, the b
+// sides are its trails (slots of equal length) -- scored by overlap_score_frontier, one score per pair.
+__global__ void test_align_slices_kernel(int op, const u8* reads, const u64* readOff, const i32* desc, u32 n, int aux, int aux2,
+                                         u32 K, u8* arenas, u32 arenaBytes, i32* result) {
+  const u32 i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const u32 lane = threadIdx.x & 31;
+  const u32 nUnits = (op == 6) ? n / (u32)aux : n;
+  if (i >= nUnits) return;
+  Arena ar;
+  ar.init(arenas + (u64)i * arenaBytes, arenaBytes);
+  auto side = [&](u32 p, u32 s) {
+    const i32* d = desc + 8 * p + 4 * s;
+    ReadView rd;
+    rd.s = reads + readOff[d[0]];
+    rd.len = (u32)(readOff[d[0] + 1] - readOff[d[0]]);
+    return selftest_view(rd, d[1], d[2], (u32)d[3], 2 * (u64)p + s, ar);
+  };
+#if defined(__CUDA_ARCH__)  // the frontier form has no host declaration
+  if (op == 6) {
+    const u32 g = (u32)aux, p0 = i * g;
+    const SeqView ref = side(p0, 0);
+    const u64** tw = (const u64**)ar.alloc(g * 8);
+    for (u32 j = 0; tw && j < g; ++j) tw[j] = side(p0 + j, 1).w;
+    const bool ok = !ar.overflow &&
+                    overlap_score_frontier(ref, ref.len, (u32)desc[8 * p0 + 7], g, [&](u32 j) { return tw[j]; },
+                                           [&](u32 j, int s) { if (lane == 0) result[p0 + j] = s; }, ar, nullptr);
+    if (!ok && lane == 0)
+      for (u32 j = 0; j < g; ++j) result[p0 + j] = INT32_MIN;
+    return;
+  }
+#endif
+  const SeqView va = side(i, 0), vb = side(i, 1);
+  i32 r[4] = {INT32_MIN, 0, 0, 0};
+  if (!ar.overflow) selftest_align_op(op, va, vb, aux, aux2, K, ar, r);
+  if (lane == 0) {
+    if (op >= 3) {
+      for (int q = 0; q < 4; ++q) result[4 * i + q] = r[q];
+    } else
+      result[i] = r[0];
   }
 }
 __global__ void test_sort_kernel(const i64* keys, u32 n, u32* perm, void* scratchKeys) {
@@ -2058,6 +2074,52 @@ int talc_test_align(talc_ctx* c, int op, const uint8_t* a, const uint64_t* aOff,
   CUDA_TRY(c, cudaMemcpyAsync(result, dR, rn * 4, cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   cudaFree(dA); cudaFree(dB); cudaFree(dAo); cudaFree(dBo); cudaFree(dAr); cudaFree(dR);
+  return TALC_OK;
+}
+
+int talc_test_align_slices(talc_ctx* c, int op, const uint8_t* reads, const uint64_t* readOff, uint32_t nReads,
+                           const int32_t* desc, uint32_t n, int aux, int aux2, int32_t* result) {
+  if (!c || !n || !reads || !readOff || !desc || !result || op < 0 || op > 6) return TALC_ERR_ARG;
+  if (op == 6 && (aux < 1 || n % (u32)aux)) { c->err = "op 6 scores frontiers of aux >= 1 pairs each"; return TALC_ERR_ARG; }
+  for (u32 i = 0; i < n; ++i) {
+    for (u32 s = 0; s < 2; ++s) {
+      const i32* d = desc + 8 * i + 4 * s;
+      const i64 rd = d[0], start = d[1], step = d[2], len = d[3];
+      const i64 rl = (rd >= 0 && rd < (i64)nReads) ? (i64)(readOff[rd + 1] - readOff[rd]) : -1;
+      bool ok = rl >= 0 && rl <= (1 << 20) && len >= 0 && step >= -1 && step <= 1;
+      if (ok && step == 0) {
+        ok = start >= 0 && start + len <= rl;
+        for (i64 j = 0; ok && j < len; ++j) ok = base_code(reads[readOff[rd] + start + j]) < 4;
+      } else if (ok && len > 0) {
+        ok = start >= 0 && start < rl && start + (len - 1) * step >= 0 && start + (len - 1) * step < rl;
+      } else if (ok) {
+        ok = start >= 0 && start <= rl;
+      }
+      if (op == 6 && ok && s == 1) ok = step == 0 && len == desc[8 * (i - i % (u32)aux) + 7];
+      if (!ok) { c->err = "slice outside its read, a step other than -1, 0, +1, or an N in a trail"; return TALC_ERR_ARG; }
+    }
+  }
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  const u32 arenaBytes = 2u << 20;
+  const u32 units = (op == 6) ? n / (u32)aux : n;
+  const size_t rn = (size_t)n * ((op >= 3 && op <= 5) ? 4 : 1);
+  u8 *dR, *dAr;
+  u64* dO;
+  i32 *dD, *dRes;
+  CUDA_TRY(c, cudaMalloc((void**)&dR, readOff[nReads] + 1));
+  CUDA_TRY(c, cudaMalloc((void**)&dO, (size_t)(nReads + 1) * 8));
+  CUDA_TRY(c, cudaMalloc((void**)&dD, (size_t)n * 32));
+  CUDA_TRY(c, cudaMalloc((void**)&dAr, (size_t)units * arenaBytes));
+  CUDA_TRY(c, cudaMalloc((void**)&dRes, rn * 4));
+  CUDA_TRY(c, cudaMemcpyAsync(dR, reads, readOff[nReads], cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(c, cudaMemcpyAsync(dO, readOff, (size_t)(nReads + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(c, cudaMemcpyAsync(dD, desc, (size_t)n * 32, cudaMemcpyHostToDevice, c->stream));
+  test_align_slices_kernel<<<(units + 3) / 4, 128, 0, c->stream>>>(op, dR, dO, dD, n, aux, aux2, c->params.K, dAr, arenaBytes,
+                                                                  dRes);
+  CUDA_TRY(c, cudaGetLastError());
+  CUDA_TRY(c, cudaMemcpyAsync(result, dRes, rn * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  cudaFree(dR); cudaFree(dO); cudaFree(dD); cudaFree(dAr); cudaFree(dRes);
   return TALC_OK;
 }
 

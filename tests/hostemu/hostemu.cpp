@@ -789,6 +789,29 @@ void emu_seed_extend(const char* reference, const char* candidate, int xdrop, in
   SeedExt e = seed_and_extension(bytes_view(reference, rn), bytes_view(candidate, cn), xdrop, right != 0, K, A, true, nullptr);
   *ref_ext = e.ref_ext; *cand_ext = e.cand_ext; *score = e.score; *stop = e.stop ? 1 : 0;
 }
+// talc_test_align_slices on the host: the same views and the same dispatch, with the scalar forms of the primitives
+// (ops 0-5; result layout as there).  Returns -1 for an op it does not run.
+int emu_align_slices(int op, const uint8_t* reads, const uint64_t* read_off, const int32_t* desc, uint32_t n, int aux,
+                     int aux2, uint32_t K, int32_t* result) {
+  if (op < 0 || op > 5) return -1;
+  std::vector<u8> ar(1 << 22);
+  for (u32 i = 0; i < n; ++i) {
+    Arena A; A.init(ar.data(), (u32)ar.size());
+    SeqView v[2];
+    for (u32 s = 0; s < 2; ++s) {
+      const int32_t* d = desc + 8 * i + 4 * s;
+      ReadView rd;
+      rd.s = reads + read_off[d[0]];
+      rd.len = (u32)(read_off[d[0] + 1] - read_off[d[0]]);
+      v[s] = selftest_view(rd, d[1], d[2], (u32)d[3], 2 * (u64)i + s, A);
+    }
+    i32 r[4] = {INT32_MIN, 0, 0, 0};
+    if (!A.overflow) selftest_align_op(op, v[0], v[1], aux, aux2, K, A, r);
+    if (op >= 3) memcpy(result + 4 * i, r, sizeof(r));
+    else result[i] = r[0];
+  }
+  return 0;
+}
 void emu_std_sort_perm(const int64_t* keys, uint32_t n, uint32_t* perm) {
   for (u32 i = 0; i < n; ++i) perm[i] = i;
   std_sort(perm, perm + n, [keys](const u32& a, const u32& b) { return keys[a] < keys[b]; });

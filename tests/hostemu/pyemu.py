@@ -61,6 +61,8 @@ def lib():
         L.emu_xdrop_lv_mode.argtypes = [C.c_int]
         L.emu_seed_extend.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_uint32, C.POINTER(C.c_int32),
                                       C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.emu_align_slices.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int,
+                                       C.c_uint32, C.c_void_p]
         L.emu_std_sort_perm.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         L.emu_tag_next_nodes.argtypes = [C.POINTER(EmuParams), C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_void_p,
                                          C.c_void_p]
@@ -108,6 +110,20 @@ class EmuTable:
         if rc != 0:
             raise RuntimeError("emu output buffer too small")
         return out[: int(ooff[-1])], ooff, status[:n], dict(zip(COUNTER_NAMES, [int(x) for x in ctr]))
+
+
+def align_slices(op: int, reads, desc, aux: int = 0, aux2: int = 0, k: int = 21) -> np.ndarray:
+    """emu_align_slices: talc_test_align_slices (ops 0-5) with the scalar forms, same arguments and result layout."""
+    off = np.zeros(len(reads) + 1, dtype=np.uint64)
+    off[1:] = np.cumsum([len(r) for r in reads])
+    data = np.frombuffer(b"".join(reads) + b"\0", dtype=np.uint8).copy()
+    desc = np.ascontiguousarray(desc, dtype=np.int32).reshape(-1, 8)
+    n = len(desc)
+    wide = 3 <= op <= 5
+    res = np.zeros(n * (4 if wide else 1), dtype=np.int32)
+    if lib().emu_align_slices(op, _ptr(data), _ptr(off), _ptr(desc), n, aux, aux2, k, _ptr(res)) != 0:
+        raise ValueError("op %d is not emulated" % op)
+    return res.reshape(n, 4) if wide else res
 
 
 def correct_interleaved(table: EmuTable, reads, offsets, arena_bytes=1 << 20):
