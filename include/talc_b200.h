@@ -13,6 +13,8 @@
  *          (Read.cpp:174-386, Explorer.cpp, Trail.cpp, Trajectory.cpp)
  *   talc_ctx_set_reverse
  *       <- if (reverse) reverseComplement(seq) before, and of the corrected read after, the above   main.cpp:253,285-286
+ *   talc_ctx_set_strand / talc_orient_batch / talc_last_strands / talc_stream_strands
+ *       <- not in the reference: the strand chosen per read (--strand auto), for inputs of both orientations
  *   talc_coverage_batch
  *       <- getLRCountsInSR(seq, K, SR_DBG, ..)                                     Jellyfish.cpp:471-496
  *   talc_table_lookup
@@ -128,6 +130,30 @@ int talc_ctx_set_exec(talc_ctx* ctx, uint32_t split_walk, uint32_t read_contexts
  * batches pending.  Default 0.                                                                                     */
 int talc_ctx_set_reverse(talc_ctx* ctx, int reverse);
 
+/* Strand mode of the correction (not in the reference; talc --strand).  A k-mer table counted from short reads holds
+ * one strand, so a long read finds solid k-mers only on that strand; cDNA long-read libraries mix sense and antisense
+ * reads.
+ *   TALC_STRAND_FORWARD (default)  every read as it is
+ *   TALC_STRAND_REVERSE            talc_ctx_set_reverse(ctx, 1): every read on the opposite strand
+ *   TALC_STRAND_AUTO               each read on the strand where it finds more of the table.  For each read, found_fwd
+ *                                  = its K-mer windows without N whose k-mer is in the table (count != 0), found_rc =
+ *                                  the same for its Dna5 reverse complement (as talc_ctx_set_reverse builds it); strand
+ *                                  1 (antisense) iff found_rc > found_fwd, ties (reads shorter than K, all-N reads,
+ *                                  reverse palindromes) stay 0.  A strand-1 read is corrected exactly as reverse mode
+ *                                  corrects it; EVERY read comes back in its input orientation: a corrected strand-1 read
+ *                                  as the reverse complement of its correction, any other strand-1 read as its
+ *                                  Dna5-normalised input (unlike reverse mode's Q24), strand-0 reads as in forward mode.
+ *                                  Status, offsets and the algorithmic counters are those of forward mode on the batch
+ *                                  with every strand-1 read reverse-complemented; the orientation probes are not counted
+ *                                  in lookups_seg.  Coverage (talc_coverage_batch) and the read_stats of the stream
+ *                                  describe each read on its chosen strand.
+ * The same rules as talc_ctx_set_reverse: set on a context, not on a lane (TALC_ERR_ARG; a lane follows its parent),
+ * not while a stream on the context has batches pending.  Another mode value is TALC_ERR_ARG.                     */
+#define TALC_STRAND_FORWARD 0
+#define TALC_STRAND_REVERSE 1
+#define TALC_STRAND_AUTO 2
+int talc_ctx_set_strand(talc_ctx* ctx, int mode);
+
 /* ---- k-mer table (main.cpp:231-232) -------------------------------------------------------- */
 /* Jellyfish `dump -c` text (KMER<ws>COUNT per line), optional junction dump (NULL = none).      */
 int talc_table_load_dump(talc_ctx* ctx, const char* dump_path, const char* junction_path, uint64_t* n_lines,
@@ -205,6 +231,15 @@ int talc_correct_batch_device(talc_ctx* ctx, const uint8_t* d_bases, const uint6
 /* Per-read coverage vectors only (Read::reCoverage): counts[sum(max(0,len-K+1))], host buffers.   */
 int talc_coverage_batch(talc_ctx* ctx, const uint8_t* bases, const uint64_t* offsets, uint32_t n_reads,
                         uint32_t* counts, uint64_t counts_capacity);
+/* The decision of TALC_STRAND_AUTO without correcting, in any strand mode (e.g. to orient reads for other tools).
+ * Host buffers: offsets[n_reads+1] with offsets[0] == 0, strand[n_reads] in {0,1}; found_fwd[n_reads] and
+ * found_rc[n_reads] may be NULL.                                                                                  */
+int talc_orient_batch(talc_ctx* ctx, const uint8_t* bases, const uint64_t* offsets, uint32_t n_reads, uint8_t* strand,
+                      uint32_t* found_fwd, uint32_t* found_rc);
+/* The strands (0 / 1) of the first n reads of the last batch corrected through this context (talc_correct_batch,
+ * talc_correct_batch_device, or a stream's batch on this very context or lane); all 0 for a batch corrected in forward
+ * or reverse mode.  dst is a host or a device pointer.  TALC_ERR_ARG when n exceeds that batch.                     */
+int talc_last_strands(talc_ctx* ctx, uint8_t* dst, uint32_t n);
 
 /* ---- streamed correction (replaces loadSeqData / outputSeqData holding every read: main.cpp:219,310, io.cpp:26-75) ----
  * Batches of reads pass through one context with the host-to-device copy of batch i+1, the kernels of batch i, the
@@ -228,6 +263,10 @@ int talc_stream_submit(talc_stream* s, const uint8_t* bases, const uint64_t* off
 int talc_stream_next(talc_stream* s, const uint8_t** out, const uint64_t** out_offsets, const uint8_t** status,
                      uint32_t* n_reads, const uint32_t** read_stats, talc_counters* counters);
 uint64_t talc_stream_pending(talc_stream* s);   /* batches submitted and not yet fetched */
+/* strand[n_reads] (see TALC_STRAND_AUTO) of the batch last returned by talc_stream_next, in pinned host memory owned by
+ * the stream and valid until the following next / close; NULL for a batch corrected in forward or reverse mode.
+ * TALC_ERR_ARG before the first next.                                                                              */
+int talc_stream_strands(talc_stream* s, const uint8_t** strand);
 const char* talc_stream_last_error(talc_stream* s);
 void talc_stream_close(talc_stream* s);
 

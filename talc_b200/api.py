@@ -36,6 +36,7 @@ class TalcCounters(C.Structure):
 
 STATUS_MESSAGES = {1: "No solid kmer could be found.", 2: "Unable to define convenient structure."}
 STATUS_RESOURCE = 4  # TALC_READ_RESOURCE: passed through uncorrected, not a reference status
+STRAND_MODES = {"forward": 0, "reverse": 1, "auto": 2}  # TALC_STRAND_FORWARD / _REVERSE / _AUTO
 
 _lib = None
 
@@ -56,6 +57,10 @@ def lib():
         L.talc_ctx_set_scratch.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32]
         L.talc_ctx_set_exec.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32]
         L.talc_ctx_set_reverse.argtypes = [vp, C.c_int]
+        L.talc_ctx_set_strand.argtypes = [vp, C.c_int]
+        L.talc_orient_batch.argtypes = [vp, vp, vp, C.c_uint32, vp, vp, vp]
+        L.talc_last_strands.argtypes = [vp, vp, C.c_uint32]
+        L.talc_stream_strands.argtypes = [vp, C.POINTER(vp)]
         L.talc_table_load_dump.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_table_load_dump_host.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_dump_write_packed.argtypes = [C.c_char_p, vp, vp, C.c_uint64, C.c_uint32]
@@ -159,6 +164,36 @@ class Talc:
         """talc --reverse: reads are corrected on the opposite strand; corrected reads come back in their input
         orientation, all others reverse-complemented (talc_ctx_set_reverse).  Raises on a lane."""
         self._check(lib().talc_ctx_set_reverse(self.h, 1 if reverse else 0), "talc_ctx_set_reverse")
+
+    def set_strand(self, mode):
+        """talc --strand: "forward", "reverse" (= set_reverse(True)) or "auto" (each read corrected on the strand where
+        it finds more of the table, every read returned in its input orientation), or 0 / 1 / 2 (talc_ctx_set_strand).
+        Raises on a lane."""
+        m = STRAND_MODES[mode] if isinstance(mode, str) else int(mode)
+        self._check(lib().talc_ctx_set_strand(self.h, m), "talc_ctx_set_strand")
+
+    def orient(self, reads: np.ndarray, offsets: np.ndarray):
+        """The auto-mode strand decision without correcting, in any mode (talc_orient_batch):
+        (strand uint8[n] in {0,1}, found_fwd uint32[n], found_rc uint32[n])."""
+        reads = np.ascontiguousarray(reads, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = len(offsets) - 1
+        strand = np.zeros(max(n, 1), dtype=np.uint8)
+        ff = np.zeros(max(n, 1), dtype=np.uint32)
+        fr = np.zeros(max(n, 1), dtype=np.uint32)
+        self._check(lib().talc_orient_batch(self.h, _ptr(reads), _ptr(offsets), n, _ptr(strand), _ptr(ff), _ptr(fr)),
+                    "talc_orient_batch")
+        return strand[:n], ff[:n], fr[:n]
+
+    def last_strands(self, n: int, out=None):
+        """Strands of the first n reads of the last batch corrected through this context (talc_last_strands); all 0
+        unless it ran in auto mode.  out: a uint8 torch tensor on the context's device to fill instead of a new array."""
+        if out is not None:
+            self._check(lib().talc_last_strands(self.h, C.c_void_p(out.data_ptr()), n), "talc_last_strands")
+            return out
+        dst = np.zeros(max(n, 1), dtype=np.uint8)
+        self._check(lib().talc_last_strands(self.h, _ptr(dst), n), "talc_last_strands")
+        return dst[:n]
 
     # ---- table
     def load_dump(self, dump: str, junctions: Optional[str] = None):
@@ -370,6 +405,7 @@ class TalcStream:
     def __init__(self, ctx: Talc, read_stats: bool = False):
         self.ctx = ctx
         self.h = C.c_void_p()
+        self._n = 0
         ctx._check(lib().talc_stream_open(ctx.h, 1 if read_stats else 0, C.byref(self.h)), "talc_stream_open")
 
     def _check(self, rc, what):
@@ -406,7 +442,19 @@ class TalcStream:
         if copy:
             out, off, st = out.copy(), off.copy(), st.copy()
             stats = stats.copy() if stats is not None else None
+        self._n = nn
         return out, off, st, stats, ctr.as_dict()
+
+    def strands(self, copy: bool = True):
+        """uint8[n] strands of the batch last returned by next() (talc_stream_strands), None unless it ran in auto
+        mode; a view into the stream's pinned buffer unless copy=True."""
+        p = C.c_void_p()
+        self._check(lib().talc_stream_strands(self.h, C.byref(p)), "talc_stream_strands")
+        if not p.value:
+            return None
+        nn = self._n
+        st = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint8)), shape=(max(nn, 1),))[:nn]
+        return st.copy() if copy else st
 
     def close(self):
         if self.h:

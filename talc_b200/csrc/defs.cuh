@@ -109,7 +109,40 @@ inline bool warp_any(bool v) { return v; }
 #endif
 TALC_HD u8 code_char(u32 code) { return (u8)("ACGTN"[code]); }
 
+// Dna5 conversion followed by SeqAn's reverseComplement, one base: ACGT in either case -> complement, anything else -> N
+TALC_HD u8 dna5_complement(u8 c) {
+  switch (c) {
+    case 'A': case 'a': return 'T';
+    case 'C': case 'c': return 'G';
+    case 'G': case 'g': return 'C';
+    case 'T': case 't': return 'A';
+    default: return 'N';
+  }
+}
+
 TALC_HD u64 kmer_mask(u32 K) { return (K >= 32) ? ~0ull : ((1ull << (2 * K)) - 1ull); }
+
+// --strand auto.  A read's k-mers and the k-mers of its reverse complement (dna5_complement, read backwards) rolled
+// together, one byte per base, K <= 31.  After base p + K - 1 has been pushed, `fwd` is the window of the read at p and
+// `rc` the window of the reverse complement at len - K - p, i.e. the reverse complement of `fwd`; a window holds no N
+// when the matching run counter is >= K.  The two runs differ only on 'U', which base_code reads as T and
+// dna5_complement turns into N.
+struct StrandRoll {
+  u64 fwd, rc;
+  u32 runF, runR;  // bases since the last N of the read / of its reverse complement
+};
+TALC_HD StrandRoll strand_roll_start() { return StrandRoll{0ull, 0ull, 0u, 0u}; }
+TALC_HD void strand_roll_push(StrandRoll& s, u8 ch, u32 K) {
+  const u32 c = base_code(ch);
+  const bool nR = (c > 3u) | (((u32)ch | 0x20u) == (u32)'u');
+  s.runF = (c > 3u) ? 0u : s.runF + 1u;
+  s.runR = nR ? 0u : s.runR + 1u;
+  s.fwd = ((s.fwd << 2) | (u64)(c & 3u)) & kmer_mask(K);
+  s.rc = (s.rc >> 2) | ((u64)(3u - (c & 3u)) << (2 * (K - 1)));
+}
+// found_fwd / found_rc: windows without N found in the table on either strand.  Antisense (1) only on a strict
+// majority: ties -- reads shorter than K, all-N reads, reverse palindromes -- stay forward (0).
+TALC_HD u32 strand_decide(u32 found_fwd, u32 found_rc) { return found_rc > found_fwd ? 1u : 0u; }
 
 // k-mers are 2-bit packed with the first base in the most significant position.
 // Successors (utils.cpp:370-387): RIGHT x[1..]+b ; LEFT b+x[..K-2]

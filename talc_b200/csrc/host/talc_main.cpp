@@ -1,7 +1,7 @@
 // talc_main.cpp -- the drop-in `talc` command line on top of libtalc_b200.so.
 //
 // Same interface and the same output files as the reference program (main.cpp:83-325):
-//   talc <reads.fa|fq> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse] [tunables]
+//   talc <reads.fa|fq> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse | --strand forward|reverse|auto] [tunables]
 //   <prefix>.config.txt (Settings.cpp:160-185)   <prefix>.stats_basics.txt header (Read.cpp:394-415)
 //   <prefix>.log, appended, one line per failed read (io.cpp:105-111; messages main.cpp:290,294)
 //   <prefix>.fa, every read in input order, 70 columns (main.cpp:310, io.cpp:50-75)
@@ -15,7 +15,8 @@
 // records in input order.  Host memory is bounded by the batches in flight, whatever the size of the input.
 // Extensions: --gpus N deals the batches round-robin over N devices (table replicated with one NCCL broadcast issued
 // by the library, or with peer copies: --replicate peer), --tableCache <file>, --readStats (the per-read rows of Read.cpp:418-433 the reference left disabled
-// at main.cpp:305).
+// at main.cpp:305), --strand forward|reverse|auto (reverse = --reverse; auto chooses each read's strand and also
+// writes <prefix>.strand.txt, one "<id>\t+" or "<id>\t-" line per read in input order).
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -37,9 +38,9 @@
 #include "talc_b200.h"
 
 struct Cli {
-  std::string reads, dump, junctions, out = "out", queryMode = "memory", tableCache, replicate = "nccl";
+  std::string reads, dump, junctions, out = "out", queryMode = "memory", tableCache, replicate = "nccl", strand;
   bool useJunctions = false, reverse = false, readStats = false;
-  int threads = 1, gpus = 1;
+  int threads = 1, gpus = 1, strandMode = TALC_STRAND_FORWARD;
   long batchReads = 131072, batchBases = 256l << 20;
   talc_params p;
   bool haveK = false, haveSR = false;
@@ -85,6 +86,7 @@ static int parse(int argc, const char** argv, Cli& c) {
     else if (a == "-t" || a == "--num_threads") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.threads = (int)n; }
     else if (a == "-DEBUG_MODE" || a == "--DEBUG_MODE") { if (!val(v)) return 1; }
     else if (a == "-rev" || a == "--reverse") { c.reverse = true; }
+    else if (a == "--strand") { if (!val(c.strand) || (c.strand != "forward" && c.strand != "reverse" && c.strand != "auto")) return 1; }
     else if (a == "--readStats") { c.readStats = true; }
     else if (a == "--batch-reads") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.batchReads = n; }
     else if (a == "--batch-bases") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.batchBases = n; }
@@ -94,6 +96,8 @@ static int parse(int argc, const char** argv, Cli& c) {
     else pos.push_back(a);
   }
   if (pos.size() != 1 || !c.haveK || !c.haveSR) return 1;
+  if (c.reverse && !c.strand.empty() && c.strand != "reverse") return 1;  // --reverse is --strand reverse
+  c.strandMode = (c.reverse || c.strand == "reverse") ? TALC_STRAND_REVERSE : c.strand == "auto" ? TALC_STRAND_AUTO : TALC_STRAND_FORWARD;
   if (c.queryMode != "memory") { std::cerr << "talc: only query mode 'memory' is supported\n"; return 1; }
   c.reads = pos[0];
   return 0;
@@ -133,7 +137,7 @@ int main(int argc, const char** argv) {
   Cli cli;
   const int pr = parse(argc, argv, cli);
   if (pr == 2) {
-    std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse] [--gpus <N>] [--tableCache <file>]"
+    std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse | --strand forward|reverse|auto] [--gpus <N>] [--tableCache <file>]"
                  " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer]\n";
     return 0;
   }
@@ -164,8 +168,8 @@ int main(int argc, const char** argv) {
       std::cerr << "talc: cannot create a GPU context on device " << g << ": " << talc_last_error(nullptr) << "\n";
       return 2;
     }
-    // --reverse (main.cpp:253,285-286): the long reads only; the stream's lanes follow their context
-    if (cli.reverse && talc_ctx_set_reverse(ctx[g], 1) != 0) {
+    // --reverse (main.cpp:253,285-286) / --strand: the long reads only; the stream's lanes follow their context
+    if (cli.strandMode != TALC_STRAND_FORWARD && talc_ctx_set_strand(ctx[g], cli.strandMode) != 0) {
       std::cerr << "talc: " << talc_last_error(ctx[g]) << "\n";
       return 2;
     }
@@ -248,7 +252,8 @@ int main(int argc, const char** argv) {
   uint64_t nReads = 0, nResource = 0;
   double sWait = 0, sFormat = 0, sWrite = 0, sParse = 0, sSubmit = 0;  // where the threads of this phase spent their time
   std::thread writer([&]() {
-    std::ofstream lg, st;
+    std::ofstream lg, st, sf;
+    if (cli.strandMode == TALC_STRAND_AUTO) sf.open(cli.out + ".strand.txt", std::ios_base::trunc);
     std::vector<std::string> parts;
     while (auto b = idq.pop()) {
       talc_stream* s = streams[b->seq % cli.gpus];
@@ -264,6 +269,16 @@ int main(int argc, const char** argv) {
         writerRc = 2;
         while (idq.pop()) {}  // keep draining so that the reader does not block for ever
         return;
+      }
+      if (sf.is_open()) {
+        const uint8_t* strand = nullptr;
+        if (talc_stream_strands(s, &strand) != 0 || (n && !strand)) {
+          std::cerr << "talc: no strands for a batch on device " << (b->seq % cli.gpus) << "\n";
+          writerRc = 2;
+          while (idq.pop()) {}
+          return;
+        }
+        for (uint32_t r = 0; r < n; ++r) sf << b->ids[r] << (strand[r] ? "\t-\n" : "\t+\n");
       }
       for (uint32_t r = 0; r < n; ++r) {
         const uint8_t v = status[r];

@@ -59,8 +59,9 @@ struct PinBuf {
 };
 
 struct StreamSlot {
-  PinBuf hBases, hOffs, hOut, hOutOffs, hStatus, hStats;
-  DevBuf dBases, dOffs, dOut, dOutOffs, dStatus, dStats;
+  PinBuf hBases, hOffs, hOut, hOutOffs, hStatus, hStats, hStrand;
+  DevBuf dBases, dOffs, dOut, dOutOffs, dStatus, dStats, dStrand;
+  bool strandAuto = false;  // the batch ran in TALC_STRAND_AUTO: hStrand holds its strands
   cudaEvent_t h2dDone = nullptr, d2hDone = nullptr;
   u32 n = 0;
   u64 totalBases = 0;
@@ -106,10 +107,16 @@ static void stream_worker(talc_stream* s, int w) {
     int rc = TALC_OK;
     cudaError_t e = cudaStreamWaitEvent(c->stream, sl->h2dDone, 0);
     if (e != cudaSuccess) rc = TALC_ERR_CUDA;
+    const bool strandAuto = c->parent ? c->parent->strand == TALC_STRAND_AUTO : c->strand == TALC_STRAND_AUTO;
+    if (rc == TALC_OK && strandAuto && (sl->dStrand.reserve(sl->n + 1) != cudaSuccess || sl->hStrand.reserve(sl->n + 1) != cudaSuccess)) {
+      rc = TALC_ERR_CUDA;
+      c->err = "out of pinned host or device memory for the strands of a batch";
+    }
     if (rc == TALC_OK)
       rc = correct_batch_device_impl(c, (const u8*)sl->dBases.p, (const u64*)sl->dOffs.p, sl->n, sl->totalBases, (u8*)sl->dOut.p,
                                      sl->dOut.cap, (u64*)sl->dOutOffs.p, (u8*)sl->dStatus.p, &sl->ctr,
-                                     s->wantStats ? (u32*)sl->dStats.p : nullptr);
+                                     s->wantStats ? (u32*)sl->dStats.p : nullptr, strandAuto ? (u8*)sl->dStrand.p : nullptr);
+    sl->strandAuto = rc == TALC_OK && c->lastAuto;
     if (rc == TALC_OK) {
       // this lane's compute stream is idle here (the call above ends with a synchronize): results leave on the
       // copy-out stream while the next batch computes
@@ -121,6 +128,8 @@ static void stream_worker(talc_stream* s, int w) {
         if (ok && totalOut) ok = cudaMemcpyAsync(sl->hOut.p, sl->dOut.p, totalOut, cudaMemcpyDeviceToHost, s->copyOut) == cudaSuccess;
         if (ok && s->wantStats)
           ok = cudaMemcpyAsync(sl->hStats.p, sl->dStats.p, (size_t)sl->n * 8, cudaMemcpyDeviceToHost, s->copyOut) == cudaSuccess;
+        if (ok && sl->strandAuto)
+          ok = cudaMemcpyAsync(sl->hStrand.p, sl->dStrand.p, sl->n, cudaMemcpyDeviceToHost, s->copyOut) == cudaSuccess;
       }
       ok = ok && cudaEventRecord(sl->d2hDone, s->copyOut) == cudaSuccess;
       if (!ok) { rc = TALC_ERR_CUDA; sl->err = "device-to-host copy of a batch failed"; }
@@ -271,6 +280,16 @@ int talc_stream_next(talc_stream* s, const uint8_t** out, const uint64_t** out_o
   return TALC_OK;
 }
 
+// the slot handed out by the last talc_stream_next stays in state 3 until the following call
+int talc_stream_strands(talc_stream* s, const uint8_t** strand) {
+  if (!s || !strand) return TALC_ERR_ARG;
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (s->seqFetch == 0) { s->err = "talc_stream_strands: no batch returned yet"; return TALC_ERR_ARG; }
+  const StreamSlot* sl = &s->slot[(s->seqFetch - 1) % s->kSlots];
+  *strand = (sl->state == 3 && sl->rc == TALC_OK && sl->strandAuto) ? (const uint8_t*)sl->hStrand.p : nullptr;
+  return TALC_OK;
+}
+
 const char* talc_stream_last_error(talc_stream* s) { return s ? s->err.c_str() : ""; }
 
 void talc_stream_close(talc_stream* s) {
@@ -287,9 +306,9 @@ void talc_stream_close(talc_stream* s) {
   cudaStreamSynchronize(s->copyIn);
   cudaStreamSynchronize(s->copyOut);
   for (auto& sl : s->slot) {
-    PinBuf* hb[] = {&sl.hBases, &sl.hOffs, &sl.hOut, &sl.hOutOffs, &sl.hStatus, &sl.hStats};
+    PinBuf* hb[] = {&sl.hBases, &sl.hOffs, &sl.hOut, &sl.hOutOffs, &sl.hStatus, &sl.hStats, &sl.hStrand};
     for (PinBuf* b : hb) b->release();
-    DevBuf* db[] = {&sl.dBases, &sl.dOffs, &sl.dOut, &sl.dOutOffs, &sl.dStatus, &sl.dStats};
+    DevBuf* db[] = {&sl.dBases, &sl.dOffs, &sl.dOut, &sl.dOutOffs, &sl.dStatus, &sl.dStats, &sl.dStrand};
     for (DevBuf* b : db) b->release();
     if (sl.h2dDone) cudaEventDestroy(sl.h2dDone);
     if (sl.d2hDone) cudaEventDestroy(sl.d2hDone);

@@ -8,6 +8,8 @@
 //   correct_kernel                                                      segmentation + graph search + scoring
 //   gather_kernel                                                       corrected reads back into input order
 //   revcomp_reads_kernel                                                --reverse: every read reverse-complemented first
+//   orient_kernel                                                       --strand auto: both strands probed, each read's
+//                                                                       strand chosen, in place of coverage_kernel
 // Grid sizes are multiples of the SM count; per-thread scratch lives in HBM (180 GB makes that cheap).
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -264,6 +266,100 @@ __global__ void __launch_bounds__(256) coverage_kernel(TableView tv, u32 K, cons
       } else {
         for (u32 q = 0; q < 4 && p0 + q < C; ++q) out[p0 + q] = cnt[q];
       }
+    }
+  }
+}
+
+// --strand auto: coverage of both strands and the choice between them, in place of coverage_kernel (and of
+// revcomp_reads_kernel).  The layout of coverage_kernel: one warp per read, four windows per lane; each lane rolls
+// the forward k-mers and their reverse complements together (strand_roll_push, K+3 byte loads) and issues the home-
+// sector fetches of both strands at once, up to eight 256-bit loads in flight.  Forward counts go to cov in read
+// order, reverse-complement counts to covRc in the order of the reverse-complemented read.  The warp then counts the
+// windows found on each strand, decides (strand_decide) and writes the read as it will be corrected into `oriented`
+// (same offsets): a plain copy on strand 0, the Dna5 reverse complement on strand 1, whose coverage it moves into cov.
+// foundFwd / foundRc may be null.
+__global__ void __launch_bounds__(256) orient_kernel(TableView tv, u32 K, const u8* __restrict__ bases,
+                                                     const u64* __restrict__ offs, const u64* __restrict__ kmerOff, u32 n,
+                                                     u32* __restrict__ cov, u32* __restrict__ covRc, u8* __restrict__ oriented,
+                                                     u8* __restrict__ strand, u32* __restrict__ foundFwd,
+                                                     u32* __restrict__ foundRc) {
+  const u32 lane = threadIdx.x & 31;
+  const u32 warpsPerBlock = blockDim.x >> 5;
+  for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
+    const u64 o = offs[r];
+    const u32 len = (u32)(offs[r + 1] - o);
+    const u32 C = len >= K ? len - K + 1 : 0;
+    const u8* s = bases + o;
+    u32* out = cov + kmerOff[r];
+    u32* outR = covRc + kmerOff[r];
+    u32 nF = 0, nR = 0;
+    for (u32 base = 0; base < C; base += 128) {
+      const u32 p0 = base + lane * 4;
+      if (p0 >= C) continue;
+      StrandRoll st = strand_roll_start();
+      for (u32 j = 0; j < K; ++j) strand_roll_push(st, __ldg(s + p0 + j), K);
+      u64 kf[4], kr[4];
+      u32 okF = 0, okR = 0;
+#pragma unroll
+      for (u32 q = 0; q < 4; ++q) {
+        if (q > 0 && p0 + q < C) strand_roll_push(st, __ldg(s + p0 + q + K - 1), K);
+        const bool in = p0 + q < C;
+        kf[q] = st.fwd;
+        kr[q] = st.rc;
+        okF |= (in && st.runF >= K) ? (1u << q) : 0u;
+        okR |= (in && st.runR >= K) ? (1u << q) : 0u;
+      }
+      // the home sectors of both strands, all issued before any is looked at
+      Slot f0[4], f1[4], r0[4], r1[4];
+      u64 bf[4], br[4];
+#pragma unroll
+      for (u32 q = 0; q < 4; ++q) {
+        bf[q] = hash_kmer(kf[q]) & tv.mask & ~1ull;
+        br[q] = hash_kmer(kr[q]) & tv.mask & ~1ull;
+        if ((okF >> q) & 1u) load_sector(tv.slots + bf[q], f0[q], f1[q]);
+        if ((okR >> q) & 1u) load_sector(tv.slots + br[q], r0[q], r1[q]);
+      }
+      u32 cf[4] = {0, 0, 0, 0}, cr[4] = {0, 0, 0, 0};
+#pragma unroll
+      for (u32 q = 0; q < 4; ++q) {
+        u32 col;
+        if ((okF >> q) & 1u) {
+          if (sector_resolve(f0[q], f1[q], kf[q], cf[q], col) < 0) table_probe_from(tv, bf[q], kf[q], cf[q], col);
+        }
+        if ((okR >> q) & 1u) {
+          if (sector_resolve(r0[q], r1[q], kr[q], cr[q], col) < 0) table_probe_from(tv, br[q], kr[q], cr[q], col);
+        }
+        nF += cf[q] != 0;
+        nR += cr[q] != 0;
+      }
+      if (p0 + 3 < C && ((((size_t)(out + p0)) & 15) == 0)) {
+        *reinterpret_cast<uint4*>(out + p0) = make_uint4(cf[0], cf[1], cf[2], cf[3]);
+      } else {
+        for (u32 q = 0; q < 4 && p0 + q < C; ++q) out[p0 + q] = cf[q];
+      }
+      // window p of the read is window C - 1 - p of its reverse complement
+      u32* dR = outR + (C - 1 - p0);
+      if (p0 + 3 < C && ((((size_t)(dR - 3)) & 15) == 0)) {
+        *reinterpret_cast<uint4*>(dR - 3) = make_uint4(cr[3], cr[2], cr[1], cr[0]);
+      } else {
+        for (u32 q = 0; q < 4 && p0 + q < C; ++q) dR[-(i32)q] = cr[q];
+      }
+    }
+    nF = warp_sum(nF);
+    nR = warp_sum(nR);
+    const u32 sd = strand_decide(nF, nR);
+    if (lane == 0) {
+      strand[r] = (u8)sd;
+      if (foundFwd) foundFwd[r] = nF;
+      if (foundRc) foundRc[r] = nR;
+    }
+    u8* dst = oriented + o;
+    if (sd) {
+      for (u32 i = lane; i < len; i += 32) dst[i] = dna5_complement(s[len - 1 - i]);
+      __syncwarp();  // covRc of this read was written by every lane of the warp
+      for (u32 j = lane; j < C; j += 32) out[j] = outR[j];
+    } else {
+      for (u32 i = lane; i < len; i += 32) dst[i] = s[i];
     }
   }
 }
@@ -576,17 +672,6 @@ __global__ void ctx_init_kernel(ReadCtx* ctxs, u32 nCtx, u32* readyList, u32* nR
   if (i == 0) *nReady = nCtx;
 }
 
-// Dna5 conversion followed by SeqAn's reverseComplement, one base: ACGT in either case -> complement, anything else -> N
-__device__ __forceinline__ u8 dna5_complement(u8 c) {
-  switch (c) {
-    case 'A': case 'a': return 'T';
-    case 'C': case 'c': return 'G';
-    case 'G': case 'g': return 'C';
-    case 'T': case 't': return 'A';
-    default: return 'N';
-  }
-}
-
 // --reverse (main.cpp:253): every read reverse-complemented before anything else; one warp per read, same offsets
 __global__ void revcomp_reads_kernel(const u8* __restrict__ in, const u64* __restrict__ offs, u32 n, u8* __restrict__ out) {
   const u32 lane = threadIdx.x & 31;
@@ -600,19 +685,20 @@ __global__ void revcomp_reads_kernel(const u8* __restrict__ in, const u64* __res
   }
 }
 
-// corrected reads from allocation order into input order; one warp per read.  reverse (uniform per launch): a read
-// that was corrected goes back to the input's strand (main.cpp:285-286); every other read leaves as its reverse-
-// complemented input (Q24)
+// corrected reads from allocation order into input order; one warp per read.  A read is flipped back to the input's
+// strand per read: in reverse mode when it was corrected (main.cpp:285-286; every other read leaves as its reverse-
+// complemented input, Q24), in auto mode when it was corrected on the reverse strand (strand[r] == 1), whatever its status
 __global__ void gather_kernel(const u8* __restrict__ arena, const u64* __restrict__ pos, const u32* __restrict__ len,
                               const u64* __restrict__ outOff, u32 n, u8* __restrict__ out, const u8* __restrict__ status,
-                              u32 reverse) {
+                              const u8* __restrict__ strand, u32 mode) {
   const u32 lane = threadIdx.x & 31;
   const u32 warpsPerBlock = blockDim.x >> 5;
   for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
     const u8* src = arena + pos[r];
     u8* dst = out + outOff[r];
     const u32 L = len[r];
-    if (reverse && status[r] == TALC_READ_OK)
+    const bool flip = mode == TALC_STRAND_AUTO ? strand[r] != 0 : mode == TALC_STRAND_REVERSE && status[r] == TALC_READ_OK;
+    if (flip)
       for (u32 i = lane; i < L; i += 32) dst[i] = dna5_complement(src[L - 1 - i]);
     else
       for (u32 i = lane; i < L; i += 32) dst[i] = src[i];
@@ -804,12 +890,15 @@ struct talc_ctx {
   u32 walkStepCap = 48;    // steps a frontier may take per round of the walk kernel (bounds the round's tail)
   u32 pauseCycles = 200000;  // SM cycles (~100 us) a read may run per round of the control kernel
   u32 inlineInner = 6, inlineBorder = 6;
-  u32 reverse = 0;  // talc_ctx_set_reverse: the long reads are corrected on the opposite strand (rcBases)
+  u32 strand = TALC_STRAND_FORWARD;  // talc_ctx_set_strand: reverse and auto correct (some) reads on the opposite
+                                     // strand, from the oriented copy in rcBases
+  u32 lastN = 0;                     // the last batch corrected through this context (talc_last_strands):
+  bool lastAuto = false;             // its size, and whether its decisions are in `strands`
   u64 lastRounds = 0;
   double* modelTabs = nullptr;  // 3 x kModelTabN doubles
   // cached device buffers
   DevBuf bases, offs, kmerOff, nk, cov, order, sortKey, sortKeyOut, sortVal, cubTmp, arenas, outArena, outPos, outLen,
-      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases;
+      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases, covRc, strands, orientOut;
 };
 
 static const u32 kModelTabN = 16384;
@@ -933,7 +1022,8 @@ void talc_ctx_destroy(talc_ctx* c) {
   if (c->modelTabs) cudaFree(c->modelTabs);
   DevBuf* bufs[] = {&c->bases, &c->offs, &c->kmerOff, &c->nk, &c->cov, &c->order, &c->sortKey, &c->sortKeyOut, &c->sortVal,
                     &c->cubTmp, &c->arenas, &c->outArena, &c->outPos, &c->outLen, &c->outLen64, &c->status, &c->outOffs,
-                    &c->out, &c->misc, &c->overflowList, &c->readCtxs, &c->roundLists, &c->rcBases};
+                    &c->out, &c->misc, &c->overflowList, &c->readCtxs, &c->roundLists, &c->rcBases, &c->covRc,
+                    &c->strands, &c->orientOut};
   for (DevBuf* b : bufs) b->release();
   for (int i = 0; i < 8; ++i) cudaEventDestroy(c->ev[i]);
   cudaStreamDestroy(c->stream);
@@ -967,7 +1057,7 @@ static void lane_follow(talc_ctx* sh) {
   sh->pauseCycles = c->pauseCycles;
   sh->inlineInner = c->inlineInner;
   sh->inlineBorder = c->inlineBorder;
-  sh->reverse = c->reverse;
+  sh->strand = c->strand;
 }
 int talc_ctx_create_lane(talc_ctx* parent, talc_ctx** out) {
   if (!parent || !out || parent->parent) return TALC_ERR_ARG;
@@ -996,12 +1086,20 @@ int talc_ctx_set_exec(talc_ctx* c, uint32_t split_walk, uint32_t read_contexts, 
   return TALC_OK;
 }
 
-// --reverse (main.cpp:253,285-286).  A lane follows its parent; the stream's lanes read it at the start of each batch.
-int talc_ctx_set_reverse(talc_ctx* c, int reverse) {
+// --reverse (main.cpp:253,285-286) and --strand auto.  A lane follows its parent; the stream's lanes read it at the
+// start of each batch.
+int talc_ctx_set_strand(talc_ctx* c, int mode) {
   if (!c) return TALC_ERR_ARG;
   if (c->parent) { c->err = "a lane follows the strand setting of the context it was made from"; return TALC_ERR_ARG; }
-  c->reverse = reverse != 0;
+  if (mode != TALC_STRAND_FORWARD && mode != TALC_STRAND_REVERSE && mode != TALC_STRAND_AUTO) {
+    c->err = "strand mode must be TALC_STRAND_FORWARD, TALC_STRAND_REVERSE or TALC_STRAND_AUTO";
+    return TALC_ERR_ARG;
+  }
+  c->strand = (u32)mode;
   return TALC_OK;
+}
+int talc_ctx_set_reverse(talc_ctx* c, int reverse) {
+  return talc_ctx_set_strand(c, reverse ? TALC_STRAND_REVERSE : TALC_STRAND_FORWARD);
 }
 
 // ---------------------------------------------------------------------------------- table
@@ -1721,8 +1819,11 @@ static int run_pass(talc_ctx* c, CorrectArgs& A, u32 nCtx, u64* launches) {
 
 // ---------------------------------------------------------------------------------- correction
 // shared front end: k-mer offsets, length-sorted order, coverage.  d_bases/d_offs on device.  In reverse mode the reads
-// are first reverse-complemented into rcBases (same offsets) and dBases is pointed there for the rest of the batch.
-static int prepare_batch(talc_ctx* c, const u8*& dBases, const u64* dOffs, u32 n, u64 totalBases, u64& totalKmers) {
+// are first reverse-complemented into rcBases (same offsets) and dBases is pointed there for the rest of the batch.  In
+// auto mode orient_kernel writes the per-read strand to dStrand (n bytes), the oriented reads to rcBases and their
+// coverage to cov; dFound (may be null) receives found_fwd[n] then found_rc[n].
+static int prepare_batch(talc_ctx* c, const u8*& dBases, const u64* dOffs, u32 n, u64 totalBases, u64& totalKmers,
+                         u32 mode, u8* dStrand, u32* dFound) {
   const u32 K = c->params.K;
   CUDA_TRY(c, c->nk.reserve((size_t)(n + 1) * 8));
   CUDA_TRY(c, c->kmerOff.reserve((size_t)(n + 1) * 8));
@@ -1742,20 +1843,29 @@ static int prepare_batch(talc_ctx* c, const u8*& dBases, const u64* dOffs, u32 n
   CUDA_TRY(c, cub::DeviceScan::ExclusiveSum(c->cubTmp.p, tb, (u64*)c->nk.p, (u64*)c->kmerOff.p, n + 1, c->stream));
   u64 hk = 0, hEnd = 0;
   CUDA_TRY(c, cudaMemcpyAsync(&hk, (u64*)c->kmerOff.p + n, 8, cudaMemcpyDeviceToHost, c->stream));
-  if (c->reverse) CUDA_TRY(c, cudaMemcpyAsync(&hEnd, dOffs + n, 8, cudaMemcpyDeviceToHost, c->stream));
+  if (mode != TALC_STRAND_FORWARD) CUDA_TRY(c, cudaMemcpyAsync(&hEnd, dOffs + n, 8, cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   totalKmers = hk;
   CUDA_TRY(c, c->cov.reserve((size_t)(hk + 4) * 4));
   TableView tv{c->slots, c->capacity - 1};
   const int blocks = c->sms * 8;
-  if (c->reverse) {  // sized from the offsets themselves: the caller's buffer is read where they point
-    CUDA_TRY(c, c->rcBases.reserve(hEnd + 64));
+  // rcBases is sized from the offsets themselves: the caller's buffer is read where they point
+  if (mode != TALC_STRAND_FORWARD) CUDA_TRY(c, c->rcBases.reserve(hEnd + 64));
+  if (mode == TALC_STRAND_REVERSE) {
     revcomp_reads_kernel<<<blocks, 256, 0, c->stream>>>(dBases, dOffs, n, (u8*)c->rcBases.p);
     CUDA_TRY(c, cudaGetLastError());
     dBases = (const u8*)c->rcBases.p;
   }
   CUDA_TRY(c, cudaEventRecord(c->ev[1], c->stream));
-  coverage_kernel<<<blocks, 256, 0, c->stream>>>(tv, K, dBases, dOffs, (const u64*)c->kmerOff.p, n, (u32*)c->cov.p);
+  if (mode == TALC_STRAND_AUTO) {
+    CUDA_TRY(c, c->covRc.reserve((size_t)(hk + 4) * 4));
+    orient_kernel<<<blocks, 256, 0, c->stream>>>(tv, K, dBases, dOffs, (const u64*)c->kmerOff.p, n, (u32*)c->cov.p,
+                                                 (u32*)c->covRc.p, (u8*)c->rcBases.p, dStrand, dFound,
+                                                 dFound ? dFound + n : nullptr);
+    dBases = (const u8*)c->rcBases.p;
+  } else {
+    coverage_kernel<<<blocks, 256, 0, c->stream>>>(tv, K, dBases, dOffs, (const u64*)c->kmerOff.p, n, (u32*)c->cov.p);
+  }
   CUDA_TRY(c, cudaGetLastError());
   CUDA_TRY(c, cudaEventRecord(c->ev[2], c->stream));
   // processing order of the correction kernel: estimated cost, descending
@@ -1771,28 +1881,35 @@ static int prepare_batch(talc_ctx* c, const u8*& dBases, const u64* dOffs, u32 n
 
 static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const uint64_t* dOffs, uint32_t n, uint64_t totalBases,
                                      uint8_t* dOut, uint64_t outCapacity, uint64_t* dOutOffs, uint8_t* dStatus,
-                                     talc_counters* counters, u32* dReadStats);
+                                     talc_counters* counters, u32* dReadStats, u8* dStrandOut);
 int talc_correct_batch_device(talc_ctx* c, const uint8_t* dBases, const uint64_t* dOffs, uint32_t n, uint64_t totalBases,
                               uint8_t* dOut, uint64_t outCapacity, uint64_t* dOutOffs, uint8_t* dStatus,
                               talc_counters* counters) {
-  return correct_batch_device_impl(c, dBases, dOffs, n, totalBases, dOut, outCapacity, dOutOffs, dStatus, counters, nullptr);
+  return correct_batch_device_impl(c, dBases, dOffs, n, totalBases, dOut, outCapacity, dOutOffs, dStatus, counters, nullptr,
+                                   nullptr);
 }
+// dStrandOut (may be null): in auto mode a device copy of the batch's strands[n], made before the call returns
 static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const uint64_t* dOffs, uint32_t n, uint64_t totalBases,
                                      uint8_t* dOut, uint64_t outCapacity, uint64_t* dOutOffs, uint8_t* dStatus,
-                                     talc_counters* counters, u32* dReadStats) {
+                                     talc_counters* counters, u32* dReadStats, u8* dStrandOut) {
   if (!c) return TALC_ERR_ARG;
   if (c->parent) lane_follow(c);
   if (!c->tableReady) { c->err = "no k-mer table loaded"; return TALC_ERR_NO_TABLE; }
   CUDA_TRY(c, cudaSetDevice(c->device));
   if (counters) memset(counters, 0, sizeof(*counters));
+  const u32 mode = c->strand;
+  c->lastN = 0;
+  c->lastAuto = false;
   if (n == 0) {
     if (dOutOffs) CUDA_TRY(c, cudaMemsetAsync(dOutOffs, 0, 8, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    c->lastAuto = mode == TALC_STRAND_AUTO;
     return TALC_OK;
   }
   CUDA_TRY(c, cudaEventRecord(c->ev[0], c->stream));
+  if (mode == TALC_STRAND_AUTO) CUDA_TRY(c, c->strands.reserve((size_t)n + 1));
   u64 totalKmers = 0;
-  int rc = prepare_batch(c, dBases, dOffs, n, totalBases, totalKmers);
+  int rc = prepare_batch(c, dBases, dOffs, n, totalBases, totalKmers, mode, (u8*)c->strands.p, nullptr);
   if (rc) return rc;
 
   // launch geometry.  Monolithic mode: 128-thread blocks (4 warps = 4 reads in flight per block), a multiple of the
@@ -1899,10 +2016,14 @@ static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const u
   if (hOutFull) { c->err = "internal output arena too small"; return TALC_ERR_CAPACITY; }
   if (hTotalOut > outCapacity) { c->err = "out_capacity too small for the corrected reads"; return TALC_ERR_CAPACITY; }
   gather_kernel<<<c->sms * 8, 256, 0, c->stream>>>((const u8*)c->outArena.p, (const u64*)c->outPos.p, (const u32*)c->outLen.p,
-                                                  dOutOffs, n, dOut, dStatus, c->reverse);
+                                                  dOutOffs, n, dOut, dStatus, (const u8*)c->strands.p, mode);
   CUDA_TRY(c, cudaGetLastError());
   CUDA_TRY(c, cudaEventRecord(c->ev[5], c->stream));
+  if (mode == TALC_STRAND_AUTO && dStrandOut)
+    CUDA_TRY(c, cudaMemcpyAsync(dStrandOut, c->strands.p, n, cudaMemcpyDeviceToDevice, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  c->lastN = n;
+  c->lastAuto = mode == TALC_STRAND_AUTO;
   if (dbg) {
     std::vector<u32> kc(n);
     std::vector<u64> ho(n + 1);
@@ -1999,11 +2120,55 @@ int talc_coverage_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offse
   CUDA_TRY(c, cudaMemcpyAsync(c->bases.p, bases, total, cudaMemcpyHostToDevice, c->stream));
   CUDA_TRY(c, cudaMemcpyAsync(c->offs.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, c->stream));
   u64 totalKmers = 0;
-  const u8* dBases = (const u8*)c->bases.p;  // the reverse-complemented copy in reverse mode
-  int rc = prepare_batch(c, dBases, (const u64*)c->offs.p, n, total, totalKmers);
+  const u8* dBases = (const u8*)c->bases.p;  // the reverse-complemented / oriented copy in reverse / auto mode
+  if (c->strand == TALC_STRAND_AUTO) CUDA_TRY(c, c->orientOut.reserve((size_t)n + 1));  // the strands of a correction stay
+  int rc = prepare_batch(c, dBases, (const u64*)c->offs.p, n, total, totalKmers, c->strand, (u8*)c->orientOut.p, nullptr);
   if (rc) return rc;
   if (totalKmers > countsCapacity) { c->err = "counts_capacity too small"; return TALC_ERR_CAPACITY; }
   CUDA_TRY(c, cudaMemcpyAsync(counts, c->cov.p, totalKmers * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return TALC_OK;
+}
+
+// the strand decision of --strand auto on its own, whatever the context's mode
+int talc_orient_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offsets, uint32_t n, uint8_t* strand,
+                      uint32_t* found_fwd, uint32_t* found_rc) {
+  if (!c || !offsets || (n && (!bases || !strand))) return TALC_ERR_ARG;
+  if (c->parent) lane_follow(c);
+  if (!c->tableReady) { c->err = "no k-mer table loaded"; return TALC_ERR_NO_TABLE; }
+  if (offsets[0] != 0) { c->err = "offsets[0] must be 0"; return TALC_ERR_ARG; }
+  if (!n) return TALC_OK;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  const u64 total = offsets[n];
+  CUDA_TRY(c, c->bases.reserve(total + 64));
+  CUDA_TRY(c, c->offs.reserve((size_t)(n + 1) * 8));
+  const size_t foundAt = ((size_t)n + 16) & ~(size_t)15;  // orientOut: strand[n], then found_fwd[n], found_rc[n]
+  CUDA_TRY(c, c->orientOut.reserve(foundAt + (size_t)n * 8));
+  CUDA_TRY(c, cudaMemcpyAsync(c->bases.p, bases, total, cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(c, cudaMemcpyAsync(c->offs.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+  u8* dStrand = (u8*)c->orientOut.p;
+  u32* dFound = (u32*)(dStrand + foundAt);
+  u64 totalKmers = 0;
+  const u8* dBases = (const u8*)c->bases.p;
+  int rc = prepare_batch(c, dBases, (const u64*)c->offs.p, n, total, totalKmers, TALC_STRAND_AUTO, dStrand, dFound);
+  if (rc) return rc;
+  CUDA_TRY(c, cudaMemcpyAsync(strand, dStrand, n, cudaMemcpyDeviceToHost, c->stream));
+  if (found_fwd) CUDA_TRY(c, cudaMemcpyAsync(found_fwd, dFound, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  if (found_rc) CUDA_TRY(c, cudaMemcpyAsync(found_rc, dFound + n, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return TALC_OK;
+}
+
+int talc_last_strands(talc_ctx* c, uint8_t* dst, uint32_t n) {
+  if (!c || (n && !dst)) return TALC_ERR_ARG;
+  if (n > c->lastN) { c->err = "n exceeds the number of reads of the last batch corrected through this context"; return TALC_ERR_ARG; }
+  if (!n) return TALC_OK;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  if (!c->lastAuto) {  // a batch corrected in forward or reverse mode: every read on the strand the mode chose
+    CUDA_TRY(c, c->strands.reserve(n));
+    CUDA_TRY(c, cudaMemsetAsync(c->strands.p, 0, n, c->stream));
+  }
+  CUDA_TRY(c, cudaMemcpyAsync(dst, c->strands.p, n, cudaMemcpyDefault, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   return TALC_OK;
 }
