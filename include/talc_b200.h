@@ -172,6 +172,26 @@ int talc_table_load_dump_host(talc_ctx* ctx, const char* dump_path, const char* 
  * when it was too small.  n_kmers = occurrences counted, n_distinct = distinct k-mers seen, n_kept = entries kept.   */
 int talc_table_count_reads(talc_ctx* ctx, const char* const* paths, int n_paths, uint64_t expected_distinct,
                            const char* junction_path_or_null, uint64_t* n_kmers, uint64_t* n_distinct, uint64_t* n_kept);
+/* The same with an orientation per file (not in the reference; talc --SRLibType), so that the table holds one strand of
+ * the transcriptome whatever the library: for each window x that SENSE counts (the windows are the same in every mode)
+ *   TALC_SR_SENSE      x                                      (talc_table_count_reads: every file SENSE)
+ *   TALC_SR_ANTISENSE  rc(x)                                  (R1 of fr-firststrand / dUTP, R2 of fr-secondstrand)
+ *   TALC_SR_BOTH       x and rc(x), once when x == rc(x)      (unstranded: `jellyfish count -C`, expanded to both strands)
+ * n_kmers = count increments (two per BOTH window that is not its own reverse complement).  With expected_distinct = 0 a
+ * BOTH file adds size/2 to the sizing instead of size/4.  Another orient value is TALC_ERR_ARG.                     */
+#define TALC_SR_SENSE 0
+#define TALC_SR_ANTISENSE 1
+#define TALC_SR_BOTH 2
+int talc_table_count_reads_oriented(talc_ctx* ctx, const char* const* paths, const int* orient, int n_paths,
+                                    uint64_t expected_distinct, const char* junction_path_or_null, uint64_t* n_kmers,
+                                    uint64_t* n_distinct, uint64_t* n_kept);
+/* load_dump with flags (talc_table_load_dump = flags 0).  TALC_DUMP_CANONICAL: the dump holds canonical counts
+ * (`jellyfish count -C`); line i (x, c) stands for the two lines (x, c), (rc(x), c) at 2i and 2i+1, and the usual rules
+ * (MIN_COUNT per line, first line wins, junction colours) apply to that expanded dump.  n_lines counts the dump's own
+ * lines.  Other flag bits are TALC_ERR_ARG.                                                                          */
+#define TALC_DUMP_CANONICAL 1u
+int talc_table_load_dump_ex(talc_ctx* ctx, const char* dump_path, const char* junction_path, uint32_t flags,
+                            uint64_t* n_lines, uint64_t* n_kept);
 /* Jellyfish `dump -c` text of packed k-mers (KMER<space>COUNT\n, given order): the inverse of the parser, for tests,
  * benches and for exporting a table.  Host only.                                                                    */
 int talc_dump_write_packed(const char* path, const uint64_t* keys, const int64_t* counts, uint64_t n, uint32_t K);
@@ -214,6 +234,11 @@ int talc_table_load_cache(talc_ctx* ctx, const char* path, uint64_t* n_entries);
  * header, recount the occupied slots on the device and refuse a table that is more than half full.            */
 int talc_table_load_cache_for(talc_ctx* ctx, const char* path, const char* dump_path, const char* junction_path_or_null,
                               uint64_t* n_entries);
+/* The header also records the TALC_DUMP_* flags the dump was loaded with (0 in caches written before they existed);
+ * load_cache_for_ex refuses (TALC_ERR_STALE) a cache with other flags, load_cache_for is flags = 0.  talc_table_copy
+ * and the replication calls carry the flags to the copies.                                                         */
+int talc_table_load_cache_for_ex(talc_ctx* ctx, const char* path, const char* dump_path, const char* junction_path_or_null,
+                                 uint32_t flags, uint64_t* n_entries);
 /* point look-ups from the host (tests, debugging): found[i] in {0,1}                              */
 int talc_table_lookup(talc_ctx* ctx, const uint64_t* keys, uint64_t n, uint32_t* counts, uint32_t* colours,
                       uint8_t* found);

@@ -37,6 +37,8 @@ class TalcCounters(C.Structure):
 STATUS_MESSAGES = {1: "No solid kmer could be found.", 2: "Unable to define convenient structure."}
 STATUS_RESOURCE = 4  # TALC_READ_RESOURCE: passed through uncorrected, not a reference status
 STRAND_MODES = {"forward": 0, "reverse": 1, "auto": 2}  # TALC_STRAND_FORWARD / _REVERSE / _AUTO
+SR_SENSE, SR_ANTISENSE, SR_BOTH = 0, 1, 2  # TALC_SR_*: orientation of a short-read file
+DUMP_CANONICAL = 1  # TALC_DUMP_CANONICAL
 
 _lib = None
 
@@ -65,6 +67,10 @@ def lib():
         L.talc_table_load_dump_host.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_dump_write_packed.argtypes = [C.c_char_p, vp, vp, C.c_uint64, C.c_uint32]
         L.talc_table_count_reads.argtypes = [vp, C.POINTER(C.c_char_p), C.c_int, C.c_uint64, C.c_char_p, u64p, u64p, u64p]
+        L.talc_table_count_reads_oriented.argtypes = [vp, C.POINTER(C.c_char_p), C.POINTER(C.c_int), C.c_int, C.c_uint64,
+                                                      C.c_char_p, u64p, u64p, u64p]
+        L.talc_table_load_dump_ex.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_uint32, u64p, u64p]
+        L.talc_table_load_cache_for_ex.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint32, u64p]
         L.talc_table_load_packed.argtypes = [vp, vp, vp, C.c_uint64, vp, vp, C.c_uint64, C.c_int, u64p]
         L.talc_table_info.argtypes = [vp, u64p, u64p, u64p]
         L.talc_table_alloc.argtypes = [vp, C.c_uint64]
@@ -196,10 +202,17 @@ class Talc:
         return dst[:n]
 
     # ---- table
-    def load_dump(self, dump: str, junctions: Optional[str] = None):
+    def load_dump(self, dump: str, junctions: Optional[str] = None, canonical: bool = False):
+        """canonical=True: the dump holds `jellyfish count -C` counts; each line (x, c) also stands for (rc(x), c)
+        (talc_table_load_dump_ex with TALC_DUMP_CANONICAL).  Returns (dump lines, entries kept)."""
         nl, nk = C.c_uint64(0), C.c_uint64(0)
-        self._check(lib().talc_table_load_dump(self.h, dump.encode(), junctions.encode() if junctions else None,
-                                               C.byref(nl), C.byref(nk)), "talc_table_load_dump")
+        j = junctions.encode() if junctions else None
+        if canonical:
+            self._check(lib().talc_table_load_dump_ex(self.h, dump.encode(), j, DUMP_CANONICAL, C.byref(nl), C.byref(nk)),
+                        "talc_table_load_dump_ex")
+        else:
+            self._check(lib().talc_table_load_dump(self.h, dump.encode(), j, C.byref(nl), C.byref(nk)),
+                        "talc_table_load_dump")
         return nl.value, nk.value
 
     def load_dump_host(self, dump: str, junctions: Optional[str] = None):
@@ -209,14 +222,22 @@ class Talc:
                                                     C.byref(nl), C.byref(nk)), "talc_table_load_dump_host")
         return nl.value, nk.value
 
-    def count_reads(self, paths, expected_distinct: int = 0, junctions: Optional[str] = None):
-        """Row f3: build the table by counting k-mers of short-read FASTQ/FASTA files on the GPU.
-        Returns (k-mer occurrences, distinct k-mers, entries kept)."""
+    def count_reads(self, paths, orient=None, expected_distinct: int = 0, junctions: Optional[str] = None):
+        """Row f3: build the table by counting k-mers of short-read FASTQ/FASTA files on the GPU.  orient: one
+        SR_SENSE / SR_ANTISENSE / SR_BOTH per file (talc_table_count_reads_oriented); None counts every file as it is
+        (talc_table_count_reads).  Returns (count increments, distinct k-mers, entries kept)."""
         arr = (C.c_char_p * len(paths))(*[p.encode() for p in paths])
         a, b, d = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
-        self._check(lib().talc_table_count_reads(self.h, arr, len(paths), expected_distinct,
-                                                 junctions.encode() if junctions else None, C.byref(a), C.byref(b),
-                                                 C.byref(d)), "talc_table_count_reads")
+        j = junctions.encode() if junctions else None
+        if orient is None:
+            self._check(lib().talc_table_count_reads(self.h, arr, len(paths), expected_distinct, j, C.byref(a), C.byref(b),
+                                                     C.byref(d)), "talc_table_count_reads")
+        else:
+            if len(orient) != len(paths):
+                raise ValueError("count_reads: one orientation per file")
+            o = (C.c_int * len(paths))(*[int(x) for x in orient])
+            self._check(lib().talc_table_count_reads_oriented(self.h, arr, o, len(paths), expected_distinct, j, C.byref(a),
+                                                              C.byref(b), C.byref(d)), "talc_table_count_reads_oriented")
         return a.value, b.value, d.value
 
     def load_packed(self, keys, counts, jkeys=None, jcounts=None) -> int:
@@ -238,11 +259,17 @@ class Talc:
         self._check(lib().talc_table_load_cache(self.h, path.encode(), C.byref(n)), "talc_table_load_cache")
         return n.value
 
-    def table_load_cache_for(self, path: str, dump: str, junctions: Optional[str] = None) -> int:
+    def table_load_cache_for(self, path: str, dump: str, junctions: Optional[str] = None, canonical: bool = False) -> int:
+        """canonical: the cache must have been saved from a table loaded with load_dump(..., canonical=True), and
+        without it from one that was not (talc_table_load_cache_for_ex)."""
         n = C.c_uint64(0)
-        self._check(lib().talc_table_load_cache_for(self.h, path.encode(), dump.encode(),
-                                                    junctions.encode() if junctions else None, C.byref(n)),
-                    "talc_table_load_cache_for")
+        j = junctions.encode() if junctions else None
+        if canonical:
+            self._check(lib().talc_table_load_cache_for_ex(self.h, path.encode(), dump.encode(), j, DUMP_CANONICAL,
+                                                           C.byref(n)), "talc_table_load_cache_for_ex")
+        else:
+            self._check(lib().talc_table_load_cache_for(self.h, path.encode(), dump.encode(), j, C.byref(n)),
+                        "talc_table_load_cache_for")
         return n.value
 
     def bench_random_sectors(self, buffer_bytes: int = 4 << 30, dependent: bool = False, warps_per_sm: int = 64):

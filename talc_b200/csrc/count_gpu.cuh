@@ -10,13 +10,40 @@
 // Files stream through two pinned staging buffers; a piece is cut at a record boundary, its line offsets are found as in
 // dump_gpu.cuh, and one thread per sequence line rolls a 2-bit k-mer over the line and bumps an open-addressed counting
 // table (16-byte slots, CAS on the key + atomicAdd on the count).  Formats: FASTQ with four lines per record and FASTA
-// with one sequence line per record (what short-read pipelines write).
+// with one sequence line per record (what short-read pipelines write).  Each file has an orientation (SrOrient): a
+// stranded library counts its antisense mates as their reverse complements, an unstranded one counts both strands.
 #pragma once
 #include "dump_gpu.cuh"
 
 namespace talc {
 
-// seqPhase / period: sequence lines are those with (firstLine + li) % period == seqPhase
+// Orientation of a short-read file (TALC_SR_* of include/talc_b200.h): what is counted for each window x of a read.
+enum SrOrient : int {
+  kSrSense = 0,      // x (the reference's recipe)
+  kSrAntisense = 1,  // rc(x): reads of the strand opposite to the transcripts (R1 of a dUTP library)
+  kSrBoth = 2        // x and rc(x), once when x == rc(x): unstranded libraries, `jellyfish count -C` expanded
+};
+
+// one occurrence of `key`: claim its slot (CAS on the key) and bump the count; a full table raises *fail
+__device__ __forceinline__ void count_bump(Slot* slots, u64 mask, u64 key, u32* fail) {
+  u64 b = hash_kmer(key) & mask & ~1ull;
+  Slot* hit = nullptr;
+  for (u64 lap = 0; !hit && lap <= mask; lap += 2) {
+    for (int j = 0; j < 2 && !hit; ++j) {
+      Slot* s = slots + b + j;
+      unsigned long long prev = *(volatile unsigned long long*)&s->key;
+      if (prev == kEmptyKey) prev = atomicCAS((unsigned long long*)&s->key, (unsigned long long)kEmptyKey, (unsigned long long)key);
+      if (prev == kEmptyKey || prev == key) hit = s;
+    }
+    b = (b + 2) & mask;
+  }
+  if (!hit) { atomicExch(fail, 1u); return; }
+  atomicAdd(&hit->count, 1u);
+}
+
+// sequence lines are those with li % period == 1.  The windows are the same in every orientation: K consecutive bases
+// that base_code reads as A, C, G or T (U counts as T); ORIENT only chooses which key(s) a window adds.
+template <int ORIENT>
 __global__ void count_kmers_kernel(const char* __restrict__ text, u64 size, const u64* __restrict__ starts, u64 nLines, u32 period,
                                    u32 K, Slot* slots, u64 mask, unsigned long long* nKmers, u32* fail) {
   const u64 stride = (u64)gridDim.x * blockDim.x;
@@ -27,7 +54,7 @@ __global__ void count_kmers_kernel(const char* __restrict__ text, u64 size, cons
     const u64 p = starts[li];
     u64 eol = (li + 1 < nLines) ? starts[li + 1] - 1 : size;
     if (li + 1 == nLines && size > 0 && text[size - 1] == '\n') eol = size - 1;
-    u64 km = 0;
+    u64 km = 0, rc = 0;
     u32 run = 0;  // consecutive valid bases
     for (u64 q = p; q < eol; ++q) {
       const char ch = text[q];
@@ -35,21 +62,16 @@ __global__ void count_kmers_kernel(const char* __restrict__ text, u64 size, cons
       const u32 c = base_code((u8)ch);
       if (c > 3) { run = 0; km = 0; continue; }
       km = ((km << 2) | c) & kmask;
+      if (ORIENT != kSrSense) rc = kmer_roll_rc(rc, c, K);
       if (++run < K) continue;
-      ++mine;
-      u64 b = hash_kmer(km) & mask & ~1ull;
-      Slot* hit = nullptr;
-      for (u64 lap = 0; !hit && lap <= mask; lap += 2) {
-        for (int j = 0; j < 2 && !hit; ++j) {
-          Slot* s = slots + b + j;
-          unsigned long long prev = *(volatile unsigned long long*)&s->key;
-          if (prev == kEmptyKey) prev = atomicCAS((unsigned long long*)&s->key, (unsigned long long)kEmptyKey, (unsigned long long)km);
-          if (prev == kEmptyKey || prev == km) hit = s;
-        }
-        b = (b + 2) & mask;
+      if (ORIENT != kSrAntisense) {
+        ++mine;
+        count_bump(slots, mask, km, fail);
       }
-      if (!hit) { atomicExch(fail, 1u); continue; }
-      atomicAdd(&hit->count, 1u);
+      if (ORIENT == kSrAntisense || (ORIENT == kSrBoth && rc != km)) {
+        ++mine;
+        count_bump(slots, mask, rc, fail);
+      }
     }
   }
   mine = __reduce_add_sync(0xffffffffu, (u32)mine);

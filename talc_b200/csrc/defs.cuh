@@ -122,6 +122,18 @@ TALC_HD u8 dna5_complement(u8 c) {
 
 TALC_HD u64 kmer_mask(u32 K) { return (K >= 32) ? ~0ull : ((1ull << (2 * K)) - 1ull); }
 
+// The reverse complement of a rolled k-mer, rolled alongside it: push base code c (0..3) of the read.  After K pushes
+// it is the reverse complement of the last K bases, whatever it held before.
+TALC_HD u64 kmer_roll_rc(u64 rc, u32 c, u32 K) { return (rc >> 2) | ((u64)(3u - (c & 3u)) << (2 * (K - 1))); }
+TALC_HD u64 kmer_revcomp(u64 k, u32 K) {
+  u64 r = 0;
+  for (u32 i = 0; i < K; ++i) {
+    r = (r << 2) | (3 - (k & 3));
+    k >>= 2;
+  }
+  return r;
+}
+
 // --strand auto.  A read's k-mers and the k-mers of its reverse complement (dna5_complement, read backwards) rolled
 // together, one byte per base, K <= 31.  After base p + K - 1 has been pushed, `fwd` is the window of the read at p and
 // `rc` the window of the reverse complement at len - K - p, i.e. the reverse complement of `fwd`; a window holds no N
@@ -138,7 +150,7 @@ TALC_HD void strand_roll_push(StrandRoll& s, u8 ch, u32 K) {
   s.runF = (c > 3u) ? 0u : s.runF + 1u;
   s.runR = nR ? 0u : s.runR + 1u;
   s.fwd = ((s.fwd << 2) | (u64)(c & 3u)) & kmer_mask(K);
-  s.rc = (s.rc >> 2) | ((u64)(3u - (c & 3u)) << (2 * (K - 1)));
+  s.rc = kmer_roll_rc(s.rc, c, K);
 }
 // found_fwd / found_rc: windows without N found in the table on either strand.  Antisense (1) only on a strict
 // majority: ties -- reads shorter than K, all-N reads, reverse palindromes -- stay forward (0).

@@ -103,6 +103,22 @@ __global__ void parse_lines_kernel(const char* __restrict__ text, u64 size, cons
   }
 }
 
+// A canonical dump (`jellyfish count -C`): line i (x, c) stands for the lines 2i (x, c) and 2i+1 (rc(x), c) of a
+// directional dump, so that table_insert_kernel's "first line wins" applies to the expansion.  A dropped line (kEmptyKey)
+// stays dropped on both.
+__global__ void dump_expand_rc_kernel(const u64* __restrict__ keys, const u32* __restrict__ counts, u64 nLines, u32 K,
+                                      u64* __restrict__ outKeys, u32* __restrict__ outCounts) {
+  const u64 stride = (u64)gridDim.x * blockDim.x;
+  for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < nLines; i += stride) {
+    const u64 x = keys[i];
+    const u32 v = counts[i];
+    outKeys[2 * i] = x;
+    outKeys[2 * i + 1] = x == kEmptyKey ? kEmptyKey : kmer_revcomp(x, K);
+    outCounts[2 * i] = v;
+    outCounts[2 * i + 1] = v;
+  }
+}
+
 // the text of a file in HBM: fread into two pinned buffers, copies overlapped with the next read
 static cudaError_t file_to_device(const char* path, cudaStream_t stream, char** dText, u64* size, std::string& err) {
   *dText = nullptr;

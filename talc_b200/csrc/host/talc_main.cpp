@@ -17,6 +17,16 @@
 // by the library, or with peer copies: --replicate peer), --tableCache <file>, --readStats (the per-read rows of Read.cpp:418-433 the reference left disabled
 // at main.cpp:305), --strand forward|reverse|auto (reverse = --reverse; auto chooses each read's strand and also
 // writes <prefix>.strand.txt, one "<id>\t+" or "<id>\t-" line per read in input order).
+// The k-mer table comes from exactly one of
+//   --SRCounts <dump> [--SRCanonical]   a Jellyfish `dump -c`; --SRCanonical: a `jellyfish count -C` dump, each line
+//                                       (x, c) also standing for (rc(x), c)
+//   --SRReads <fq|fa> ... [--SRReads2 <fq|fa> ...] [--SRLibType asis|unstranded|fr-firststrand|fr-secondstrand]
+//   [--SRExpected <N>]                  short reads counted on the GPU (talc_table_count_reads_oriented).  --SRReads:
+//                                       single-end or R1 files, --SRReads2: their R2 mates, as many.  asis (default):
+//                                       every file as it is (the reference's recipe); unstranded: both strands of every
+//                                       file; fr-firststrand (dUTP): R1 / single-end reverse-complemented, R2 as is;
+//                                       fr-secondstrand: the opposite.  --SRExpected: jellyfish's -s.  Not with
+//                                       --SRCanonical or --tableCache.  A counting table that is too small exits 2.
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -44,7 +54,22 @@ struct Cli {
   long batchReads = 131072, batchBases = 256l << 20;
   talc_params p;
   bool haveK = false, haveSR = false;
+  // counting the table from short reads instead of --SRCounts
+  std::vector<std::string> srReads, srReads2;  // single-end or R1 files; R2 mates
+  std::string srLibType;
+  long srExpected = 0;
+  bool haveExpected = false, srCanonical = false;
 };
+
+// orientation (TALC_SR_*) of every short-read file, R1 / single-end files first, then the R2 mates
+static std::vector<int> sr_orientations(const Cli& c) {
+  const std::string& t = c.srLibType;
+  const int r1 = t == "unstranded" ? TALC_SR_BOTH : t == "fr-firststrand" ? TALC_SR_ANTISENSE : TALC_SR_SENSE;
+  const int r2 = t == "unstranded" ? TALC_SR_BOTH : t == "fr-secondstrand" ? TALC_SR_ANTISENSE : TALC_SR_SENSE;
+  std::vector<int> o(c.srReads.size(), r1);
+  o.insert(o.end(), c.srReads2.size(), r2);
+  return o;
+}
 
 static bool to_int(const std::string& s, long& v) {
   char* e = nullptr;
@@ -72,6 +97,14 @@ static int parse(int argc, const char** argv, Cli& c) {
     else if (a == "-k" || a == "--kmerSize") { if (!val(v) || !to_int(v, n) || n < 18 || n > 30) return 1; c.p.K = (uint32_t)n; c.haveK = true; }
     else if (a == "-qm" || a == "--query-mode") { if (!val(c.queryMode) || (c.queryMode != "memory" && c.queryMode != "jellyfish2")) return 1; }
     else if (a == "-SR" || a == "--SRCounts") { if (!val(c.dump)) return 1; c.haveSR = true; }
+    else if (a == "--SRReads") { if (!val(v)) return 1; c.srReads.push_back(v); }
+    else if (a == "--SRReads2") { if (!val(v)) return 1; c.srReads2.push_back(v); }
+    else if (a == "--SRLibType") {
+      if (!val(c.srLibType) || (c.srLibType != "asis" && c.srLibType != "unstranded" && c.srLibType != "fr-firststrand" &&
+                                c.srLibType != "fr-secondstrand")) return 1;
+    }
+    else if (a == "--SRExpected") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.srExpected = n; c.haveExpected = true; }
+    else if (a == "--SRCanonical") { c.srCanonical = true; }
     else if (a == "-j" || a == "--junctions") { if (!val(c.junctions)) return 1; c.useJunctions = true; }
     else if (a == "--tableCache") { if (!val(c.tableCache)) return 1; }  // extension: binary cache of the built table
     else if (a == "--replicate") { if (!val(c.replicate) || (c.replicate != "nccl" && c.replicate != "peer")) return 1; }
@@ -95,7 +128,11 @@ static int parse(int argc, const char** argv, Cli& c) {
     else if (a.size() > 1 && a[0] == '-') return 1;
     else pos.push_back(a);
   }
-  if (pos.size() != 1 || !c.haveK || !c.haveSR) return 1;
+  const bool counting = !c.srReads.empty();
+  if (pos.size() != 1 || !c.haveK || c.haveSR == counting) return 1;  // exactly one of --SRCounts and --SRReads
+  if (!counting && (!c.srLibType.empty() || !c.srReads2.empty() || c.haveExpected)) return 1;
+  if (!c.srReads2.empty() && c.srReads2.size() != c.srReads.size()) return 1;  // one R2 per R1
+  if (counting && (c.srCanonical || !c.tableCache.empty())) return 1;
   if (c.reverse && !c.strand.empty() && c.strand != "reverse") return 1;  // --reverse is --strand reverse
   c.strandMode = (c.reverse || c.strand == "reverse") ? TALC_STRAND_REVERSE : c.strand == "auto" ? TALC_STRAND_AUTO : TALC_STRAND_FORWARD;
   if (c.queryMode != "memory") { std::cerr << "talc: only query mode 'memory' is supported\n"; return 1; }
@@ -138,7 +175,11 @@ int main(int argc, const char** argv) {
   const int pr = parse(argc, argv, cli);
   if (pr == 2) {
     std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse | --strand forward|reverse|auto] [--gpus <N>] [--tableCache <file>]"
-                 " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer]\n";
+                 " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer]\n"
+                 "  the k-mer table: --SRCounts <dump> [--SRCanonical] (a `jellyfish count -C` dump: each k-mer also stands for its"
+                 " reverse complement)\n"
+                 "               or --SRReads <fq|fa> ... [--SRReads2 <fq|fa> ...] [--SRLibType asis|unstranded|fr-firststrand|fr-secondstrand]"
+                 " [--SRExpected <N>] (counted on the GPU; --SRReads2: R2 mates, one per --SRReads)\n";
     return 0;
   }
   if (pr != 0) { std::cerr << "talc: PARSE_ERROR\n"; return 1; }
@@ -181,14 +222,34 @@ int main(int argc, const char** argv) {
   // --tableCache <file> (extension, SURVEY row f1): reuse the built table if the file exists, else build it from the
   // dump and write the file; a cache made from other --SRCounts / --junctions files (size, mtime), another -k or
   // MIN_COUNT is refused by the library and rebuilt
-  if (!cli.tableCache.empty())
-    rc = talc_table_load_cache_for(ctx[0], cli.tableCache.c_str(), cli.dump.c_str(),
-                                   cli.useJunctions ? cli.junctions.c_str() : nullptr, &nKept);
-  if (rc == TALC_ERR_STALE) std::cout << "[TALC]: " << talc_last_error(ctx[0]) << " -> rebuilding it." << std::endl;
-  if (rc != 0) {
-    rc = talc_table_load_dump(ctx[0], cli.dump.c_str(), cli.useJunctions ? cli.junctions.c_str() : nullptr, &nLines, &nKept);
-    if (rc == 0 && nKept > 0 && !cli.tableCache.empty() && talc_table_save(ctx[0], cli.tableCache.c_str()) != 0)
-      std::cerr << "talc: " << talc_last_error(ctx[0]) << "\n";
+  const char* junctions = cli.useJunctions ? cli.junctions.c_str() : nullptr;
+  const uint32_t dumpFlags = cli.srCanonical ? TALC_DUMP_CANONICAL : 0u;
+  if (!cli.srReads.empty()) {
+    // --SRReads [--SRReads2] --SRLibType: the table counted on the GPU, each file on the strand its library type gives it
+    std::vector<const char*> paths;
+    for (const auto& f : cli.srReads) paths.push_back(f.c_str());
+    for (const auto& f : cli.srReads2) paths.push_back(f.c_str());
+    const std::vector<int> orient = sr_orientations(cli);
+    uint64_t nOcc = 0, nDistinct = 0;
+    rc = talc_table_count_reads_oriented(ctx[0], paths.data(), orient.data(), (int)paths.size(), (uint64_t)cli.srExpected,
+                                         junctions, &nOcc, &nDistinct, &nKept);
+    if (rc == TALC_ERR_CAPACITY) {
+      std::cerr << "talc: " << talc_last_error(ctx[0]) << " (--SRExpected)\n";
+      return 2;
+    }
+    if (rc == 0)
+      std::cout << "[TALC]: counted " << nOcc << " k-mer occurrences in " << paths.size() << " short-read file(s) (library type "
+                << (cli.srLibType.empty() ? "asis" : cli.srLibType) << "): " << nDistinct << " distinct, " << nKept
+                << " with count >= " << cli.p.min_count << "." << std::endl;
+  } else {
+    if (!cli.tableCache.empty())
+      rc = talc_table_load_cache_for_ex(ctx[0], cli.tableCache.c_str(), cli.dump.c_str(), junctions, dumpFlags, &nKept);
+    if (rc == TALC_ERR_STALE) std::cout << "[TALC]: " << talc_last_error(ctx[0]) << " -> rebuilding it." << std::endl;
+    if (rc != 0) {
+      rc = talc_table_load_dump_ex(ctx[0], cli.dump.c_str(), junctions, dumpFlags, &nLines, &nKept);
+      if (rc == 0 && nKept > 0 && !cli.tableCache.empty() && talc_table_save(ctx[0], cli.tableCache.c_str()) != 0)
+        std::cerr << "talc: " << talc_last_error(ctx[0]) << "\n";
+    }
   }
   if (rc != 0) { std::cerr << "talc: " << talc_last_error(ctx[0]) << "\n"; nKept = 0; }
   std::cout << "[TALC]: SR-dBG contains " << nKept << " nodes." << std::endl;
@@ -196,6 +257,9 @@ int main(int argc, const char** argv) {
     std::cout << "[TALC]: The de Bruijn Graph is empty...Correction aborted." << std::endl;
     return 1;  // main.cpp:320
   }
+  if (cli.strandMode == TALC_STRAND_AUTO && (cli.srLibType == "unstranded" || cli.srCanonical))
+    std::cout << "[TALC]: note: the k-mer table holds both strands, so --strand auto finds every read equally on both and "
+                 "keeps it forward (reads holding U excepted)." << std::endl;
   const double sTable = since(tTable);
   const auto tRep = std::chrono::steady_clock::now();
   if (cli.gpus > 1) {

@@ -81,7 +81,7 @@ int talc_table_broadcast(talc_ctx* c, const uint8_t id[128], int rank, int world
   int r = N.CommInitRank(&comm, world, u, rank);
   if (r != 0) { c->err = std::string("ncclCommInitRank: ") + (N.GetErrorString ? N.GetErrorString(r) : "error"); return TALC_ERR_NCCL; }
   u64* dMeta = nullptr;
-  u64 hMeta[8] = {c->capacity, c->nEntries, c->provJunctions, c->provDumpSize, c->provDumpMtime, c->provJuncSize, c->provJuncMtime, 0};
+  u64 hMeta[8] = {c->capacity, c->nEntries, c->provJunctions, c->provDumpSize, c->provDumpMtime, c->provJuncSize, c->provJuncMtime, c->provFlags};
   int rc = TALC_OK;
   do {
     if (cudaMalloc((void**)&dMeta, sizeof(hMeta)) != cudaSuccess) { rc = TALC_ERR_CUDA; break; }
@@ -93,6 +93,7 @@ int talc_table_broadcast(talc_ctx* c, const uint8_t id[128], int rank, int world
       rc = talc_table_alloc(c, hMeta[0]);
       if (rc) break;
       c->provJunctions = (u32)hMeta[2];
+      c->provFlags = (u32)hMeta[7];
       c->provDumpSize = hMeta[3]; c->provDumpMtime = hMeta[4]; c->provJuncSize = hMeta[5]; c->provJuncMtime = hMeta[6];
     }
     cudaEventRecord(c->ev[6], c->stream);
@@ -134,6 +135,7 @@ int talc_table_replicate(talc_ctx** ctxs, int n, double* broadcast_ms, int* used
     const int rc = talc_table_alloc(ctxs[i], src->capacity);
     if (rc) return rc;
     ctxs[i]->provJunctions = src->provJunctions;
+    ctxs[i]->provFlags = src->provFlags;
     ctxs[i]->provDumpSize = src->provDumpSize; ctxs[i]->provDumpMtime = src->provDumpMtime;
     ctxs[i]->provJuncSize = src->provJuncSize; ctxs[i]->provJuncMtime = src->provJuncMtime;
   }

@@ -876,6 +876,7 @@ struct talc_ctx {
   talc_ctx* parent = nullptr;  // a lane (talc_ctx_create_lane): tables and settings are the parent's, scratch and stream its own
   // where the table came from (recorded in the binary cache so that a cache of other inputs is not reused silently)
   u32 provJunctions = 0;
+  u32 provFlags = 0;  // TALC_DUMP_* the dump was read with
   u64 provDumpSize = 0, provDumpMtime = 0, provJuncSize = 0, provJuncMtime = 0;
   CtxBucket* ctxRight = nullptr;  // successor tables, derived from the k-mer table when it is sealed
   CtxBucket* ctxLeft = nullptr;
@@ -1198,6 +1199,7 @@ extern "C" int talc_table_copy(talc_ctx* dst, talc_ctx* src) {
   if (rc) return rc;
   CUDA_TRY(dst, cudaMemcpyPeer(dst->slots, dst->device, src->slots, src->device, src->capacity * sizeof(Slot)));
   dst->provJunctions = src->provJunctions;
+  dst->provFlags = src->provFlags;
   dst->provDumpSize = src->provDumpSize; dst->provDumpMtime = src->provDumpMtime;
   dst->provJuncSize = src->provJuncSize; dst->provJuncMtime = src->provJuncMtime;
   return talc_table_seal(dst, src->nEntries);
@@ -1208,7 +1210,7 @@ struct TableCacheHeader {
   char magic[8];  // "TALCTBL2"
   u32 K, min_count;
   u64 capacity, entries;
-  u32 junctions, pad;                                // junction colours baked in?
+  u32 junctions, flags;                              // junction colours baked in?  TALC_DUMP_* (0 before there were any)
   u64 dumpSize, dumpMtime, juncSize, juncMtime;      // identity of the text inputs (0 = built from packed arrays)
 };
 static void file_identity(const char* path, u64& size, u64& mtime) {
@@ -1226,6 +1228,7 @@ extern "C" int talc_table_save(talc_ctx* c, const char* path) {
   memcpy(h.magic, "TALCTBL2", 8);
   h.K = c->P.K; h.min_count = c->P.min_count; h.capacity = c->capacity; h.entries = c->nEntries;
   h.junctions = c->provJunctions;
+  h.flags = c->provFlags;
   h.dumpSize = c->provDumpSize; h.dumpMtime = c->provDumpMtime; h.juncSize = c->provJuncSize; h.juncMtime = c->provJuncMtime;
   bool ok = fwrite(&h, sizeof(h), 1, f) == 1;
   const size_t total = (size_t)c->capacity * sizeof(Slot), piece = 64u << 20;
@@ -1239,9 +1242,9 @@ extern "C" int talc_table_save(talc_ctx* c, const char* path) {
   if (!ok) { c->err = std::string("error while writing ") + path; return TALC_ERR_IO; }
   return TALC_OK;
 }
-// check_inputs: the cache must have been made from exactly these text files (size + mtime) and junction setting
+// check_inputs: the cache must have been made from exactly these text files (size + mtime), junction setting and flags
 static int load_cache(talc_ctx* c, const char* path, bool check_inputs, const char* dump_path, const char* junction_path,
-                      uint64_t* n_entries) {
+                      u32 flags, uint64_t* n_entries) {
   if (!c || !path) return TALC_ERR_ARG;
   FILE* f = fopen(path, "rb");
   if (!f) { c->err = std::string("cannot read ") + path; return TALC_ERR_IO; }
@@ -1268,6 +1271,12 @@ static int load_cache(talc_ctx* c, const char* path, bool check_inputs, const ch
       c->err = "table cache was built from other --SRCounts / --junctions inputs";
       return TALC_ERR_STALE;
     }
+    if (h.flags != flags) {
+      fclose(f);
+      c->err = (h.flags & TALC_DUMP_CANONICAL) ? "table cache was built from a canonical dump (--SRCanonical)"
+                                              : "table cache was built from a directional dump (without --SRCanonical)";
+      return TALC_ERR_STALE;
+    }
   }
   int rc = talc_table_alloc(c, h.capacity);
   if (rc) { fclose(f); return rc; }
@@ -1282,6 +1291,7 @@ static int load_cache(talc_ctx* c, const char* path, bool check_inputs, const ch
   fclose(f);
   if (!ok) { c->err = std::string("truncated table cache ") + path; return TALC_ERR_IO; }
   c->provJunctions = h.junctions;
+  c->provFlags = h.flags;
   c->provDumpSize = h.dumpSize; c->provDumpMtime = h.dumpMtime; c->provJuncSize = h.juncSize; c->provJuncMtime = h.juncMtime;
   rc = talc_table_seal(c, h.entries);
   if (rc) return rc;
@@ -1294,12 +1304,16 @@ static int load_cache(talc_ctx* c, const char* path, bool check_inputs, const ch
   return TALC_OK;
 }
 extern "C" int talc_table_load_cache(talc_ctx* c, const char* path, uint64_t* n_entries) {
-  return load_cache(c, path, false, nullptr, nullptr, n_entries);
+  return load_cache(c, path, false, nullptr, nullptr, 0, n_entries);
+}
+extern "C" int talc_table_load_cache_for_ex(talc_ctx* c, const char* path, const char* dump_path, const char* junction_path,
+                                            uint32_t flags, uint64_t* n_entries) {
+  if (!dump_path || (flags & ~(u32)TALC_DUMP_CANONICAL)) return TALC_ERR_ARG;
+  return load_cache(c, path, true, dump_path, junction_path, flags, n_entries);
 }
 extern "C" int talc_table_load_cache_for(talc_ctx* c, const char* path, const char* dump_path, const char* junction_path,
                                          uint64_t* n_entries) {
-  if (!dump_path) return TALC_ERR_ARG;
-  return load_cache(c, path, true, dump_path, junction_path, n_entries);
+  return talc_table_load_cache_for_ex(c, path, dump_path, junction_path, 0, n_entries);
 }
 
 // common tail of every build: strip the line indices, apply the reduced junction colours + homopolymer resets, check
@@ -1373,15 +1387,6 @@ static int build_table(talc_ctx* c, const std::vector<u64>& keys, const std::vec
   return rc;
 }
 
-static u64 revcomp_kmer(u64 k, u32 K) {
-  u64 r = 0;
-  for (u32 i = 0; i < K; ++i) {
-    r = (r << 2) | (3 - (k & 3));
-    k >>= 2;
-  }
-  return r;
-}
-
 // reduce the junction list to final colours (sequential semantics of Jellyfish.cpp:278-289) and append the
 // four homopolymer resets of decolourRepeatsFromDBG (utils.cpp:658-669)
 static void reduce_colours(const talc_params& p, const u64* jkeys, const i64* jcounts, u64 nj, bool use, std::vector<u64>& ck,
@@ -1393,7 +1398,7 @@ static void reduce_colours(const talc_params& p, const u64* jkeys, const i64* jc
       const u32 v = (u32)(int)jcounts[i];
       if (v < kColouredCountThr) {
         last[jkeys[i]] = v;
-        last[revcomp_kmer(jkeys[i], p.K)] = v;
+        last[kmer_revcomp(jkeys[i], p.K)] = v;
       }
     }
   }
@@ -1429,6 +1434,7 @@ int talc_table_load_packed(talc_ctx* c, const uint64_t* keys, const int64_t* cou
   std::vector<u32> cc;
   reduce_colours(c->params, jkeys, jcounts, nj, use_junctions != 0, ck, cc);
   c->provJunctions = use_junctions ? 1u : 0u;
+  c->provFlags = 0;
   c->provDumpSize = c->provDumpMtime = c->provJuncSize = c->provJuncMtime = 0;
   return build_table(c, k, v, ck, cc, n_kept);
 }
@@ -1436,8 +1442,11 @@ int talc_table_load_packed(talc_ctx* c, const uint64_t* keys, const int64_t* cou
 // buildCDBG + decolourRepeatsFromDBG (Jellyfish.cpp:236-295, utils.cpp:658-669) with the text parsed on the GPU
 // (dump_gpu.cuh): the entries never visit the host.  The junction dump (small) is parsed the same way, then reduced to
 // final colours on the host ("last writer wins, forward before reverse complement" is sequential by nature).
-int talc_table_load_dump(talc_ctx* c, const char* dump_path, const char* junction_path, uint64_t* n_lines, uint64_t* n_kept) {
-  if (!c || !dump_path) return TALC_ERR_ARG;
+// TALC_DUMP_CANONICAL: dump_expand_rc_kernel turns the per-line arrays into those of the expanded dump, then the same
+// insertion runs on 2 * nLines lines.
+int talc_table_load_dump_ex(talc_ctx* c, const char* dump_path, const char* junction_path, uint32_t flags, uint64_t* n_lines,
+                            uint64_t* n_kept) {
+  if (!c || !dump_path || (flags & ~(u32)TALC_DUMP_CANONICAL)) return TALC_ERR_ARG;
   CUDA_TRY(c, cudaSetDevice(c->device));
   DeviceDump d;
   std::string err;
@@ -1472,12 +1481,36 @@ int talc_table_load_dump(talc_ctx* c, const char* dump_path, const char* junctio
   } else {
     reduce_colours(c->params, nullptr, nullptr, 0, false, ck, cc);
   }
+  if ((flags & TALC_DUMP_CANONICAL) && d.nLines) {
+    // the line index travels in the upper half of a 64-bit atomicMin (table_insert_kernel)
+    if (2 * d.nLines > 0xFFFFFFFFull) { d.release(); c->err = "canonical dump: more than 2^31 lines"; return TALC_ERR_ARG; }
+    u64* ek = nullptr;
+    u32* ev = nullptr;
+    if (cudaMalloc((void**)&ek, 2 * d.nLines * 8) != cudaSuccess || cudaMalloc((void**)&ev, 2 * d.nLines * 4) != cudaSuccess) {
+      if (ek) cudaFree(ek);
+      d.release();
+      c->err = "canonical dump: out of device memory";
+      return TALC_ERR_CUDA;
+    }
+    dump_expand_rc_kernel<<<c->sms * 8, 256, 0, c->stream>>>(d.keys, d.counts, d.nLines, c->params.K, ek, ev);
+    const cudaError_t e = cudaGetLastError();
+    d.release();  // cudaFree waits for the expansion to finish
+    d.keys = ek;
+    d.counts = ev;
+    d.nLines *= 2;
+    d.tally.kept *= 2;
+    if (e != cudaSuccess) { d.release(); c->err = cudaGetErrorString(e); return TALC_ERR_CUDA; }
+  }
   c->provJunctions = junction_path ? 1u : 0u;
+  c->provFlags = flags;
   file_identity(dump_path, c->provDumpSize, c->provDumpMtime);
   file_identity(junction_path, c->provJuncSize, c->provJuncMtime);
   const int rc = build_table_device(c, d.keys, d.counts, d.nLines, d.tally.kept, ck, cc, n_kept);
   d.release();
   return rc;
+}
+int talc_table_load_dump(talc_ctx* c, const char* dump_path, const char* junction_path, uint64_t* n_lines, uint64_t* n_kept) {
+  return talc_table_load_dump_ex(c, dump_path, junction_path, 0, n_lines, n_kept);
 }
 
 // The round-1 ingest path, kept for A/B timing only (bench.py --time-table-load): threaded host parse of the mapped
@@ -1507,6 +1540,7 @@ int talc_table_load_dump_host(talc_ctx* c, const char* dump_path, const char* ju
   std::vector<u32> v(d.counts.size());
   for (size_t i = 0; i < v.size(); ++i) v[i] = (u32)(int)d.counts[i];
   c->provJunctions = junction_path ? 1u : 0u;
+  c->provFlags = 0;
   file_identity(dump_path, c->provDumpSize, c->provDumpMtime);
   file_identity(junction_path, c->provJuncSize, c->provJuncMtime);
   return build_table(c, d.keys, v, ck, cc, n_kept);
@@ -1533,15 +1567,19 @@ static int junction_colours_gpu(talc_ctx* c, const char* junction_path, std::vec
   return TALC_OK;
 }
 
-int talc_table_count_reads(talc_ctx* c, const char* const* paths, int n_paths, uint64_t expected_distinct, const char* junction_path,
-                           uint64_t* n_kmers, uint64_t* n_distinct, uint64_t* n_kept) {
-  if (!c || !paths || n_paths < 1) return TALC_ERR_ARG;
+static_assert(TALC_SR_SENSE == kSrSense && TALC_SR_ANTISENSE == kSrAntisense && TALC_SR_BOTH == kSrBoth, "orientation codes");
+
+int talc_table_count_reads_oriented(talc_ctx* c, const char* const* paths, const int* orient, int n_paths, uint64_t expected_distinct,
+                                    const char* junction_path, uint64_t* n_kmers, uint64_t* n_distinct, uint64_t* n_kept) {
+  if (!c || !paths || !orient || n_paths < 1) return TALC_ERR_ARG;
+  for (int i = 0; i < n_paths; ++i)
+    if (orient[i] != kSrSense && orient[i] != kSrAntisense && orient[i] != kSrBoth) return TALC_ERR_ARG;
   CUDA_TRY(c, cudaSetDevice(c->device));
   const u32 K = c->params.K;
-  if (expected_distinct == 0) {  // no hint (jellyfish's -s): one distinct k-mer per 4 bytes of input is generous
+  if (expected_distinct == 0) {  // no hint (jellyfish's -s): one distinct k-mer per 4 bytes of input is generous (2 on both strands)
     for (int i = 0; i < n_paths; ++i) {
       struct stat st;
-      if (stat(paths[i], &st) == 0) expected_distinct += (u64)st.st_size / 4;
+      if (stat(paths[i], &st) == 0) expected_distinct += (u64)st.st_size / (orient[i] == kSrBoth ? 2 : 4);
     }
     if (expected_distinct < (1u << 20)) expected_distinct = 1u << 20;
   }
@@ -1609,7 +1647,9 @@ int talc_table_count_reads(talc_ctx* c, const char* const* paths, int n_paths, u
         if (cudaStreamSynchronize(c->stream) != cudaSuccess) { fail(TALC_ERR_CUDA, "line scan failed"); break; }
       }
       if (usable) {
-        count_kmers_kernel<<<blocks, 256, 0, c->stream>>>(dText, cut, dStarts, usable, period, K, big, cap - 1, dNum + 1, (u32*)(dNum + 2));
+        auto kern = orient[fi] == kSrAntisense ? count_kmers_kernel<kSrAntisense>
+                    : orient[fi] == kSrBoth    ? count_kmers_kernel<kSrBoth> : count_kmers_kernel<kSrSense>;
+        kern<<<blocks, 256, 0, c->stream>>>(dText, cut, dStarts, usable, period, K, big, cap - 1, dNum + 1, (u32*)(dNum + 2));
         if (cudaGetLastError() != cudaSuccess) { fail(TALC_ERR_CUDA, "count kernel launch failed"); break; }
       }
       carry = size - cut;
@@ -1639,6 +1679,7 @@ int talc_table_count_reads(talc_ctx* c, const char* const* paths, int n_paths, u
       std::vector<u32> cc;
       rc = junction_colours_gpu(c, junction_path, ck, cc);
       c->provJunctions = junction_path ? 1u : 0u;
+      c->provFlags = 0;
       c->provDumpSize = c->provDumpMtime = 0;
       file_identity(junction_path, c->provJuncSize, c->provJuncMtime);
       if (rc == TALC_OK) rc = finish_table(c, dNum, ck, cc, n_kept);
@@ -1652,6 +1693,13 @@ int talc_table_count_reads(talc_ctx* c, const char* const* paths, int n_paths, u
   if (dTmp) cudaFree(dTmp);
   cudaFree(big);
   return rc;
+}
+int talc_table_count_reads(talc_ctx* c, const char* const* paths, int n_paths, uint64_t expected_distinct, const char* junction_path,
+                           uint64_t* n_kmers, uint64_t* n_distinct, uint64_t* n_kept) {
+  if (!c || !paths || n_paths < 1) return TALC_ERR_ARG;
+  const std::vector<int> sense((size_t)n_paths, kSrSense);
+  return talc_table_count_reads_oriented(c, paths, sense.data(), n_paths, expected_distinct, junction_path, n_kmers, n_distinct,
+                                         n_kept);
 }
 
 int talc_dump_write_packed(const char* path, const uint64_t* keys, const int64_t* counts, uint64_t n, uint32_t K) {
