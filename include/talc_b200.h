@@ -49,7 +49,8 @@ typedef struct talc_params {
   uint32_t window_size;             /* --WINDOW_SIZE      gp_WINDOW_SIZE (9)            */
   uint32_t max_nb_branches;         /* --MAX_NB_BRANCHES  gp_MAX_NB_COMPETING_PATHS (7) */
   double alpha;                     /* --ALPHA_FOR_PRED   gp_ALPHA (2.57)               */
-  double sr_error_rate;             /* --SR_ERROR_RATE    gp_SR_ERROR_RATE (0.025)      */
+  double sr_error_rate;             /* --SR_ERROR_RATE    gp_SR_ERROR_RATE (0.025); the command line takes [0.01, 0.1],
+                                       talc_ctx_create refuses NaN and anything outside [0, 0.5] (TALC_ERR_ARG) */
   double min_inner_score;           /* --MIN_INNER_SCORE  (0.7)                         */
   double min_border_score;          /* --MIN_BORDER_SCORE (0.7)                         */
   int32_t cycle_mode;               /* 0: SeqAn2 Horspool over mixed alphabets (default), 1: exact first occurrence */
@@ -320,6 +321,22 @@ int talc_test_align(talc_ctx* ctx, int op, const uint8_t* a, const uint64_t* a_o
  * reuse of the corrector.  A score of INT32_MIN means the per-pair scratch (2 MB) was too small.                  */
 int talc_test_align_slices(talc_ctx* ctx, int op, const uint8_t* reads, const uint64_t* read_off, uint32_t n_reads,
                            const int32_t* desc, uint32_t n, int aux, int aux2, int32_t* result);
+/* the successor tables of the walks (one bucket per (K-1)-mer context with the counts of its four successors, derived
+ * from the k-mer table at every seal): for each kmers[i], the look-up the walk makes for its successors, right != 0 the
+ * k-mers x[1..]+b, else b+x[..K-2]; cnt[4*i+b] = count of successor b (0 when absent), colmask[i] bit b = successor b
+ * carries a junction colour.  *ctx_capacity (may be NULL) = buckets per table.  TALC_ERR_NO_TABLE before a seal.     */
+int talc_test_successors(talc_ctx* ctx, int right, const uint64_t* kmers, uint32_t n, uint32_t* cnt, uint32_t* colmask,
+                         uint64_t* ctx_capacity);
+/* the count model of the walk on the context's parameters and device tables (counts below 16384 are tabulated, larger
+ * ones computed).  args[8*i..], out[9*i..] (a double as its IEEE bits):
+ *   op 0  step bounds of count       args {count}                       out {lower, upperNoise, sqrt(count), lambda,
+ *                                                                             noiseModel}
+ *   op 1  successor tags             args {count, c[4], colmask, complex} out {n (0 or 4), tag[4] (0 EXPECTED,
+ *                                                                             1 UNEXPECTED, 2 BREAKPOINT), dist[4]}
+ *   op 2  child of a fast-walk step  args {count, c[4], colmask}        out {child 0..3, or -1 as int64}
+ *   op 3  upper bound test           args {nextc, cc}                   out {nextc within the noise interval of cc}
+ *   op 4  last-node test             args {nextc, cc}                   out {nextc within both bounds of cc}          */
+int talc_test_model(talc_ctx* ctx, int op, const uint32_t* args, uint32_t n, uint64_t* out);
 /* permutation produced by the device replica of libstdc++ std::sort on keys[n] (operator<)        */
 int talc_test_sort(talc_ctx* ctx, const int64_t* keys, uint32_t n, uint32_t* perm);
 

@@ -105,6 +105,8 @@ def lib():
         L.talc_test_align.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_uint32, C.c_int, C.c_int, vp]
         L.talc_test_align_slices.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, C.c_uint32, C.c_int, C.c_int, vp]
         L.talc_test_sort.argtypes = [vp, vp, C.c_uint32, vp]
+        L.talc_test_successors.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, u64p]
+        L.talc_test_model.argtypes = [vp, C.c_int, vp, C.c_uint32, vp]
         _lib = L
     return _lib
 
@@ -389,6 +391,27 @@ class Talc:
         self._check(lib().talc_test_align_slices(self.h, op, _ptr(data), _ptr(off), len(reads), _ptr(desc), n, aux, aux2,
                                                  _ptr(res)), "talc_test_align_slices")
         return res.reshape(n, 4) if wide else res
+
+    def test_successors(self, kmers, right: bool):
+        """talc_test_successors: the walk's successor-table look-up of each k-mer, (cnt uint32[n, 4], colmask uint32[n],
+        buckets per successor table)."""
+        kmers = np.ascontiguousarray(kmers, dtype=np.uint64)
+        n = len(kmers)
+        cnt = np.zeros((max(n, 1), 4), dtype=np.uint32)
+        cm = np.zeros(max(n, 1), dtype=np.uint32)
+        cap = C.c_uint64(0)
+        self._check(lib().talc_test_successors(self.h, 1 if right else 0, _ptr(kmers), n, _ptr(cnt), _ptr(cm),
+                                               C.byref(cap)), "talc_test_successors")
+        return cnt[:n], cm[:n], cap.value
+
+    def test_model(self, op: int, args) -> np.ndarray:
+        """talc_test_model: `args` an [n, <=8] array of uint32 (zero-padded to 8 columns); returns uint64[n, 9]."""
+        a = np.asarray(args, dtype=np.uint32).reshape(len(args), -1)
+        full = np.zeros((len(a), 8), dtype=np.uint32)
+        full[:, :a.shape[1]] = a
+        out = np.zeros((max(len(a), 1), 9), dtype=np.uint64)
+        self._check(lib().talc_test_model(self.h, op, _ptr(full), len(a), _ptr(out)), "talc_test_model")
+        return out[:len(a)]
 
     def test_sort(self, keys) -> np.ndarray:
         keys = np.ascontiguousarray(keys, dtype=np.int64)

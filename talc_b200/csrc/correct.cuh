@@ -191,16 +191,8 @@ class Corrector {
   TALC_HD u32 K() const { return P.K; }
 
   // ------------------------------------------------------------------ prediction intervals from the per-context tables
-  // (filled on the device by model_lower_bound / model_upper_bound themselves, so the comparisons are the ones of
-  // expected_by_model, Explorer.cpp:1185-1217, bit for bit; counts beyond the tables are computed)
-  TALC_HD bool expected_upper_tab(u32 nextc, u32 cc) {
-    if (cc < tabs.n) return (double)nextc <= tabs.upper[cc];
-    return expected_by_model(nextc, cc, P.alpha, true);
-  }
-  TALC_HD bool expected_last_node_tab(u32 nextc, u32 cc) {
-    if (cc < tabs.n) return ((double)nextc <= tabs.upper[cc]) & ((double)nextc >= tabs.lower[cc]);
-    return expected_by_last_node(nextc, cc, P.alpha);
-  }
+  TALC_HD bool expected_upper_tab(u32 nextc, u32 cc) { return talc::expected_upper_tab(nextc, cc, P, tabs); }
+  TALC_HD bool expected_last_node_tab(u32 nextc, u32 cc) { return talc::expected_last_node_tab(nextc, cc, P, tabs); }
 
   // ------------------------------------------------------------------ table access with counters
   // a k-mer holding N: its successors x[1..]+b may or may not hold N; look each one up by bases (rare, out of line)
@@ -819,7 +811,6 @@ class Corrector {
     const u32 k = P.K;
     const bool right = dirRight;
     const CtxView cv = right ? CR : CL;
-    const u32 minCount = P.min_count;
     const u64 kmask = kmer_mask(k), cmask = kmer_mask(k - 1);
     const u32 stride = (P.cycle_mode == 0) ? k : 1u;
     const Trail tr = cur[act ? lane : 0];
@@ -844,13 +835,7 @@ class Corrector {
       if (act) {
         u32 c4[4], cm;
         ctx_lookup(cv, right ? (kmer & cmask) : (kmer >> 2), c4, cm);
-        const u32 m = (u32)(c4[0] >= minCount) | ((u32)(c4[1] >= minCount) << 1) | ((u32)(c4[2] >= minCount) << 2) |
-                      ((u32)(c4[3] >= minCount) << 3);
-        if (m != 0 && (m & (m - 1)) == 0) {
-          child = __ffs((int)m) - 1;  // the only successor in the graph: EXPECTED by the counter == 1 rule
-        } else if (m != 0) {
-          child = pick_single_child(c4, cm, count);  // exact tagger; -1 unless exactly one successor is admissible
-        }
+        child = fast_step_child(c4, cm, count, P, tabs);
         const u32 ch = (u32)(child < 0 ? 0 : child);
         childCnt = ch == 0 ? c4[0] : ch == 1 ? c4[1] : ch == 2 ? c4[2] : c4[3];
       }
@@ -918,20 +903,6 @@ class Corrector {
       }
     }
     return capped;
-  }
-  // more than one successor in the graph: the exact tagging rules decide (rare on the fast path, kept out of line)
-  __device__ __noinline__ int pick_single_child(const u32 c4[4], u32 cm, u32 count) {
-    u32 col4[4];
-    TALC_ROLLED
-    for (int i = 0; i < 4; ++i) col4[i] = (cm >> i) & 1u;
-    const StepBounds sb = step_bounds_tab(count, P, tabs);
-    u8 tag[4];
-    tag_next_nodes(c4, col4, sb, P, false, tag);
-    int child = -1, n = 0;
-    TALC_ROLLED
-    for (int i = 0; i < 4; ++i)
-      if (tag[i] != kUnexpected) { child = i; ++n; }
-    return n == 1 ? child : -1;
   }
 #else
   inline bool fast_walk(u32& step, u32 pathMax, const AnchorRec* aims, u32 nAims, bool border, u32 maxSteps) {

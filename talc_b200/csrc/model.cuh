@@ -73,6 +73,9 @@ struct ModelTabs {
   const double* sq;     // sqrt((double)c)
   u32 n;
 };
+static const u32 kModelTabN = 16384;  // counts with tabulated bounds on the device
+// Indexing M.upper[lambda] below relies on lambda <= count, i.e. on 0 <= sr_error <= 1: talc_ctx_create refuses any
+// rate outside [0, 0.5].
 TALC_HD StepBounds step_bounds_tab(u32 count, const Params& P, const ModelTabs& M) {
   if (count >= M.n) return step_bounds(count, P);
   StepBounds b;
@@ -135,6 +138,89 @@ TALC_HDN int tag_next_nodes(const u32 cnt[4], const u32 col[4], const StepBounds
     if (!((double)(u32)sum <= B.upperNoise)) tag[index] = kBreakpoint;
   }
   return 4;
+}
+
+// The prediction intervals of expected_by_model / expected_by_last_node from the per-context tables (Explorer.cpp:
+// 1185-1217, bit for bit: the tables hold model_lower_bound / model_upper_bound themselves); counts beyond them are
+// computed.
+TALC_HD bool expected_upper_tab(u32 nextc, u32 cc, const Params& P, const ModelTabs& M) {
+  if (cc < M.n) return (double)nextc <= M.upper[cc];
+  return expected_by_model(nextc, cc, P.alpha, true);
+}
+TALC_HD bool expected_last_node_tab(u32 nextc, u32 cc, const Params& P, const ModelTabs& M) {
+  if (cc < M.n) return ((double)nextc <= M.upper[cc]) & ((double)nextc >= M.lower[cc]);
+  return expected_by_last_node(nextc, cc, P.alpha);
+}
+
+// The child of a fast-walk step (Corrector::fast_walk, walk_kernel): a bucket with more than one successor in the
+// graph goes through the exact tagger (complex_ = false, as the walk is never in a complex region when it takes the
+// fast path); -1 unless exactly one successor is admissible.  Rare on the fast path, kept out of line.
+TALC_HDN int pick_single_child(const u32 c4[4], u32 cm, u32 count, const Params& P, const ModelTabs& tabs) {
+  u32 col4[4];
+  TALC_ROLLED
+  for (int i = 0; i < 4; ++i) col4[i] = (cm >> i) & 1u;
+  const StepBounds sb = step_bounds_tab(count, P, tabs);
+  u8 tag[4];
+  tag_next_nodes(c4, col4, sb, P, false, tag);
+  int child = -1, n = 0;
+  TALC_ROLLED
+  for (int i = 0; i < 4; ++i)
+    if (tag[i] != kUnexpected) { child = i; ++n; }
+  return n == 1 ? child : -1;
+}
+// The only successor in the graph is EXPECTED by the counter == 1 rule and needs no tagging; none is a dead end (-1).
+TALC_HD int fast_step_child(const u32 c4[4], u32 cm, u32 count, const Params& P, const ModelTabs& tabs) {
+  const u32 minCount = P.min_count;
+  const u32 m = (u32)(c4[0] >= minCount) | ((u32)(c4[1] >= minCount) << 1) | ((u32)(c4[2] >= minCount) << 2) |
+                ((u32)(c4[3] >= minCount) << 3);
+  if (m != 0 && (m & (m - 1)) == 0) {
+#if defined(__CUDA_ARCH__)
+    return __ffs((int)m) - 1;
+#else
+    return __builtin_ctz(m);
+#endif
+  }
+  if (m != 0) return pick_single_child(c4, cm, count, P, tabs);
+  return -1;
+}
+
+// One query of talc_test_model (include/talc_b200.h) on the functions above, for the device self-test and the host
+// emulation alike.  a[8]: ops 0-2 {count, c4[4], colmask, complex, -}, ops 3-4 {nextc, cc, ...}; out[9] (doubles as
+// their bits): op 0 {lower, upperNoise, sq, lambda, noiseModel}; op 1 {tags, tag[4], step_dist[4]}; op 2 {child as
+// int64}; ops 3-4 {0 / 1}.
+TALC_HD u64 double_bits(double d) {
+  u64 u;
+  memcpy(&u, &d, 8);
+  return u;
+}
+TALC_HDN void selftest_model_op(int op, const u32 a[8], const Params& P, const ModelTabs& M, u64 out[9]) {
+  for (int q = 0; q < 9; ++q) out[q] = 0;
+  const u32 c4[4] = {a[1], a[2], a[3], a[4]};
+  if (op == 0) {
+    const StepBounds b = step_bounds_tab(a[0], P, M);
+    out[0] = double_bits(b.lower);
+    out[1] = double_bits(b.upperNoise);
+    out[2] = double_bits(b.sq);
+    out[3] = b.lambda;
+    out[4] = b.noiseModel ? 1 : 0;
+  } else if (op == 1) {
+    u32 col4[4];
+    for (int i = 0; i < 4; ++i) col4[i] = (a[5] >> i) & 1u;
+    const StepBounds sb = step_bounds_tab(a[0], P, M);
+    u8 tag[4] = {kUnexpected, kUnexpected, kUnexpected, kUnexpected};
+    const int n = tag_next_nodes(c4, col4, sb, P, a[6] != 0, tag);
+    out[0] = (u64)n;
+    for (int i = 0; i < n; ++i) {
+      out[1 + i] = tag[i];
+      out[5 + i] = double_bits(step_dist(a[0], c4[i], sb));
+    }
+  } else if (op == 2) {
+    out[0] = (u64)(i64)fast_step_child(c4, a[5], a[0], P, M);
+  } else if (op == 3) {
+    out[0] = expected_upper_tab(a[0], a[1], P, M) ? 1 : 0;
+  } else if (op == 4) {
+    out[0] = expected_last_node_tab(a[0], a[1], P, M) ? 1 : 0;
+  }
 }
 
 }  // namespace talc

@@ -828,6 +828,23 @@ __global__ void test_align_slices_kernel(int op, const u8* reads, const u64* rea
       result[i] = r[0];
   }
 }
+// successor-table look-ups as the walks make them (Corrector::next_counts, fast_walk, walk_kernel): one thread per k-mer
+__global__ void test_successors_kernel(CtxView v, int right, u32 K, const u64* kmers, u32 n, u32* cnt, u32* colmask) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+#if defined(__CUDA_ARCH__)  // ctx_lookup exists in the device pass only
+  u32 c4[4], cm;
+  ctx_lookup(v, ctx_of(kmers[i], right != 0, K), c4, cm);
+  for (int q = 0; q < 4; ++q) cnt[4 * i + q] = c4[q];
+  colmask[i] = cm;
+#endif
+}
+// the count model and the fast walks' child choice on the context's own tables (selftest_model_op): one thread per query
+__global__ void test_model_kernel(int op, const u32* args, u32 n, Params P, ModelTabs tabs, u64* out) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  selftest_model_op(op, args + 8 * (u64)i, P, tabs, out + 9 * (u64)i);
+}
 __global__ void test_sort_kernel(const i64* keys, u32 n, u32* perm, void* scratchKeys) {
   if (blockIdx.x != 0 || threadIdx.x != 0) return;
   SortKey* sk = (SortKey*)scratchKeys;
@@ -902,7 +919,6 @@ struct talc_ctx {
       outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases, covRc, strands, orientOut;
 };
 
-static const u32 kModelTabN = 16384;
 static void free_ctx_tables(talc_ctx* c) {
   if (c->ctxRight) cudaFree(c->ctxRight);
   if (c->ctxLeft) cudaFree(c->ctxLeft);
@@ -962,6 +978,12 @@ int talc_ctx_create(const talc_params* p, int cuda_device, talc_ctx** out) {
   *out = nullptr;
   if (p->K < 2 || p->K > 31 || p->min_count < 1 || p->max_nb_branches < 1) {
     g_createError = "invalid parameters (K must be in [2,31])";
+    return TALC_ERR_ARG;
+  }
+  // the walk indexes the count-model tables with lambda = (int)(count * sr_error_rate) <= count (model.cuh), and at
+  // <= 0.5 that product fits an int for every 32-bit count, so the conversion is defined and the same on every host
+  if (!(p->sr_error_rate >= 0.0 && p->sr_error_rate <= 0.5)) {
+    g_createError = "invalid parameters (sr_error_rate must be in [0, 0.5])";
     return TALC_ERR_ARG;
   }
   int ndev = 0;
@@ -2333,6 +2355,53 @@ int talc_test_align_slices(talc_ctx* c, int op, const uint8_t* reads, const uint
   CUDA_TRY(c, cudaMemcpyAsync(result, dRes, rn * 4, cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   cudaFree(dR); cudaFree(dO); cudaFree(dD); cudaFree(dAr); cudaFree(dRes);
+  return TALC_OK;
+}
+
+int talc_test_successors(talc_ctx* c, int right, const uint64_t* kmers, uint32_t n, uint32_t* cnt, uint32_t* colmask,
+                         uint64_t* ctx_capacity) {
+  if (!c || (n && (!kmers || !cnt || !colmask))) return TALC_ERR_ARG;
+  if (c->parent) lane_follow(c);
+  if (!c->tableReady) { c->err = "no k-mer table loaded"; return TALC_ERR_NO_TABLE; }
+  if (ctx_capacity) *ctx_capacity = c->ctxCap;
+  if (!n) return TALC_OK;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  u64* dK;
+  u32 *dC, *dM;
+  CUDA_TRY(c, cudaMalloc((void**)&dK, (size_t)n * 8));
+  CUDA_TRY(c, cudaMalloc((void**)&dC, (size_t)n * 16));
+  CUDA_TRY(c, cudaMalloc((void**)&dM, (size_t)n * 4));
+  CUDA_TRY(c, cudaMemcpyAsync(dK, kmers, (size_t)n * 8, cudaMemcpyHostToDevice, c->stream));
+  const CtxView v{right ? c->ctxRight : c->ctxLeft, c->ctxCap - 1};
+  test_successors_kernel<<<(n + 255) / 256, 256, 0, c->stream>>>(v, right, c->P.K, dK, n, dC, dM);
+  CUDA_TRY(c, cudaGetLastError());
+  CUDA_TRY(c, cudaMemcpyAsync(cnt, dC, (size_t)n * 16, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaMemcpyAsync(colmask, dM, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  cudaFree(dK); cudaFree(dC); cudaFree(dM);
+  return TALC_OK;
+}
+
+int talc_test_model(talc_ctx* c, int op, const uint32_t* args, uint32_t n, uint64_t* out) {
+  if (!c || op < 0 || op > 4 || (n && (!args || !out))) return TALC_ERR_ARG;
+  if (c->parent) lane_follow(c);
+  if (!n) return TALC_OK;
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  u32* dA;
+  u64* dO;
+  CUDA_TRY(c, cudaMalloc((void**)&dA, (size_t)n * 32));
+  CUDA_TRY(c, cudaMalloc((void**)&dO, (size_t)n * 72));
+  CUDA_TRY(c, cudaMemcpyAsync(dA, args, (size_t)n * 32, cudaMemcpyHostToDevice, c->stream));
+  ModelTabs tabs;  // the tables the correction of this context reads (talc_correct_batch)
+  tabs.lower = c->modelTabs;
+  tabs.upper = c->modelTabs + kModelTabN;
+  tabs.sq = c->modelTabs + 2 * kModelTabN;
+  tabs.n = kModelTabN;
+  test_model_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(op, dA, n, c->P, tabs, dO);
+  CUDA_TRY(c, cudaGetLastError());
+  CUDA_TRY(c, cudaMemcpyAsync(out, dO, (size_t)n * 72, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  cudaFree(dA); cudaFree(dO);
   return TALC_OK;
 }
 

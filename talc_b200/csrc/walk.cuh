@@ -30,20 +30,6 @@ struct __attribute__((aligned(16))) ReadCtx {
 static const u32 kCtxFree = 0xFFFFFFFFu;
 
 #if defined(__CUDACC__)
-// exact tagger for a bucket with more than one successor in the graph: -1 unless exactly one is admissible
-__device__ __noinline__ int walk_pick_single_child(const u32 c4[4], u32 cm, u32 count, const Params& P, const ModelTabs& tabs) {
-  u32 col4[4];
-  TALC_ROLLED
-  for (int i = 0; i < 4; ++i) col4[i] = (cm >> i) & 1u;
-  const StepBounds sb = step_bounds_tab(count, P, tabs);
-  u8 tag[4];
-  tag_next_nodes(c4, col4, sb, P, false, tag);
-  int child = -1, n = 0;
-  TALC_ROLLED
-  for (int i = 0; i < 4; ++i)
-    if (tag[i] != kUnexpected) { child = i; ++n; }
-  return n == 1 ? child : -1;
-}
 __device__ __noinline__ double walk_sqrt_cold(u32 c) { return sqrt((double)c); }
 
 __global__ void __launch_bounds__(256) walk_kernel(ReadCtx* __restrict__ ctxs, const u32* __restrict__ walkList, const u32* __restrict__ nWalk,
@@ -68,7 +54,7 @@ __global__ void __launch_bounds__(256) walk_kernel(ReadCtx* __restrict__ ctxs, c
     const bool act = gl < nT;
     const Params P = cx.P;
     const ModelTabs tabs = cx.tabs;
-    const u32 k = P.K, minCount = P.min_count;
+    const u32 k = P.K;
     const bool right = cx.dirRight;
     const bool border = cx.wq.border != 0;
     const CtxView cv = right ? cx.CR : cx.CL;
@@ -106,13 +92,7 @@ __global__ void __launch_bounds__(256) walk_kernel(ReadCtx* __restrict__ ctxs, c
       if (act) {
         u32 c4[4], cm;
         ctx_lookup(cv, right ? (kmer & cmask) : (kmer >> 2), c4, cm);
-        const u32 m = (u32)(c4[0] >= minCount) | ((u32)(c4[1] >= minCount) << 1) | ((u32)(c4[2] >= minCount) << 2) |
-                      ((u32)(c4[3] >= minCount) << 3);
-        if (m != 0 && (m & (m - 1)) == 0) {
-          child = __ffs((int)m) - 1;  // the only successor in the graph: EXPECTED by the counter == 1 rule
-        } else if (m != 0) {
-          child = walk_pick_single_child(c4, cm, count, P, tabs);
-        }
+        child = fast_step_child(c4, cm, count, P, tabs);
         const u32 ch0 = (u32)(child < 0 ? 0 : child);
         childCnt = ch0 == 0 ? c4[0] : ch0 == 1 ? c4[1] : ch0 == 2 ? c4[2] : c4[3];
       }

@@ -825,4 +825,26 @@ int emu_tag_next_nodes(const emu_params* q, const uint32_t* counts4, const uint3
   for (int i = 0; i < n; ++i) { tags4[i] = tag[i] == kExpected ? 0 : tag[i] == kUnexpected ? 1 : 7; dist4[i] = step_dist(count, counts4[i], sb); }
   return n;
 }
+// talc_test_model on the host: use_tabs = 0 runs the computed path (tabs.n = 0, as the emulated corrector does),
+// use_tabs = 1 model tables of kModelTabN counts filled here with model_lower_bound / model_upper_bound
+void emu_test_model(const emu_params* q, int op, const uint32_t* args, uint32_t n, int use_tabs, uint64_t* out) {
+  Params P = to_params(q);
+  std::vector<double> t;
+  ModelTabs M;
+  M.n = 0;
+  M.lower = M.upper = M.sq = nullptr;
+  if (use_tabs) {
+    t.resize(3 * (size_t)kModelTabN);
+    for (u32 c = 0; c < kModelTabN; ++c) {
+      t[c] = model_lower_bound(c, P.alpha);
+      t[kModelTabN + c] = model_upper_bound(c, P.alpha);
+      t[2 * kModelTabN + c] = sqrt((double)c);
+    }
+    M.lower = t.data();
+    M.upper = t.data() + kModelTabN;
+    M.sq = t.data() + 2 * kModelTabN;
+    M.n = kModelTabN;
+  }
+  for (u32 i = 0; i < n; ++i) selftest_model_op(op, args + 8 * (u64)i, P, M, out + 9 * (u64)i);
+}
 }

@@ -66,6 +66,7 @@ def lib():
         L.emu_std_sort_perm.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         L.emu_tag_next_nodes.argtypes = [C.POINTER(EmuParams), C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_void_p,
                                          C.c_void_p]
+        L.emu_test_model.argtypes = [C.POINTER(EmuParams), C.c_int, C.c_void_p, C.c_uint32, C.c_int, C.c_void_p]
         _lib = L
     return _lib
 
@@ -141,3 +142,14 @@ def correct_interleaved(table: EmuTable, reads, offsets, arena_bytes=1 << 20):
     if rc != 0:
         raise RuntimeError("emu output buffer too small")
     return out[: int(ooff[-1])], ooff, status[:n], dict(zip(COUNTER_NAMES, [int(x) for x in ctr]))
+
+
+def test_model(p: EmuParams, op: int, args, use_tabs: bool) -> np.ndarray:
+    """emu_test_model: talc_test_model with the g++ build of the same functions, without (use_tabs=False) or with
+    host-filled model tables; same argument and result layout."""
+    a = np.asarray(args, dtype=np.uint32).reshape(len(args), -1)
+    full = np.zeros((len(a), 8), dtype=np.uint32)
+    full[:, :a.shape[1]] = a
+    out = np.zeros((max(len(a), 1), 9), dtype=np.uint64)
+    lib().emu_test_model(C.byref(p), op, _ptr(full), len(a), 1 if use_tabs else 0, _ptr(out))
+    return out[:len(a)]
