@@ -466,15 +466,20 @@ class Corrector {
   // ------------------------------------------------------------------ Explorer.cpp:402-411
   TALC_HDN void sort_anchors(AnchorRec* a, u32 n) {
     if (n < 2) return;
-    const int cc = (int)(noise / P.sr_error);
+    // std::abs((int)cc - (int)count) as the reference's x86-64 build evaluates it.  At sr_error = 0 the centre is
+    // 0 / 0 = NaN: x86 converts NaN (and any double outside int) to INT_MIN, where the device's conversion gives 0;
+    // the difference then wraps, and |INT_MIN| stays INT_MIN, so an anchor of count 0 sorts first and the others by
+    // descending count.  For a centre inside int and no wrap this is the plain absolute difference.
+    const double q = noise / P.sr_error;
+    const i32 cc = fabs(q) < 2147483648.0 ? (i32)q : INT32_MIN;  // below -2^31 truncation gives INT_MIN as well
     const u32 mk = scratch.mark();
     SortKey* keys = (SortKey*)scratch.alloc(n * sizeof(SortKey));
     AnchorRec* tmp = (AnchorRec*)scratch.alloc(n * sizeof(AnchorRec));
     if (!keys || !tmp) return;
     TALC_ROLLED
     for (u32 i = 0; i < n; ++i) {
-      int d = cc - (int)a[i].count;
-      keys[i].key = d < 0 ? -(i64)d : (i64)d;
+      const u32 d = (u32)cc - a[i].count;
+      keys[i].key = (i64)(i32)((i32)d < 0 ? 0u - d : d);
       keys[i].idx = i;
       tmp[i] = a[i];
     }
