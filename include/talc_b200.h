@@ -15,6 +15,8 @@
  *       <- if (reverse) reverseComplement(seq) before, and of the corrected read after, the above   main.cpp:253,285-286
  *   talc_ctx_set_strand / talc_orient_batch / talc_last_strands / talc_stream_strands
  *       <- not in the reference: the strand chosen per read (--strand auto), for inputs of both orientations
+ *   talc_ctx_set_pieces / talc_pieces_batch / talc_last_pieces / talc_stream_pieces
+ *       <- not in the reference: the table-supported stretches of each corrected read (--trim, --split)
  *   talc_coverage_batch
  *       <- getLRCountsInSR(seq, K, SR_DBG, ..)                                     Jellyfish.cpp:471-496
  *   talc_table_lookup
@@ -267,6 +269,35 @@ int talc_orient_batch(talc_ctx* ctx, const uint8_t* bases, const uint64_t* offse
  * or reverse mode.  dst is a host or a device pointer.  TALC_ERR_ARG when n exceeds that batch.                     */
 int talc_last_strands(talc_ctx* ctx, uint8_t* dst, uint32_t n);
 
+/* Pieces of the corrected reads that the k-mer table supports (not in the reference; talc --trim / --split).  The rule
+ * applies to every read's output, whatever its status.  A window [p, p+K) of the output is solid when its K bytes are
+ * ACGT (either case, U as T) and its k-mer is in the table (count != 0) -- for a read that came back flipped (reverse
+ * mode: status TALC_READ_OK; auto mode: strand 1) the reverse complement of that k-mer, i.e. the strand the read was
+ * corrected on.  A base covered by a solid window is supported; a stretch is a maximal run of supported bases (>= K
+ * bases).  Pieces are 0-based, half-open [start, end) in output coordinates:
+ *   TALC_PIECES_OFF    (default) nothing is computed: no launch and no copy is added to a correction
+ *   TALC_PIECES_TRIM   at most one piece per read, [first supported base, last supported base + 1)
+ *   TALC_PIECES_SPLIT  one piece per stretch
+ * Pieces shorter than min_len (>= 1) are dropped.  Computed on the device after the correction, from the table already
+ * there.  The same rules as talc_ctx_set_strand: set on a context, not on a lane (TALC_ERR_ARG; a lane follows its
+ * parent), not while a stream on the context has batches pending.  Another mode or min_len 0 is TALC_ERR_ARG.       */
+#define TALC_PIECES_OFF 0
+#define TALC_PIECES_TRIM 1
+#define TALC_PIECES_SPLIT 2
+int talc_ctx_set_pieces(talc_ctx* ctx, int mode, uint32_t min_len);
+/* The pieces of the last batch corrected through this context with pieces on (talc_correct_batch(_device), or a
+ * stream's batch on this very context or lane), as CSR over that batch's n reads: piece_off[n+1] (piece_off[0] = 0),
+ * bounds[2*total] = {start, end} per piece, in read order.  Host or device pointers; piece_off may be NULL, bounds may be
+ * NULL when cap is 0.  *total is always set; TALC_ERR_CAPACITY (nothing copied) when total > cap pieces.  TALC_ERR_ARG
+ * when that batch ran with pieces off.                                                                              */
+int talc_last_pieces(talc_ctx* ctx, uint64_t* piece_off, uint32_t* bounds, uint64_t cap, uint64_t* total);
+/* The same rule on any reads, without correcting them (the context's own settings are not used or changed).  Host
+ * buffers: bases, offsets[n_reads+1] with offsets[0] == 0, flip[n_reads] (non-zero: judge the read on its reverse
+ * complement; NULL: none), mode TALC_PIECES_TRIM or _SPLIT, min_len >= 1; piece_off[n_reads+1], bounds[2*cap] and
+ * *total as for talc_last_pieces.  cap = (offsets[n_reads] + n_reads) / (K+1) + 1 is always enough.               */
+int talc_pieces_batch(talc_ctx* ctx, const uint8_t* bases, const uint64_t* offsets, uint32_t n_reads, const uint8_t* flip,
+                      int mode, uint32_t min_len, uint64_t* piece_off, uint32_t* bounds, uint64_t cap, uint64_t* total);
+
 /* ---- streamed correction (replaces loadSeqData / outputSeqData holding every read: main.cpp:219,310, io.cpp:26-75) ----
  * Batches of reads pass through one context with the host-to-device copy of batch i+1, the kernels of batch i, the
  * device-to-host copy of batch i-1 and the caller's own work (FASTA formatting) overlapped: a ring of slots with pinned
@@ -293,6 +324,10 @@ uint64_t talc_stream_pending(talc_stream* s);   /* batches submitted and not yet
  * the stream and valid until the following next / close; NULL for a batch corrected in forward or reverse mode.
  * TALC_ERR_ARG before the first next.                                                                              */
 int talc_stream_strands(talc_stream* s, const uint8_t** strand);
+/* piece_off[n_reads+1] and bounds[2*piece_off[n_reads]] (see talc_ctx_set_pieces) of the batch last returned by
+ * talc_stream_next, in pinned host memory owned by the stream and valid until the following next / close; both NULL
+ * for a batch corrected with pieces off.  TALC_ERR_ARG before the first next.                                      */
+int talc_stream_pieces(talc_stream* s, const uint64_t** piece_off, const uint32_t** bounds);
 const char* talc_stream_last_error(talc_stream* s);
 void talc_stream_close(talc_stream* s);
 

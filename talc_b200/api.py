@@ -39,6 +39,7 @@ STATUS_RESOURCE = 4  # TALC_READ_RESOURCE: passed through uncorrected, not a ref
 STRAND_MODES = {"forward": 0, "reverse": 1, "auto": 2}  # TALC_STRAND_FORWARD / _REVERSE / _AUTO
 SR_SENSE, SR_ANTISENSE, SR_BOTH = 0, 1, 2  # TALC_SR_*: orientation of a short-read file
 DUMP_CANONICAL = 1  # TALC_DUMP_CANONICAL
+PIECE_MODES = {"off": 0, "trim": 1, "split": 2}  # TALC_PIECES_OFF / _TRIM / _SPLIT
 
 _lib = None
 
@@ -63,6 +64,10 @@ def lib():
         L.talc_orient_batch.argtypes = [vp, vp, vp, C.c_uint32, vp, vp, vp]
         L.talc_last_strands.argtypes = [vp, vp, C.c_uint32]
         L.talc_stream_strands.argtypes = [vp, C.POINTER(vp)]
+        L.talc_ctx_set_pieces.argtypes = [vp, C.c_int, C.c_uint32]
+        L.talc_last_pieces.argtypes = [vp, vp, vp, C.c_uint64, u64p]
+        L.talc_pieces_batch.argtypes = [vp, vp, vp, C.c_uint32, vp, C.c_int, C.c_uint32, vp, vp, C.c_uint64, u64p]
+        L.talc_stream_pieces.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
         L.talc_table_load_dump.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_table_load_dump_host.argtypes = [vp, C.c_char_p, C.c_char_p, u64p, u64p]
         L.talc_dump_write_packed.argtypes = [C.c_char_p, vp, vp, C.c_uint64, C.c_uint32]
@@ -202,6 +207,41 @@ class Talc:
         dst = np.zeros(max(n, 1), dtype=np.uint8)
         self._check(lib().talc_last_strands(self.h, _ptr(dst), n), "talc_last_strands")
         return dst[:n]
+
+    def set_pieces(self, mode, min_len: int = 1):
+        """talc --trim / --split: "off", "trim" (one piece per read, first to last table-supported base) or "split" (one
+        piece per supported stretch), or 0 / 1 / 2; pieces shorter than min_len are dropped (talc_ctx_set_pieces).
+        Raises on a lane."""
+        m = PIECE_MODES[mode] if isinstance(mode, str) else int(mode)
+        self._check(lib().talc_ctx_set_pieces(self.h, m, min_len), "talc_ctx_set_pieces")
+
+    def pieces(self, reads: np.ndarray, offsets: np.ndarray, flip=None, mode="split", min_len: int = 1):
+        """The pieces rule on any reads without correcting them (talc_pieces_batch): flip[r] != 0 judges read r on its
+        reverse complement.  Returns (piece_off uint64[n+1], bounds uint32[total, 2] of [start, end))."""
+        reads = np.ascontiguousarray(reads, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = len(offsets) - 1
+        fl = None if flip is None else np.ascontiguousarray(flip, dtype=np.uint8)
+        cap = (int(offsets[-1]) + n) // (self.params.K + 1) + 1
+        po = np.zeros(n + 1, dtype=np.uint64)
+        b = np.zeros((cap, 2), dtype=np.uint32)
+        total = C.c_uint64(0)
+        m = PIECE_MODES[mode] if isinstance(mode, str) else int(mode)
+        self._check(lib().talc_pieces_batch(self.h, _ptr(reads), _ptr(offsets), n, _ptr(fl), m, min_len, _ptr(po), _ptr(b),
+                                            cap, C.byref(total)), "talc_pieces_batch")
+        return po, b[:total.value]
+
+    def last_pieces(self, n: int):
+        """(piece_off uint64[n+1], bounds uint32[total, 2]) of the last batch of n reads corrected through this
+        context with pieces on (talc_last_pieces)."""
+        total = C.c_uint64(0)
+        rc = lib().talc_last_pieces(self.h, None, None, 0, C.byref(total))
+        if rc not in (0, -5):  # TALC_ERR_CAPACITY: total is set
+            self._check(rc, "talc_last_pieces")
+        po = np.zeros(n + 1, dtype=np.uint64)
+        b = np.zeros((max(total.value, 1), 2), dtype=np.uint32)
+        self._check(lib().talc_last_pieces(self.h, _ptr(po), _ptr(b), total.value, C.byref(total)), "talc_last_pieces")
+        return po, b[:total.value]
 
     # ---- table
     def load_dump(self, dump: str, junctions: Optional[str] = None, canonical: bool = False):
@@ -505,6 +545,19 @@ class TalcStream:
         nn = self._n
         st = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint8)), shape=(max(nn, 1),))[:nn]
         return st.copy() if copy else st
+
+    def pieces(self, copy: bool = True):
+        """(piece_off uint64[n+1], bounds uint32[total, 2]) of the batch last returned by next() (talc_stream_pieces),
+        None unless it ran with pieces on; views into the stream's pinned buffers unless copy=True."""
+        po, pb = C.c_void_p(), C.c_void_p()
+        self._check(lib().talc_stream_pieces(self.h, C.byref(po), C.byref(pb)), "talc_stream_pieces")
+        if not po.value:
+            return None
+        nn = self._n
+        off = np.ctypeslib.as_array(C.cast(po, C.POINTER(C.c_uint64)), shape=(nn + 1,))
+        total = int(off[nn])
+        b = np.ctypeslib.as_array(C.cast(pb, C.POINTER(C.c_uint32)), shape=(max(total, 1), 2))[:total]
+        return (off.copy(), b.copy()) if copy else (off, b)
 
     def close(self):
         if self.h:

@@ -202,3 +202,47 @@ static void format_fasta(const Batch& b, const uint8_t* out, const uint64_t* oof
   for (int t = 0; t < nt; ++t) th.emplace_back(work, t);
   for (auto& x : th) x.join();
 }
+
+// --trim / --split: the pieces of one corrected batch as 70-column FASTA records, appended to buf.  pieceOff / bounds
+// hold every supported stretch of each read ([start, end) in output coordinates: talc_stream_pieces of a batch
+// corrected with TALC_PIECES_SPLIT and min_len 1).  trim: one record per read, from its first stretch's start to its
+// last stretch's end, under the read's own header; split: one record per stretch, headed ">{name}_{start}_{end}{rest}"
+// with name the id up to its first blank and rest the remainder of the header.  Pieces shorter than minLen are dropped,
+// and a read without a piece has no record.  tally: reads with a record, records and bases written.
+struct PieceTally {
+  uint64_t reads = 0, pieces = 0, bases = 0;
+};
+static void format_pieces(const Batch& b, const uint8_t* out, const uint64_t* ooffs, const uint64_t* pieceOff, const uint32_t* bounds,
+                          bool split, uint32_t minLen, std::string& buf, PieceTally& tally) {
+  auto record = [&](const std::string& id, const char* suffix, const uint8_t* s, uint64_t len) {
+    const size_t cut = split ? std::min(id.find_first_of(" \t"), id.size()) : id.size();
+    buf += '>';
+    buf.append(id, 0, cut);
+    buf += suffix;
+    buf.append(id, cut, std::string::npos);
+    buf += '\n';
+    for (uint64_t j = 0; j < len; j += 70) {
+      buf.append((const char*)s + j, (size_t)std::min<uint64_t>(70, len - j));
+      buf += '\n';
+    }
+    ++tally.pieces;
+    tally.bases += len;
+  };
+  for (size_t r = 0; r < b.ids.size(); ++r) {
+    const uint64_t p0 = pieceOff[r], p1 = pieceOff[r + 1];
+    const uint8_t* s = out + ooffs[r];
+    const uint64_t before = tally.pieces;
+    if (!split) {
+      if (p1 > p0 && bounds[2 * (p1 - 1) + 1] - bounds[2 * p0] >= minLen)
+        record(b.ids[r], "", s + bounds[2 * p0], bounds[2 * (p1 - 1) + 1] - bounds[2 * p0]);
+    } else {
+      for (uint64_t p = p0; p < p1; ++p) {
+        const uint32_t a = bounds[2 * p], e = bounds[2 * p + 1];
+        if (e - a < minLen) continue;
+        const std::string suffix = "_" + std::to_string(a) + "_" + std::to_string(e);
+        record(b.ids[r], suffix.c_str(), s + a, e - a);
+      }
+    }
+    tally.reads += tally.pieces > before;
+  }
+}

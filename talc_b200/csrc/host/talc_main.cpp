@@ -5,6 +5,7 @@
 //   <prefix>.config.txt (Settings.cpp:160-185)   <prefix>.stats_basics.txt header (Read.cpp:394-415)
 //   <prefix>.log, appended, one line per failed read (io.cpp:105-111; messages main.cpp:290,294)
 //   <prefix>.fa, every read in input order, 70 columns (main.cpp:310, io.cpp:50-75)
+//   <prefix>.trim.fa (--trim), <prefix>.split.fa (--split): extensions, see below
 // Exit codes follow main.cpp: 1 on a parse error (:199) or an empty table (:320), 0 otherwise -- including
 // unreadable input (:323).  The work is done on the GPU through the C ABI; there is no CPU path.
 // -t is accepted for compatibility and used for host-side FASTA formatting only.
@@ -17,6 +18,12 @@
 // by the library, or with peer copies: --replicate peer), --tableCache <file>, --readStats (the per-read rows of Read.cpp:418-433 the reference left disabled
 // at main.cpp:305), --strand forward|reverse|auto (reverse = --reverse; auto chooses each read's strand and also
 // writes <prefix>.strand.txt, one "<id>\t+" or "<id>\t-" line per read in input order).
+// --trim / --split [--minPieceLength N]: the parts of each corrected read that the k-mer table supports, computed on the
+// GPU (talc_ctx_set_pieces): a base is supported when a K-mer window of the output over it is in the table, on the strand
+// the read was corrected on.  --trim writes <prefix>.trim.fa, each read from its first to its last supported base under
+// its own header; --split writes <prefix>.split.fa, one record per maximal run of supported bases, headed
+// ">{name}_{start}_{end}{rest}" (0-based, half-open).  Pieces shorter than N (default 1) are dropped, and so are reads
+// without a piece.  Both may be given; every other output file is the same with and without them.
 // The k-mer table comes from exactly one of
 //   --SRCounts <dump> [--SRCanonical]   a Jellyfish `dump -c`; --SRCanonical: a `jellyfish count -C` dump, each line
 //                                       (x, c) also standing for (rc(x), c)
@@ -49,7 +56,8 @@
 
 struct Cli {
   std::string reads, dump, junctions, out = "out", queryMode = "memory", tableCache, replicate = "nccl", strand;
-  bool useJunctions = false, reverse = false, readStats = false;
+  bool useJunctions = false, reverse = false, readStats = false, trim = false, split = false, haveMinPiece = false;
+  long minPiece = 1;
   int threads = 1, gpus = 1, strandMode = TALC_STRAND_FORWARD;
   long batchReads = 131072, batchBases = 256l << 20;
   talc_params p;
@@ -121,6 +129,9 @@ static int parse(int argc, const char** argv, Cli& c) {
     else if (a == "-rev" || a == "--reverse") { c.reverse = true; }
     else if (a == "--strand") { if (!val(c.strand) || (c.strand != "forward" && c.strand != "reverse" && c.strand != "auto")) return 1; }
     else if (a == "--readStats") { c.readStats = true; }
+    else if (a == "--trim") { c.trim = true; }
+    else if (a == "--split") { c.split = true; }
+    else if (a == "--minPieceLength") { if (!val(v) || !to_int(v, n) || n < 1 || n > 0xFFFFFFFFl) return 1; c.minPiece = n; c.haveMinPiece = true; }
     else if (a == "--batch-reads") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.batchReads = n; }
     else if (a == "--batch-bases") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.batchBases = n; }
     else if (a == "--gpus") { if (!val(v) || !to_int(v, n) || n < 1) return 1; c.gpus = (int)n; }
@@ -134,6 +145,7 @@ static int parse(int argc, const char** argv, Cli& c) {
   if (!c.srReads2.empty() && c.srReads2.size() != c.srReads.size()) return 1;  // one R2 per R1
   if (counting && (c.srCanonical || !c.tableCache.empty())) return 1;
   if (c.reverse && !c.strand.empty() && c.strand != "reverse") return 1;  // --reverse is --strand reverse
+  if (c.haveMinPiece && !c.trim && !c.split) return 1;
   c.strandMode = (c.reverse || c.strand == "reverse") ? TALC_STRAND_REVERSE : c.strand == "auto" ? TALC_STRAND_AUTO : TALC_STRAND_FORWARD;
   if (c.queryMode != "memory") { std::cerr << "talc: only query mode 'memory' is supported\n"; return 1; }
   c.reads = pos[0];
@@ -175,11 +187,14 @@ int main(int argc, const char** argv) {
   const int pr = parse(argc, argv, cli);
   if (pr == 2) {
     std::cout << "talc <reads> --SRCounts <dump> [--junctions <dump>] -k <K> [-o <prefix>] [-t <N>] [--reverse | --strand forward|reverse|auto] [--gpus <N>] [--tableCache <file>]"
-                 " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer]\n"
+                 " [--batch-reads <N>] [--batch-bases <N>] [--readStats] [--replicate nccl|peer] [--trim] [--split] [--minPieceLength <N>]\n"
                  "  the k-mer table: --SRCounts <dump> [--SRCanonical] (a `jellyfish count -C` dump: each k-mer also stands for its"
                  " reverse complement)\n"
                  "               or --SRReads <fq|fa> ... [--SRReads2 <fq|fa> ...] [--SRLibType asis|unstranded|fr-firststrand|fr-secondstrand]"
-                 " [--SRExpected <N>] (counted on the GPU; --SRReads2: R2 mates, one per --SRReads)\n";
+                 " [--SRExpected <N>] (counted on the GPU; --SRReads2: R2 mates, one per --SRReads)\n"
+                 "  --trim / --split: also write <prefix>.trim.fa (each read from its first to its last base supported by the"
+                 " table) / <prefix>.split.fa (one record per supported stretch, >{name}_{start}_{end}); --minPieceLength:"
+                 " drop shorter pieces (default 1)\n";
     return 0;
   }
   if (pr != 0) { std::cerr << "talc: PARSE_ERROR\n"; return 1; }
@@ -211,6 +226,11 @@ int main(int argc, const char** argv) {
     }
     // --reverse (main.cpp:253,285-286) / --strand: the long reads only; the stream's lanes follow their context
     if (cli.strandMode != TALC_STRAND_FORWARD && talc_ctx_set_strand(ctx[g], cli.strandMode) != 0) {
+      std::cerr << "talc: " << talc_last_error(ctx[g]) << "\n";
+      return 2;
+    }
+    // every stretch of every read; the writer cuts the --trim and --split records from them
+    if ((cli.trim || cli.split) && talc_ctx_set_pieces(ctx[g], TALC_PIECES_SPLIT, 1) != 0) {
       std::cerr << "talc: " << talc_last_error(ctx[g]) << "\n";
       return 2;
     }
@@ -311,6 +331,15 @@ int main(int argc, const char** argv) {
   const std::string faTmp = cli.out + ".fa.partial";
   FILE* fo = fopen(faTmp.c_str(), "wb");
   if (!fo) { std::cerr << "ERROR: Could not open the file " << cli.out << ".fa\n"; return 0; }
+  // --trim / --split: written the same way, next to it
+  const std::string trimTmp = cli.out + ".trim.fa.partial", splitTmp = cli.out + ".split.fa.partial";
+  FILE* ft = cli.trim ? fopen(trimTmp.c_str(), "wb") : nullptr;
+  FILE* fs = cli.split ? fopen(splitTmp.c_str(), "wb") : nullptr;
+  if ((cli.trim && !ft) || (cli.split && !fs)) {
+    std::cerr << "ERROR: Could not open the file " << cli.out << (cli.trim && !ft ? ".trim.fa" : ".split.fa") << "\n";
+    return 0;
+  }
+  PieceTally trimTally, splitTally;
   IdQueue idq;
   int writerRc = 0;
   uint64_t nReads = 0, nResource = 0;
@@ -369,6 +398,26 @@ int main(int argc, const char** argv) {
       t0 = std::chrono::steady_clock::now();
       for (const auto& p : parts) fwrite(p.data(), 1, p.size(), fo);
       sWrite += since(t0);
+      if (ft || fs) {
+        const uint64_t* pieceOff = nullptr;
+        const uint32_t* bounds = nullptr;
+        if (talc_stream_pieces(s, &pieceOff, &bounds) != 0 || !pieceOff) {
+          std::cerr << "talc: no pieces for a batch on device " << (b->seq % cli.gpus) << "\n";
+          writerRc = 2;
+          while (idq.pop()) {}
+          return;
+        }
+        std::string buf;
+        if (ft) {
+          format_pieces(*b, out, ooffs, pieceOff, bounds, false, (uint32_t)cli.minPiece, buf, trimTally);
+          fwrite(buf.data(), 1, buf.size(), ft);
+          buf.clear();
+        }
+        if (fs) {
+          format_pieces(*b, out, ooffs, pieceOff, bounds, true, (uint32_t)cli.minPiece, buf, splitTally);
+          fwrite(buf.data(), 1, buf.size(), fs);
+        }
+      }
       nReads += n;
     }
   });
@@ -404,6 +453,8 @@ int main(int argc, const char** argv) {
   idq.finish();
   writer.join();
   fclose(fo);
+  if (ft) fclose(ft);
+  if (fs) fclose(fs);
   const double sCorr = since(tCorr);
   // error paths release everything in order; a complete run leaves the buffers to the process exit (unpinning and
   // freeing several GB per device one allocation at a time took 0.3 s on one GPU and 2.5 s on two)
@@ -412,9 +463,14 @@ int main(int argc, const char** argv) {
     for (auto* c : ctx) talc_ctx_destroy(c);
   };
   if (submitRc || writerRc || !inputOk) teardown();
-  if (submitRc || writerRc) { remove(faTmp.c_str()); return 2; }
+  auto dropPieces = [&]() {
+    if (ft) remove(trimTmp.c_str());
+    if (fs) remove(splitTmp.c_str());
+  };
+  if (submitRc || writerRc) { remove(faTmp.c_str()); dropPieces(); return 2; }
   if (!inputOk) {  // the reference would have failed while loading, before writing anything
     remove(faTmp.c_str());
+    dropPieces();
     std::cout << "[TALC]: ISSUE WITH INPUT FILES" << std::endl;
     return 0;
   }
@@ -422,7 +478,18 @@ int main(int argc, const char** argv) {
     std::cerr << "ERROR: Could not open the file " << cli.out << ".fa\n";
     return 0;
   }
+  if ((ft && rename(trimTmp.c_str(), (cli.out + ".trim.fa").c_str()) != 0) ||
+      (fs && rename(splitTmp.c_str(), (cli.out + ".split.fa").c_str()) != 0)) {
+    std::cerr << "ERROR: Could not write the pieces of " << cli.out << "\n";
+    return 0;
+  }
   std::cout << "[TALC]: " << nReads << " long read(s) processed" << std::endl;
+  if (ft)
+    std::cout << "[TALC]: --trim: " << trimTally.reads << " read(s) kept, " << trimTally.pieces << " piece(s), " << trimTally.bases
+              << " bases" << std::endl;
+  if (fs)
+    std::cout << "[TALC]: --split: " << splitTally.reads << " read(s) kept, " << splitTally.pieces << " piece(s), "
+              << splitTally.bases << " bases" << std::endl;
   std::cout << "[TALC]: seconds: contexts " << sCtx << ", table " << sTable << ", replication " << sRep << ", staging " << sOpen << ", correction (read + correct + write) "
             << sCorr << " [reader: parse " << sParse << ", submit " << sSubmit << "; writer: wait " << sWait << ", format " << sFormat
             << ", write " << sWrite << "]" << std::endl;

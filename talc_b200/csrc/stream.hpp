@@ -59,9 +59,10 @@ struct PinBuf {
 };
 
 struct StreamSlot {
-  PinBuf hBases, hOffs, hOut, hOutOffs, hStatus, hStats, hStrand;
+  PinBuf hBases, hOffs, hOut, hOutOffs, hStatus, hStats, hStrand, hPieceOff, hBounds;
   DevBuf dBases, dOffs, dOut, dOutOffs, dStatus, dStats, dStrand;
   bool strandAuto = false;  // the batch ran in TALC_STRAND_AUTO: hStrand holds its strands
+  bool pieces = false;      // the batch ran with pieces on: hPieceOff / hBounds hold them
   cudaEvent_t h2dDone = nullptr, d2hDone = nullptr;
   u32 n = 0;
   u64 totalBases = 0;
@@ -117,6 +118,20 @@ static void stream_worker(talc_stream* s, int w) {
                                      sl->dOut.cap, (u64*)sl->dOutOffs.p, (u8*)sl->dStatus.p, &sl->ctr,
                                      s->wantStats ? (u32*)sl->dStats.p : nullptr, strandAuto ? (u8*)sl->dStrand.p : nullptr);
     sl->strandAuto = rc == TALC_OK && c->lastAuto;
+    sl->pieces = rc == TALC_OK && c->lastPieces;
+    if (sl->pieces) {
+      // the pieces are small (8 bytes a read and a piece) and the context's buffers serve the next batch of this
+      // lane: copied out here, on the lane's idle stream, before the next batch is queued
+      const u64 total = c->lastPiecesTotal;
+      if (sl->hPieceOff.reserve((size_t)(sl->n + 1) * 8) != cudaSuccess || sl->hBounds.reserve((size_t)total * 8 + 8) != cudaSuccess) {
+        rc = TALC_ERR_CUDA;
+        c->err = "out of pinned host memory for the pieces of a batch";
+      } else {
+        u64 got = 0;
+        rc = talc_last_pieces(c, (uint64_t*)sl->hPieceOff.p, (uint32_t*)sl->hBounds.p, total, &got);
+      }
+      sl->pieces = rc == TALC_OK;
+    }
     if (rc == TALC_OK) {
       // this lane's compute stream is idle here (the call above ends with a synchronize): results leave on the
       // copy-out stream while the next batch computes
@@ -281,6 +296,17 @@ int talc_stream_next(talc_stream* s, const uint8_t** out, const uint64_t** out_o
 }
 
 // the slot handed out by the last talc_stream_next stays in state 3 until the following call
+int talc_stream_pieces(talc_stream* s, const uint64_t** piece_off, const uint32_t** bounds) {
+  if (!s || !piece_off || !bounds) return TALC_ERR_ARG;
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (s->seqFetch == 0) { s->err = "talc_stream_pieces: no batch returned yet"; return TALC_ERR_ARG; }
+  const StreamSlot* sl = &s->slot[(s->seqFetch - 1) % s->kSlots];
+  const bool ok = sl->state == 3 && sl->rc == TALC_OK && sl->pieces;
+  *piece_off = ok ? (const uint64_t*)sl->hPieceOff.p : nullptr;
+  *bounds = ok ? (const uint32_t*)sl->hBounds.p : nullptr;
+  return TALC_OK;
+}
+
 int talc_stream_strands(talc_stream* s, const uint8_t** strand) {
   if (!s || !strand) return TALC_ERR_ARG;
   std::lock_guard<std::mutex> lk(s->mu);
@@ -306,7 +332,7 @@ void talc_stream_close(talc_stream* s) {
   cudaStreamSynchronize(s->copyIn);
   cudaStreamSynchronize(s->copyOut);
   for (auto& sl : s->slot) {
-    PinBuf* hb[] = {&sl.hBases, &sl.hOffs, &sl.hOut, &sl.hOutOffs, &sl.hStatus, &sl.hStats, &sl.hStrand};
+    PinBuf* hb[] = {&sl.hBases, &sl.hOffs, &sl.hOut, &sl.hOutOffs, &sl.hStatus, &sl.hStats, &sl.hStrand, &sl.hPieceOff, &sl.hBounds};
     for (PinBuf* b : hb) b->release();
     DevBuf* db[] = {&sl.dBases, &sl.dOffs, &sl.dOut, &sl.dOutOffs, &sl.dStatus, &sl.dStats, &sl.dStrand};
     for (DevBuf* b : db) b->release();

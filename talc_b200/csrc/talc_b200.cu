@@ -10,6 +10,8 @@
 //   revcomp_reads_kernel                                                --reverse: every read reverse-complemented first
 //   orient_kernel                                                       --strand auto: both strands probed, each read's
 //                                                                       strand chosen, in place of coverage_kernel
+//   pieces_kernel + pieces_compact_kernel                               --trim / --split: table-supported stretches of
+//                                                                       the output, after gather_kernel
 // Grid sizes are multiples of the SM count; per-thread scratch lives in HBM (180 GB makes that cheap).
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -688,6 +690,9 @@ __global__ void revcomp_reads_kernel(const u8* __restrict__ in, const u64* __res
 // corrected reads from allocation order into input order; one warp per read.  A read is flipped back to the input's
 // strand per read: in reverse mode when it was corrected (main.cpp:285-286; every other read leaves as its reverse-
 // complemented input, Q24), in auto mode when it was corrected on the reverse strand (strand[r] == 1), whatever its status
+__device__ __forceinline__ bool output_flip(u32 mode, const u8* __restrict__ strand, const u8* __restrict__ status, u32 r) {
+  return mode == TALC_STRAND_AUTO ? strand[r] != 0 : mode == TALC_STRAND_REVERSE && status[r] == TALC_READ_OK;
+}
 __global__ void gather_kernel(const u8* __restrict__ arena, const u64* __restrict__ pos, const u32* __restrict__ len,
                               const u64* __restrict__ outOff, u32 n, u8* __restrict__ out, const u8* __restrict__ status,
                               const u8* __restrict__ strand, u32 mode) {
@@ -697,7 +702,7 @@ __global__ void gather_kernel(const u8* __restrict__ arena, const u64* __restric
     const u8* src = arena + pos[r];
     u8* dst = out + outOff[r];
     const u32 L = len[r];
-    const bool flip = mode == TALC_STRAND_AUTO ? strand[r] != 0 : mode == TALC_STRAND_REVERSE && status[r] == TALC_READ_OK;
+    const bool flip = output_flip(mode, strand, status, r);
     if (flip)
       for (u32 i = lane; i < L; i += 32) dst[i] = dna5_complement(src[L - 1 - i]);
     else
@@ -707,6 +712,156 @@ __global__ void gather_kernel(const u8* __restrict__ arena, const u64* __restric
 __global__ void len_to_u64_kernel(const u32* len, u32 n, u64* out) {
   const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = len[i];
+}
+
+// --trim / --split: the stretches of each output read that the table supports.  A window [p, p+K) is solid when its K
+// bytes are ACGT (base_code) and its k-mer -- its reverse complement when the read was flipped back (output_flip), the
+// strand the read was corrected on -- is in the table; a stretch is a maximal run of bases covered by solid windows,
+// i.e. a group of solid windows each at most K after the previous one, [first p, last p + K).  The layout of
+// coverage_kernel: one warp per read, four windows per lane, 128 windows per chunk, the four home-sector fetches issued
+// together.  The chunk's solid windows become a 128-bit mask in every lane; a solid window opens a stretch when the
+// previous solid window -- in the mask, else the last one of the earlier chunks (the carry) -- is more than K before it,
+// and the lane that opens stretch j closes stretch j-1 at that previous window + K.  Stretches are >= K long with a gap
+// between them, so a read of L bases has at most (L+1)/(K+1) of them and read r writes its (start, end) pairs from pair
+// (ooff[r] + r) / (K+1) of `raw` on, clear of every other read.  The warp then keeps, in place, the pieces of pieceMode:
+// every stretch of >= minLen bases (TALC_PIECES_SPLIT) or [first start, last end) if >= minLen (TALC_PIECES_TRIM), and
+// writes their number to count[r].
+__global__ void __launch_bounds__(256) pieces_kernel(TableView tv, u32 K, const u8* __restrict__ out,
+                                                     const u64* __restrict__ ooff, u32 n, const u8* __restrict__ status,
+                                                     const u8* __restrict__ strand, u32 strandMode, u32 pieceMode,
+                                                     u32 minLen, u32* __restrict__ raw, u64* __restrict__ count) {
+  const u32 lane = threadIdx.x & 31;
+  const u32 warpsPerBlock = blockDim.x >> 5;
+  const u64 kmask = kmer_mask(K);
+  for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
+    const u64 o = ooff[r];
+    const u32 len = (u32)(ooff[r + 1] - o);
+    const u32 C = len >= K ? len - K + 1 : 0;
+    const bool flip = output_flip(strandMode, strand, status, r);
+    const u8* s = out + o;
+    u32* reg = raw + 2 * ((o + r) / (K + 1));
+    u32 nStr = 0;                   // stretches opened so far
+    u32 last = 0;                   // the last solid window so far, when `any`
+    bool any = false;
+    for (u32 base = 0; base < C; base += 128) {
+      const u32 p0 = base + lane * 4;
+      u32 nib = 0;  // bit q: window p0 + q is solid
+      if (p0 < C) {
+        u64 km = 0, rk = 0;
+        u32 run = 0;  // bases since the last non-ACGT byte
+        for (u32 j = 0; j < K; ++j) {
+          const u32 c = base_code(__ldg(s + p0 + j));
+          run = (c > 3) ? 0 : (run + 1);
+          km = ((km << 2) | (c & 3)) & kmask;
+          rk = kmer_roll_rc(rk, c, K);
+        }
+        u64 kms[4];
+        u32 okm = 0;
+#pragma unroll
+        for (u32 q = 0; q < 4; ++q) {
+          if (q > 0 && p0 + q < C) {
+            const u32 c = base_code(__ldg(s + p0 + q + K - 1));
+            run = (c > 3) ? 0 : (run + 1);
+            km = ((km << 2) | (c & 3)) & kmask;
+            rk = kmer_roll_rc(rk, c, K);
+          }
+          kms[q] = flip ? rk : km;
+          okm |= (p0 + q < C && run >= K) ? (1u << q) : 0u;
+        }
+        Slot s0[4], s1[4];
+        u64 b[4];
+#pragma unroll
+        for (u32 q = 0; q < 4; ++q) {
+          b[q] = hash_kmer(kms[q]) & tv.mask & ~1ull;
+          if ((okm >> q) & 1u) load_sector(tv.slots + b[q], s0[q], s1[q]);
+        }
+#pragma unroll
+        for (u32 q = 0; q < 4; ++q) {
+          if ((okm >> q) & 1u) {
+            u32 cnt = 0, col;
+            if (sector_resolve(s0[q], s1[q], kms[q], cnt, col) < 0) table_probe_from(tv, b[q], kms[q], cnt, col);
+            nib |= cnt != 0 ? (1u << q) : 0u;
+          }
+        }
+      }
+      // the chunk's 128 windows as four 32-bit words, in every lane (word w: the nibbles of lanes 8w .. 8w+7)
+      u32 w[4];
+#pragma unroll
+      for (u32 i = 0; i < 4; ++i) w[i] = __reduce_or_sync(0xffffffffu, (lane >> 3) == i ? nib << (4 * (lane & 7)) : 0u);
+      u32 starts = 0, prevOf[4];
+#pragma unroll
+      for (u32 q = 0; q < 4; ++q) {
+        if (!((nib >> q) & 1u)) continue;
+        const u32 idx = lane * 4 + q;
+        bool has = false;
+        u32 prev = 0;
+        for (i32 wi = (i32)(idx >> 5); wi >= 0 && !has; --wi) {
+          const u32 m = wi == (i32)(idx >> 5) ? w[wi] & ((1u << (idx & 31)) - 1u) : w[wi];
+          if (m) { has = true; prev = base + 32 * (u32)wi + 31 - (u32)__clz((int)m); }
+        }
+        if (!has && any) { has = true; prev = last; }
+        if (!has || p0 + q - prev > K) { starts |= 1u << q; prevOf[q] = has ? prev : 0xFFFFFFFFu; }
+      }
+      // stretch index of this lane's first start: the starts of the lower lanes, after the nStr of earlier chunks
+      const u32 mine = __popc(starts);
+      u32 incl = mine;
+#pragma unroll
+      for (u32 d = 1; d < 32; d <<= 1) {
+        const u32 t = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += t;
+      }
+      u32 j = nStr + incl - mine;
+#pragma unroll
+      for (u32 q = 0; q < 4; ++q) {
+        if (!((starts >> q) & 1u)) continue;
+        if (prevOf[q] != 0xFFFFFFFFu) reg[2 * (j - 1) + 1] = prevOf[q] + K;
+        reg[2 * j] = p0 + q;
+        ++j;
+      }
+      nStr += __shfl_sync(0xffffffffu, incl, 31);
+      for (i32 wi = 3; wi >= 0; --wi)
+        if (w[wi]) { last = base + 32 * (u32)wi + 31 - (u32)__clz((int)w[wi]); any = true; break; }
+    }
+    if (any && lane == 0) reg[2 * (nStr - 1) + 1] = last + K;
+    __syncwarp();
+    if (pieceMode == TALC_PIECES_TRIM) {
+      if (lane == 0) {
+        const bool keep = nStr && reg[2 * nStr - 1] - reg[0] >= minLen;
+        if (keep) reg[1] = reg[2 * nStr - 1];
+        count[r] = keep ? 1 : 0;
+      }
+    } else {
+      u32 kept = 0;
+      for (u32 i0 = 0; i0 < nStr; i0 += 32) {  // in place: pair i moves to kept + (pairs kept before it) <= i
+        const u32 i = i0 + lane;
+        u32 a = 0, e = 0;
+        if (i < nStr) { a = reg[2 * i]; e = reg[2 * i + 1]; }
+        const bool keep = i < nStr && e - a >= minLen;
+        const u32 m = __ballot_sync(0xffffffffu, keep);
+        __syncwarp();
+        if (keep) {
+          const u32 at = kept + __popc(m & ((1u << lane) - 1u));
+          reg[2 * at] = a;
+          reg[2 * at + 1] = e;
+        }
+        kept += __popc(m);
+        __syncwarp();
+      }
+      if (lane == 0) count[r] = kept;
+    }
+  }
+}
+// the pieces of each read from its region of `raw` to bounds[2 * pieceOff[r] ..] (CSR); one warp per read
+__global__ void pieces_compact_kernel(const u32* __restrict__ raw, const u64* __restrict__ ooff, const u64* __restrict__ pieceOff,
+                                      u32 n, u32 K, u32* __restrict__ bounds) {
+  const u32 lane = threadIdx.x & 31;
+  const u32 warpsPerBlock = blockDim.x >> 5;
+  for (u32 r = blockIdx.x * warpsPerBlock + (threadIdx.x >> 5); r < n; r += gridDim.x * warpsPerBlock) {
+    const u32* src = raw + 2 * ((ooff[r] + r) / (K + 1));
+    u32* dst = bounds + 2 * pieceOff[r];
+    const u64 m = 2 * (pieceOff[r + 1] - pieceOff[r]);
+    for (u64 i = lane; i < m; i += 32) dst[i] = src[i];
+  }
 }
 
 __global__ void model_tabs_kernel(double alpha, u32 n, double* lower, double* upper, double* sq) {
@@ -912,11 +1067,15 @@ struct talc_ctx {
                                      // strand, from the oriented copy in rcBases
   u32 lastN = 0;                     // the last batch corrected through this context (talc_last_strands):
   bool lastAuto = false;             // its size, and whether its decisions are in `strands`
+  u32 pieces = TALC_PIECES_OFF;      // talc_ctx_set_pieces
+  u32 piecesMinLen = 1;
+  bool lastPieces = false;           // the last batch left its pieces in pieceOff / pieceBounds (talc_last_pieces)
+  u64 lastPiecesTotal = 0;
   u64 lastRounds = 0;
   double* modelTabs = nullptr;  // 3 x kModelTabN doubles
   // cached device buffers
   DevBuf bases, offs, kmerOff, nk, cov, order, sortKey, sortKeyOut, sortVal, cubTmp, arenas, outArena, outPos, outLen,
-      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases, covRc, strands, orientOut;
+      outLen64, status, outOffs, out, misc, overflowList, readCtxs, roundLists, rcBases, covRc, strands, orientOut, pieceRaw, pieceCnt, pieceOff, pieceBounds;
 };
 
 static void free_ctx_tables(talc_ctx* c) {
@@ -1046,7 +1205,7 @@ void talc_ctx_destroy(talc_ctx* c) {
   DevBuf* bufs[] = {&c->bases, &c->offs, &c->kmerOff, &c->nk, &c->cov, &c->order, &c->sortKey, &c->sortKeyOut, &c->sortVal,
                     &c->cubTmp, &c->arenas, &c->outArena, &c->outPos, &c->outLen, &c->outLen64, &c->status, &c->outOffs,
                     &c->out, &c->misc, &c->overflowList, &c->readCtxs, &c->roundLists, &c->rcBases, &c->covRc,
-                    &c->strands, &c->orientOut};
+                    &c->strands, &c->orientOut, &c->pieceRaw, &c->pieceCnt, &c->pieceOff, &c->pieceBounds};
   for (DevBuf* b : bufs) b->release();
   for (int i = 0; i < 8; ++i) cudaEventDestroy(c->ev[i]);
   cudaStreamDestroy(c->stream);
@@ -1081,6 +1240,8 @@ static void lane_follow(talc_ctx* sh) {
   sh->inlineInner = c->inlineInner;
   sh->inlineBorder = c->inlineBorder;
   sh->strand = c->strand;
+  sh->pieces = c->pieces;
+  sh->piecesMinLen = c->piecesMinLen;
 }
 int talc_ctx_create_lane(talc_ctx* parent, talc_ctx** out) {
   if (!parent || !out || parent->parent) return TALC_ERR_ARG;
@@ -1123,6 +1284,19 @@ int talc_ctx_set_strand(talc_ctx* c, int mode) {
 }
 int talc_ctx_set_reverse(talc_ctx* c, int reverse) {
   return talc_ctx_set_strand(c, reverse ? TALC_STRAND_REVERSE : TALC_STRAND_FORWARD);
+}
+
+// --trim / --split.  A lane follows its parent, as with the strand.
+int talc_ctx_set_pieces(talc_ctx* c, int mode, uint32_t min_len) {
+  if (!c) return TALC_ERR_ARG;
+  if (c->parent) { c->err = "a lane follows the pieces setting of the context it was made from"; return TALC_ERR_ARG; }
+  if ((mode != TALC_PIECES_OFF && mode != TALC_PIECES_TRIM && mode != TALC_PIECES_SPLIT) || min_len == 0) {
+    c->err = "pieces mode must be TALC_PIECES_OFF, TALC_PIECES_TRIM or TALC_PIECES_SPLIT, min_len at least 1";
+    return TALC_ERR_ARG;
+  }
+  c->pieces = (u32)mode;
+  c->piecesMinLen = min_len;
+  return TALC_OK;
 }
 
 // ---------------------------------------------------------------------------------- table
@@ -1887,6 +2061,34 @@ static int run_pass(talc_ctx* c, CorrectArgs& A, u32 nCtx, u64* launches) {
   return TALC_OK;
 }
 
+// ---------------------------------------------------------------------------------- pieces
+// pieces_kernel over n output reads (dOut, dOutOffs[n+1], totalOut bases), then the CSR: pieceOff[n+1], pieceBounds.
+// Queued on the context's stream; pieceOff[n] is copied to *hTotal, valid after the next synchronize.
+static int run_pieces(talc_ctx* c, const u8* dOut, const u64* dOutOffs, u32 n, u64 totalOut, const u8* dStatus,
+                      const u8* dStrand, u32 strandMode, u32 mode, u32 minLen, u64* hTotal) {
+  const u32 K = c->params.K;
+  const u64 pairs = (totalOut + n) / (K + 1) + 1;  // read r writes from pair (ooff[r] + r) / (K+1) on
+  CUDA_TRY(c, c->pieceRaw.reserve((size_t)pairs * 8));
+  CUDA_TRY(c, c->pieceBounds.reserve((size_t)pairs * 8));
+  CUDA_TRY(c, c->pieceCnt.reserve((size_t)(n + 1) * 8));
+  CUDA_TRY(c, c->pieceOff.reserve((size_t)(n + 1) * 8));
+  const int blocks = c->sms * 8;
+  pieces_kernel<<<blocks, 256, 0, c->stream>>>(TableView{c->slots, c->capacity - 1}, K, dOut, dOutOffs, n, dStatus, dStrand,
+                                               strandMode, mode, minLen, (u32*)c->pieceRaw.p, (u64*)c->pieceCnt.p);
+  CUDA_TRY(c, cudaGetLastError());
+  CUDA_TRY(c, cudaMemsetAsync((u64*)c->pieceCnt.p + n, 0, 8, c->stream));
+  size_t tb = 0;
+  CUDA_TRY(c, cub::DeviceScan::ExclusiveSum(nullptr, tb, (u64*)c->pieceCnt.p, (u64*)c->pieceOff.p, n + 1, c->stream));
+  CUDA_TRY(c, c->cubTmp.reserve(tb));
+  tb = c->cubTmp.cap;
+  CUDA_TRY(c, cub::DeviceScan::ExclusiveSum(c->cubTmp.p, tb, (u64*)c->pieceCnt.p, (u64*)c->pieceOff.p, n + 1, c->stream));
+  pieces_compact_kernel<<<blocks, 256, 0, c->stream>>>((const u32*)c->pieceRaw.p, dOutOffs, (const u64*)c->pieceOff.p, n, K,
+                                                       (u32*)c->pieceBounds.p);
+  CUDA_TRY(c, cudaGetLastError());
+  CUDA_TRY(c, cudaMemcpyAsync(hTotal, (const u64*)c->pieceOff.p + n, 8, cudaMemcpyDeviceToHost, c->stream));
+  return TALC_OK;
+}
+
 // ---------------------------------------------------------------------------------- correction
 // shared front end: k-mer offsets, length-sorted order, coverage.  d_bases/d_offs on device.  In reverse mode the reads
 // are first reverse-complemented into rcBases (same offsets) and dBases is pointed there for the rest of the batch.  In
@@ -1970,10 +2172,17 @@ static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const u
   const u32 mode = c->strand;
   c->lastN = 0;
   c->lastAuto = false;
+  c->lastPieces = false;
+  c->lastPiecesTotal = 0;
   if (n == 0) {
     if (dOutOffs) CUDA_TRY(c, cudaMemsetAsync(dOutOffs, 0, 8, c->stream));
+    if (c->pieces != TALC_PIECES_OFF) {
+      CUDA_TRY(c, c->pieceOff.reserve(8));
+      CUDA_TRY(c, cudaMemsetAsync(c->pieceOff.p, 0, 8, c->stream));
+    }
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     c->lastAuto = mode == TALC_STRAND_AUTO;
+    c->lastPieces = c->pieces != TALC_PIECES_OFF;
     return TALC_OK;
   }
   CUDA_TRY(c, cudaEventRecord(c->ev[0], c->stream));
@@ -2091,9 +2300,17 @@ static int correct_batch_device_impl(talc_ctx* c, const uint8_t* dBases, const u
   CUDA_TRY(c, cudaEventRecord(c->ev[5], c->stream));
   if (mode == TALC_STRAND_AUTO && dStrandOut)
     CUDA_TRY(c, cudaMemcpyAsync(dStrandOut, c->strands.p, n, cudaMemcpyDeviceToDevice, c->stream));
+  u64 hPieces = 0;
+  if (c->pieces != TALC_PIECES_OFF) {  // after the gather, on the bytes it wrote; the correction's timings end before
+    const int rcp = run_pieces(c, dOut, dOutOffs, n, hTotalOut, dStatus, (const u8*)c->strands.p, mode, c->pieces,
+                               c->piecesMinLen, &hPieces);
+    if (rcp) return rcp;
+  }
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   c->lastN = n;
   c->lastAuto = mode == TALC_STRAND_AUTO;
+  c->lastPieces = c->pieces != TALC_PIECES_OFF;
+  c->lastPiecesTotal = hPieces;
   if (dbg) {
     std::vector<u32> kc(n);
     std::vector<u64> ho(n + 1);
@@ -2239,6 +2456,58 @@ int talc_last_strands(talc_ctx* c, uint8_t* dst, uint32_t n) {
     CUDA_TRY(c, cudaMemsetAsync(c->strands.p, 0, n, c->stream));
   }
   CUDA_TRY(c, cudaMemcpyAsync(dst, c->strands.p, n, cudaMemcpyDefault, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return TALC_OK;
+}
+
+int talc_last_pieces(talc_ctx* c, uint64_t* piece_off, uint32_t* bounds, uint64_t cap, uint64_t* total) {
+  if (!c || !total || (cap && !bounds)) return TALC_ERR_ARG;
+  if (!c->lastPieces) { c->err = "the last batch corrected through this context ran with pieces off"; return TALC_ERR_ARG; }
+  *total = c->lastPiecesTotal;
+  if (c->lastPiecesTotal > cap) { c->err = "cap is smaller than the number of pieces"; return TALC_ERR_CAPACITY; }
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  if (piece_off)
+    CUDA_TRY(c, cudaMemcpyAsync(piece_off, c->pieceOff.p, ((size_t)c->lastN + 1) * 8, cudaMemcpyDefault, c->stream));
+  if (c->lastPiecesTotal)
+    CUDA_TRY(c, cudaMemcpyAsync(bounds, c->pieceBounds.p, (size_t)c->lastPiecesTotal * 8, cudaMemcpyDefault, c->stream));
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return TALC_OK;
+}
+
+// the pieces rule on any reads, whatever the context's settings
+int talc_pieces_batch(talc_ctx* c, const uint8_t* bases, const uint64_t* offsets, uint32_t n, const uint8_t* flip, int mode,
+                      uint32_t min_len, uint64_t* piece_off, uint32_t* bounds, uint64_t cap, uint64_t* total) {
+  if (!c || !offsets || !total || (n && !bases) || (cap && !bounds)) return TALC_ERR_ARG;
+  if ((mode != TALC_PIECES_TRIM && mode != TALC_PIECES_SPLIT) || min_len == 0) {
+    c->err = "pieces mode must be TALC_PIECES_TRIM or TALC_PIECES_SPLIT, min_len at least 1";
+    return TALC_ERR_ARG;
+  }
+  if (c->parent) lane_follow(c);
+  if (!c->tableReady) { c->err = "no k-mer table loaded"; return TALC_ERR_NO_TABLE; }
+  if (offsets[0] != 0) { c->err = "offsets[0] must be 0"; return TALC_ERR_ARG; }
+  c->lastPieces = false;  // the buffers of talc_last_pieces are reused
+  *total = 0;
+  if (!n) {
+    if (piece_off) piece_off[0] = 0;
+    return TALC_OK;
+  }
+  CUDA_TRY(c, cudaSetDevice(c->device));
+  const u64 tot = offsets[n];
+  CUDA_TRY(c, c->bases.reserve(tot + 64));
+  CUDA_TRY(c, c->offs.reserve((size_t)(n + 1) * 8));
+  CUDA_TRY(c, c->orientOut.reserve((size_t)n + 1));  // the flags; the strands of a correction stay
+  CUDA_TRY(c, cudaMemcpyAsync(c->bases.p, bases, tot, cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(c, cudaMemcpyAsync(c->offs.p, offsets, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+  if (flip) CUDA_TRY(c, cudaMemcpyAsync(c->orientOut.p, flip, n, cudaMemcpyHostToDevice, c->stream));
+  u64 hTotal = 0;
+  int rc = run_pieces(c, (const u8*)c->bases.p, (const u64*)c->offs.p, n, tot, nullptr, (const u8*)c->orientOut.p,
+                      flip ? TALC_STRAND_AUTO : TALC_STRAND_FORWARD, (u32)mode, min_len, &hTotal);
+  if (rc) return rc;
+  CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  *total = hTotal;
+  if (hTotal > cap) { c->err = "cap is smaller than the number of pieces"; return TALC_ERR_CAPACITY; }
+  if (piece_off) CUDA_TRY(c, cudaMemcpyAsync(piece_off, c->pieceOff.p, (size_t)(n + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
+  if (hTotal) CUDA_TRY(c, cudaMemcpyAsync(bounds, c->pieceBounds.p, (size_t)hTotal * 8, cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   return TALC_OK;
 }
